@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          # our CUDA path
     python bench.py --impl reference --gpus N ...          # the CPU oracle (restated reference)
+    python bench.py ... --dump-outputs DIR                 # + the image of the last timed step as DIR/*.npy
 
 A "step" is one full render of the workload: every pixel x sample of
 cornell_box.yml at 1920x1080, 1024 spp, max_depth 20 (BASELINE configs[3], the
@@ -157,6 +158,34 @@ def measured_peaks():
     return {"hbm_gbs": 6650.0}, "fallback"
 
 
+DUMP_BYTES = 64 * 10**6 - 4096     # everything --dump-outputs writes, .npy headers included
+
+
+def dump_outputs(out_dir, image):
+    """Write the (H, W, 3) image of the last timed step as out_dir/image.npy.  An image larger than DUMP_BYTES is
+    written as a fixed, seeded sample of its pixels instead: image_sample.npy (K, 3) and the sampled pixels' flat
+    indices y * W + x, ascending, in image_sample_pixels.npy (float64, exact)."""
+    os.makedirs(out_dir, exist_ok=True)
+    h, w, c = image.shape
+    if image.nbytes <= DUMP_BYTES:
+        np.save(os.path.join(out_dir, "image.npy"), image)
+        return
+    k = DUMP_BYTES // (c * image.itemsize + 8)
+    pixels = np.sort(np.random.default_rng(0).choice(h * w, size=k, replace=False))
+    np.save(os.path.join(out_dir, "image_sample.npy"), image.reshape(h * w, c)[pixels])
+    np.save(os.path.join(out_dir, "image_sample_pixels.npy"), pixels.astype(np.float64))
+
+
+def device_image(ptr, shape):
+    """A float32 CUDA tensor over device memory the library owns (no copy; valid while that memory is)."""
+    import torch
+
+    class View:
+        __cuda_array_interface__ = {"shape": shape, "typestr": "<f4", "data": (ptr, False), "strides": None,
+                                    "version": 2}
+    return torch.as_tensor(View(), device="cuda")
+
+
 def oracle_slice(job, params, spp, threads=0):
     """Time the oracle (restated reference, f64, all host threads) on an spp-slice."""
     from oracle import oracle as O
@@ -222,7 +251,14 @@ def main():
                          "(which one ran is reported in config.kernel); 1: the same but fail instead; 0: precompiled kernels")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--lbvh", action="store_true", help="rebuild the BVH on the GPU (rc_build_lbvh) after the upload")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the image the last timed step computed as DIR/*.npy (rank 0; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        # its sample slice is sized from a timing probe, so two runs need not render the same samples
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         return run_reference(args, args.workload)
@@ -292,11 +328,12 @@ def main():
         if rank != 0:
             frame = r.frame_open(bytes(hbuf.cpu().tolist()), w, h, rank, world)
 
-    def step(p=None):
+    def step(p=None, want_image=False):
+        """One render; with want_image (rank 0) returns the device pointer of its finished (H, W, 3) float image."""
         p = params if p is None else p
         if frame is not None:
-            r.render_frame(p, frame)          # enqueues only: kernels and stream-ordered waits, no host sync, no collective
-            return
+            # enqueues only: kernels and stream-ordered waits, no host sync, no collective
+            return r.render_frame(p, frame, want_device_ptr=want_image)
         accum.zero_()
         r.render_accumulate(p, accum.data_ptr())
         if world > 1:
@@ -304,6 +341,7 @@ def main():
             dist.reduce(accum, dst=0, op=dist.ReduceOp.SUM)
         if rank == 0:
             r.finalize(accum.data_ptr(), w, h, spp, rgb.data_ptr())
+        return rgb.data_ptr()
 
     def launches_per_step():
         """Our kernels per step: the render call's own launches (read back after a step), + the zero-fill of the
@@ -329,10 +367,11 @@ def main():
     kernel_ms = []
     barrier()
     wall0 = time.perf_counter()
+    dump = bool(args.dump_outputs) and rank == 0
     for i in range(args.steps):
         flush.fill_(float(i))          # L2 flush between timed iterations (outside the events)
         ev[i][0].record(stream)
-        step()
+        image_ptr = step(want_image=dump and i == args.steps - 1)
         ev[i][1].record(stream)
     barrier()
     kernel_ms.append(r.stats().gpu_ms)   # of the last step
@@ -341,6 +380,9 @@ def main():
     if sampler_thread:
         sampler_thread.stop_flag.set()
         sampler_thread.join()
+    if dump:
+        # copied now: the e2e passes below render into the same frame images
+        dump_outputs(args.dump_outputs, device_image(image_ptr, (h, w, 3)).cpu().numpy())
     ms = sum(a.elapsed_time(b) for a, b in ev)
     t = torch.tensor([ms], dtype=torch.float64, device="cuda")
     if world > 1:

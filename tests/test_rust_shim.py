@@ -1,12 +1,15 @@
 """The reference-side binding (racer_tracer_b200/rust_shim): what can be checked without a Rust toolchain.
 
-* reference.diff — the patch a maintainer applies to the reference crate — APPLIES to /root/reference
-  (`patch --dry-run`), and is exactly what tools/make_rust_patch.py generates from the sources kept here;
+* reference.diff — the patch a maintainer applies to the reference crate — carries the two new source files kept
+  here and every edit tools/make_rust_patch.py makes, and nothing else;
+* with a checkout of the reference crate (RACER_TRACER_REFERENCE = its racer-tracer/ directory; the repository
+  keeps nothing of the reference but the patch's context lines): the patch APPLIES to it (`patch --dry-run`), is
+  exactly what tools/make_rust_patch.py generates from it, and every trait method the patch adds is implemented
+  for every type of the reference that implements the trait;
 * racer-cuda-sys binds every function include/racer_cuda.h declares, and its #[repr(C)] structs list the
   header's fields in the header's order;
-* the Rust sources are at least lexically sound (balanced delimiters outside strings and comments), every trait
-  method the patch adds is implemented for every type of the reference that implements the trait.
-The image has no cargo / rustc: nothing here compiles Rust.
+* the Rust sources are at least lexically sound (balanced delimiters outside strings and comments).
+Nothing here compiles Rust.
 """
 import os
 import re
@@ -18,13 +21,16 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SHIM = os.path.join(ROOT, "racer_tracer_b200", "rust_shim")
-REF = "/root/reference/racer-tracer"
+REF = os.environ.get("RACER_TRACER_REFERENCE", "")
 HEADER = open(os.path.join(ROOT, "include", "racer_cuda.h")).read()
 SYS = open(os.path.join(SHIM, "racer-cuda-sys", "src", "lib.rs")).read()
 DIFF = os.path.join(SHIM, "patch", "reference.diff")
 
+sys.path.insert(0, os.path.join(ROOT, "tools"))
+import make_rust_patch  # noqa: E402
+
 needs_reference = pytest.mark.skipif(not os.path.isdir(REF) or shutil.which("patch") is None,
-                                     reason="the reference checkout / patch(1) is not on this machine")
+                                     reason="needs RACER_TRACER_REFERENCE (a checkout of the reference crate) and patch(1)")
 
 
 def strip_rust(src):
@@ -47,10 +53,60 @@ def test_patch_applies_to_the_reference():
         assert f in touched, f
 
 
+def diff_hunks(text):
+    """{file: [(old lines, new lines, added lines)]} of a `diff -ruN a b`; every hunk's line counts are checked
+    against its header, so that patch(1) can read it."""
+    files, hunks, hunk = {}, None, None
+    for ln in text.splitlines(keepends=True):
+        m = re.match(r"diff -ruN a/(\S+) b/\S+$", ln)
+        if m:
+            hunks = files.setdefault(m.group(1), [])
+            continue
+        if ln.startswith(("--- a/", "+++ b/")):
+            continue
+        m = re.match(r"@@ -\d+(?:,(\d+))? \+\d+(?:,(\d+))? @@", ln)
+        if m:
+            hunk = (int(m.group(1) or 1), int(m.group(2) or 1), [], [], [])
+            hunks.append(hunk)
+            continue
+        tag, body = ln[0], ln[1:]
+        assert tag in " -+", ln
+        if tag in " -":
+            hunk[2].append(body)
+        if tag in " +":
+            hunk[3].append(body)
+        if tag == "+":
+            hunk[4].append(body)
+    for f, hs in files.items():
+        for n_old, n_new, old, new, _ in hs:
+            assert (len(old), len(new)) == (n_old, n_new), f"{f}: hunk line counts differ from its header"
+    return {f: [h[2:] for h in hs] for f, hs in files.items()}
+
+
+def test_committed_patch_carries_the_generators_edits_and_new_files():
+    """What tools/make_rust_patch.py writes, as far as it can be checked without the reference: the new files
+    exactly as kept under rust_shim/, every edit's text where its anchor puts it, no line added by anything else."""
+    files = diff_hunks(open(DIFF).read())
+    edits = make_rust_patch.EDITS
+    assert sorted(files) == sorted(set(make_rust_patch.NEW_FILES) | {e[0] for e in edits})
+    for rel in make_rust_patch.NEW_FILES:
+        assert [old for old, _, _ in files[rel]] == [[]], rel
+        assert "".join(files[rel][0][1]) == open(os.path.join(SHIM, "racer-tracer", rel)).read(), \
+            f"{rel} differs from the patch: run tools/make_rust_patch.py"
+    for rel, anchor, text, where in edits:
+        fragment = {"after": anchor + text, "before": text + anchor, "replace": text}[where]
+        assert any(fragment in "".join(new) for _, new, _ in files[rel]), (rel, text[:80])
+        if where == "replace":
+            assert any(anchor in "".join(old) for old, _, _ in files[rel]), (rel, anchor[:80])
+    for rel, hunks in files.items():
+        if rel not in make_rust_patch.NEW_FILES:
+            allowed = set("".join(e[2] for e in edits if e[0] == rel).splitlines(keepends=True))
+            extra = [ln for _, _, added in hunks for ln in added if ln not in allowed]
+            assert not extra, f"{rel}: lines no edit adds: {extra[:3]}"
+
+
 @needs_reference
 def test_committed_patch_is_what_the_generator_writes(tmp_path):
-    sys.path.insert(0, os.path.join(ROOT, "tools"))
-    import make_rust_patch
     out = make_rust_patch.build(REF, str(tmp_path / "reference.diff"))
     assert open(out).read() == open(DIFF).read(), "run tools/make_rust_patch.py"
 

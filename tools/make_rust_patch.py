@@ -7,7 +7,7 @@ small edits to existing reference files listed in EDITS below (a method added to
 type, two enum variants, one factory arm, one error variant).  The script copies the reference crate to a scratch
 directory, applies the edits there (every anchor must occur exactly once), and writes `diff -ruN` of the two trees.
 Nothing of the reference is stored in this repository except the context lines of that diff.
-tests/test_rust_shim.py applies the result to /root/reference with `patch --dry-run` (where the reference exists).
+tests/test_rust_shim.py applies the result with `patch --dry-run` to the checkout RACER_TRACER_REFERENCE names.
 
 No Rust toolchain exists in this image: the patch is checked to APPLY, not to compile.
 
