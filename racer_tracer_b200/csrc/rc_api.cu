@@ -175,6 +175,36 @@ void free_tables(DeviceState& d) {
     d.prim_id.release(); d.nodes_d.release(); d.prim_inst.release(); d.instances_d.release();
 }
 
+// Checker levels of the longest chain of checker textures (checkered.rs:32-43 follows children without a limit), or -1
+// when a chain runs into a cycle; then *cycle_at is a texture on it.  The children must already be in range.
+int checker_chain_depth(const rc_scene* s, int* cycle_at) {
+    std::vector<int> depth(s->n_textures, -1);   // -1: not measured yet, -2: on the path being followed
+    int longest = 0;
+    for (int root = 0; root < s->n_textures; ++root) {
+        // iterative depth-first walk: (texture, children visited so far)
+        std::vector<std::pair<int, int>> stack{{root, 0}};
+        while (!stack.empty()) {
+            auto& top = stack.back();
+            const rc_texture& t = s->textures[top.first];
+            if (t.type != RC_TEX_CHECKER) { depth[top.first] = 0; stack.pop_back(); continue; }
+            if (top.second == 0) {
+                if (depth[top.first] >= 0) { stack.pop_back(); continue; }
+                depth[top.first] = -2;
+            }
+            if (top.second < 2) {
+                const int child = top.second++ == 0 ? t.a : t.b;
+                if (depth[child] == -2) { *cycle_at = child; return -1; }
+                if (depth[child] == -1) stack.push_back({child, 0});
+                continue;
+            }
+            depth[top.first] = 1 + std::max(depth[t.a], depth[t.b]);
+            longest = std::max(longest, depth[top.first]);
+            stack.pop_back();
+        }
+    }
+    return longest;
+}
+
 int validate_scene(const rc_scene* s) {
     if (!s) return fail(RC_ERR_INVALID, "scene is NULL");
     if (s->n_prims < 0 || s->n_materials < 0 || s->n_textures < 0 || s->n_images < 0 || s->n_perlin < 0 || s->n_nodes < 0)
@@ -215,6 +245,9 @@ int validate_scene(const rc_scene* s) {
         if (t.type == RC_TEX_IMAGE && (t.a < 0 || t.a >= s->n_images)) return fail(RC_ERR_INVALID, "image index out of range");
         if (t.type == RC_TEX_NOISE && (t.a < 0 || t.a >= s->n_perlin)) return fail(RC_ERR_INVALID, "perlin index out of range");
     }
+    int cycle_at = -1;
+    if (checker_chain_depth(s, &cycle_at) < 0)
+        return fail(RC_ERR_INVALID, "checker texture " + std::to_string(cycle_at) + " is its own descendant (a cycle of checker children)");
     for (int i = 0; i < s->n_nodes; ++i) {
         const rc_bvh_node& n = s->nodes[i];
         if (n.left >= 0) {
@@ -896,6 +929,8 @@ static void build_tables(const rc_scene* s, HostTables& t) {
     kp.ref_aabb = any_rotate ? 1 : 0;
     kp.has_motion = any_motion ? 1 : 0;
     kp.n_prims = s->n_prims; kp.n_nodes = s->n_nodes; kp.n_perlin = s->n_perlin;
+    int cycle_at = -1;
+    kp.checker_depth = checker_chain_depth(s, &cycle_at);   // validate_scene has ruled out cycles
     kp.bg_a = f4(s->bg_a[0], s->bg_a[1], s->bg_a[2], bits(s->bg_type));
     kp.bg_b = f4(s->bg_b[0], s->bg_b[1], s->bg_b[2], 0.f);
     // type-sorted table for the linear modes (stable: canonical order within a kind)

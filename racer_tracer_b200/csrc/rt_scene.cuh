@@ -123,6 +123,7 @@ struct KParams {
     int n_prims, n_nodes;
     int lin_end[4];             // type-sorted linear table: [0,lin_end[0]) spheres, then xy, xz, yz rects
     int n_perlin;
+    int checker_depth;          // checker levels of the longest texture chain (rc_upload_scene rejects cycles)
     int lens_enabled;
     int tile_cull;              // 1: a CTA first asks whether its tile's primary rays can hit anything at all (pinhole
                                 // camera, nothing moves, linear modes); if not, its samples are background only
@@ -1002,12 +1003,13 @@ struct TexCtx {            // where the Perlin tables live for this kernel
 };
 
 // Texture::value for a non-solid texture index (solid colours are folded into
-// the primitive record).  Checker children are resolved iteratively.
+// the primitive record).  Checker children are resolved iteratively, to any
+// depth: the upload measures the longest chain, which bounds the loop.
 template <class Scene>
 RT_D vec3f texture_value(const KParams& P, const TexCtx& X, const Scene& S, int tex, int prim, const Hit& h) {
     DevTexture t = P.textures[tex];
 #pragma unroll 1
-    for (int level = 0; level < 4 && t.type == RT_TEX_CHECKER; ++level) {
+    for (int level = 0; level < P.checker_depth && t.type == RT_TEX_CHECKER; ++level) {
         // checkered.rs:32-43 — world-space sines, odd if negative
         float sines = sinf(h.p.x * t.scale) * sinf(h.p.y * t.scale) * sinf(h.p.z * t.scale);
         t = P.textures[sines < 0.0f ? t.b : t.a];

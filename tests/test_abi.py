@@ -120,6 +120,22 @@ def test_specialised_source_compiles_for_sm_100a(cuda_lib, cfg, tmp_path):
     assert cuda_lib.rc_spec_source(big.scene.ptr, None, 0) > 0          # 23 spheres still fit the constant bank
 
 
+def test_checker_chains_of_any_depth_and_cycles(cuda_lib, cfg):
+    """Checker children are followed to any depth (checkered.rs:32-43), so a chain of six is a valid scene; a cycle of
+    checker children — which YAML cannot express but a host can pass — is rejected with a message that names it.
+    rc_spec_source runs the same scene validation as rc_upload_scene, without a GPU."""
+    from test_gpu_shading_probes import checker_chain_job
+    job = checker_chain_job(cfg, 6)
+    assert cuda_lib.rc_spec_source(job.scene.ptr, None, 0) > 0, cuda_lib.rc_last_error()
+    top = job.scene.c.n_textures - 1
+    for leaf in (1, top):                    # c_1's leaf pointing back at the root; the root pointing at itself
+        job = checker_chain_job(cfg, 6)
+        tex = job.scene.c.textures
+        tex[leaf].type, tex[leaf].a, tex[leaf].b = capi.RC_TEX_CHECKER, top, 0
+        assert cuda_lib.rc_spec_source(job.scene.ptr, None, 0) == -1
+        assert b"cycle" in cuda_lib.rc_last_error()
+
+
 def _compile_like_the_library(src: str, tmp_path):
     """NVRTC with the headers and options rc_spec.cuh uses (it is stricter than nvcc about inline functions
     that are declared but never defined); nvcc when the cuda-python bindings are not importable."""
