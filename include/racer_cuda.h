@@ -205,7 +205,9 @@ typedef struct rc_params {
     int32_t  variant;         /* RC_VARIANT_*                               */
     int32_t  sampler;         /* RC_SAMPLER_*                               */
     int32_t  split;           /* RC_SPLIT_*                                 */
-    int32_t  tile_w, tile_h;  /* interleaved tile size; 0 = default         */
+    int32_t  tile_w, tile_h;  /* interleaved tile size: 0 x 0 or 16 x 8, the
+                                 kernels' fixed tile; anything else is
+                                 RC_ERR_INVALID                             */
     int32_t  rank, world;     /* this participant's slot when the caller
                                  drives several processes; 0,1 otherwise    */
     int32_t  fixed_jitter;    /* 1: pixel-centre, lens-centre rays
@@ -238,7 +240,8 @@ typedef struct rc_tone_map {
 /* Counters of the last render on this context (device work only). */
 typedef struct rc_stats {
     double   gpu_ms;          /* CUDA-event time of the last render call    */
-    uint64_t samples;         /* pixel-samples traced                       */
+    uint64_t samples;         /* pixel-samples traced by this context's
+                                 participants (their shares only)           */
     uint64_t segments;        /* ray segments traced (0 if not counted)     */
     uint64_t kernel_launches; /* kernels launched by the last render call   */
     int32_t  n_devices;
@@ -294,7 +297,15 @@ int rc_set_camera(rc_ctx* ctx, const rc_camera* camera);
  * passes like do_cancel (src/renderer.rs:25-30); a cancelled render returns
  * RC_OK without touching out_rgb (cpu.rs:55-62).  With several devices in
  * the context the image is partitioned as params->split says and gathered /
- * reduced onto device 0 before the download. */
+ * reduced onto device 0 before the download.
+ * With params->world > 1 the call renders only this participant's share
+ * (params->rank): a tile share gives sqrt(sum / samples) in its tiles and
+ * 0.0 in every other pixel; a sample share gives sqrt(share_sum / samples)
+ * in every pixel, where share_sum is the sum over its samples only (so
+ * samples * out^2, summed over the ranks, is the whole frame's sum), and
+ * all zeros when the share holds no sample (samples < world).  Nothing of
+ * an earlier render shows through.  rc_get_stats' `samples` is the share's
+ * pixel-samples. */
 int rc_render(rc_ctx* ctx, const rc_params* params, double* out_rgb,
               const volatile int32_t* cancel);
 
@@ -306,8 +317,8 @@ int rc_render(rc_ctx* ctx, const rc_params* params, double* out_rgb,
  * (cpu_scaled.rs:55-60) — and, after scale_sqrt, fills the block (cpu_scaled.rs:75-86).  scale_w and
  * scale_h are what CpuRendererScaled::new derives (cpu_scaled.rs:31-34: the highest divisor of
  * image.width / num_threads_width not above config.preview.scale); columns / rows beyond the last
- * whole block stay 0 as in the reference.  out_rgb: width*height*3 doubles.  Cancel semantics as
- * rc_render. */
+ * whole block stay 0 as in the reference.  out_rgb: width*height*3 doubles.  Cancel semantics and the
+ * share of params->rank / params->world (over the grid of blocks) as rc_render. */
 int rc_render_preview(rc_ctx* ctx, const rc_params* params, int32_t scale_w, int32_t scale_h,
                       double* out_rgb, const volatile int32_t* cancel);
 

@@ -843,6 +843,8 @@ int oracle_render_preview(const rc_scene* scene, const rc_camera* camera, const 
     if (opt.tiles_w <= 0) opt.tiles_w = 10;
     if (opt.tiles_h <= 0) opt.tiles_h = 10;
     const int rounds = params->rng_rounds > 0 ? params->rng_rounds : 10;
+    const int s_begin = opt.sample_begin;
+    const int s_count = opt.sample_count > 0 ? opt.sample_count : params->samples;
     const int W = params->width, H = params->height;
     const int grid_w = W / scale_w;   // block grid of the whole screen (Philox pixel index)
     std::memset(out_rgb, 0, sizeof(double) * 3 * (size_t)W * H);   // vec![Vec3::default(); ..], cpu_scaled.rs:53
@@ -865,7 +867,7 @@ int oracle_render_preview(const rc_scene* scene, const rc_camera* camera, const 
                 dr.seq = &seq;
                 const double u = pixel_u(*params, dr, x);   // once per block, cpu_scaled.rs:55-56
                 V3 color = v3(0, 0, 0);
-                for (int s = 0; s < params->samples; ++s) {
+                for (int s = s_begin; s < s_begin + s_count; ++s) {
                     dr.sample = (uint32_t)s;
                     color = color + trace_sample(*scene, *camera, *params, dr, u, x, y, cnt).rgb;   // v: cpu_scaled.rs:59-60
                 }

@@ -130,9 +130,11 @@ def render(job, params: rc_params, rng=RNG_PHILOX, threads=0, tiles=(10, 10), sa
     return (out, cnt) if want_counters else out
 
 
-def render_preview(job, params: rc_params, scale_w: int, scale_h: int, rng=RNG_PHILOX, tiles=(10, 10)):
-    """oracle_render_preview (CpuRendererScaled, cpu_scaled.rs); returns (H,W,3) float64."""
-    opt = oracle_options(rng, 1, tiles[0], tiles[1], 0, 0, 0, 0)
+def render_preview(job, params: rc_params, scale_w: int, scale_h: int, rng=RNG_PHILOX, tiles=(10, 10), sample_begin=0,
+                   sample_count=0):
+    """oracle_render_preview (CpuRendererScaled, cpu_scaled.rs); returns (H,W,3) float64.  sample_begin / sample_count:
+    only those samples are traced (a sample share), still scaled by 1 / params.samples."""
+    opt = oracle_options(rng, 1, tiles[0], tiles[1], sample_begin, sample_count, 0, 0)
     out = np.empty((params.height, params.width, 3), dtype=np.float64)
     st = lib().oracle_render_preview(job.scene.ptr, C.byref(job.camera), C.byref(params), C.byref(opt),
                                      scale_w, scale_h, out.ctypes.data_as(_pd))

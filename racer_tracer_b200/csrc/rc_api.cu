@@ -363,6 +363,8 @@ int check_params(const rc_params* p) {
     if (p->sampler != RC_SAMPLER_DIRECT && p->sampler != RC_SAMPLER_REJECTION) return fail(RC_ERR_INVALID, "unknown sampler");
     if (p->split != RC_SPLIT_TILES && p->split != RC_SPLIT_SAMPLES) return fail(RC_ERR_INVALID, "unknown split");
     if (p->specialize < 0 || p->specialize > 2) return fail(RC_ERR_INVALID, "specialize must be 0, 1 or 2");
+    if (!(p->tile_w == 0 && p->tile_h == 0) && !(p->tile_w == RT_TILE_W && p->tile_h == RT_TILE_H))
+        return fail(RC_ERR_INVALID, "tile_w x tile_h must be 0 x 0 or 16 x 8 (the kernels' tile is fixed)");
     return RC_OK;
 }
 
@@ -589,12 +591,36 @@ int ensure_accum(rc_ctx* ctx, const rc_params* p, bool device0_too, bool zero = 
 }
 
 // rc_render / rc_render_preview own their accumulation buffers and trace every pixel's samples in ONE launch, so the
-// megakernel can STORE the sums instead of adding them to a zero-filled buffer (no memset, no read of the frame):
-// always with one device; with several when every pixel of a buffer is written by exactly one kernel — peer stores
-// into device 0's buffer, or a sample split (every device writes all pixels of its own buffer, ncclReduce adds them).
+// megakernel can STORE the sums instead of adding them to a zero-filled buffer (no memset, no read of the frame) —
+// but only when this call's launches write every pixel of every buffer read afterwards: a tile split with a single
+// participant overall (one device, or peer stores of all devices into device 0's buffer, and world = 1), or a sample
+// split in which every device of the context has samples to trace (each writes all pixels of its own buffer,
+// ncclReduce adds them).  Otherwise a pixel nobody writes would keep the previous render's sums.
 bool can_store(const rc_ctx* ctx, const rc_params* p) {
     if (p->variant != RC_VARIANT_MEGAKERNEL) return false;
-    return ctx->devs.size() == 1 || direct_tiles(ctx, p) || p->split == RC_SPLIT_SAMPLES;
+    const int n_dev = (int)ctx->devs.size();
+    const int world = p->world > 0 ? p->world : 1;
+    if (p->split == RC_SPLIT_TILES) return world == 1 && (n_dev == 1 || direct_tiles(ctx, p));
+    const int parts = world * n_dev;
+    for (int k = 0; k < n_dev; ++k) {
+        const int part = p->rank * n_dev + k;
+        if ((long long)p->samples * (part + 1) / parts <= (long long)p->samples * part / parts) return false;
+    }
+    return true;
+}
+
+// pixel-samples of participant `part`'s share: its tiles clipped to the image, times its samples
+uint64_t share_samples(const rc_params* p, int part, int parts) {
+    KParams kp;
+    std::memset(&kp, 0, sizeof(kp));
+    partition(kp, p, part, parts);
+    uint64_t pixels = 0;
+    for (int i = 0; i < kp.n_tiles; ++i) {
+        const int tile = kp.tile_first + i * kp.tile_stride;
+        const int tx = tile % kp.tiles_x, ty = tile / kp.tiles_x;
+        pixels += (uint64_t)std::min(RT_TILE_W, p->width - tx * RT_TILE_W) * std::min(RT_TILE_H, p->height - ty * RT_TILE_H);
+    }
+    return pixels * (uint64_t)(kp.s_end - kp.s_begin);
 }
 
 // End of a render call: the stop event is recorded, nothing is waited for.  Time and segment counters are
@@ -604,8 +630,10 @@ int finish_stats(rc_ctx* ctx, const rc_params* p) {
     DeviceState& d0 = ctx->devs[0];
     CUDA_TRY(cudaSetDevice(d0.device));
     CUDA_TRY(cudaEventRecord(d0.ev1, d0.stream));
-    const int world = p->world > 0 ? p->world : 1;
-    ctx->stats.samples = (uint64_t)p->width * p->height * p->samples / world;
+    const int n_dev = (int)ctx->devs.size();
+    const int parts = (p->world > 0 ? p->world : 1) * n_dev;
+    ctx->stats.samples = 0;
+    for (int k = 0; k < n_dev; ++k) ctx->stats.samples += share_samples(p, p->rank * n_dev + k, parts);
     ctx->stats_pending = true;
     return RC_OK;
 }
@@ -1456,6 +1484,10 @@ int rc_render_frame(rc_ctx* ctx, const rc_params* p, rc_frame* f, const float** 
     ctx->overwrite = false;
     ctx->final_scale = 0.0f;
     if (rc != RC_OK) return rc;
+    if (by_samples && (long long)p->samples * (f->rank + 1) / world <= (long long)p->samples * f->rank / world) {
+        // fewer samples than ranks and none for this one: its slot still holds frame n - 2's sums, and rank 0 adds it
+        CUDA_TRY(cudaMemsetAsync(target, 0, f->image_floats * sizeof(float), d.stream));
+    }
     uint64_t extra = 0;
     if (world > 1) {
         if (f->rank != 0) { frame_publish_kernel<<<1, 1, 0, d.stream>>>(f->words + 32 * f->rank, frame_no); extra = 2; }

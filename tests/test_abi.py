@@ -79,6 +79,20 @@ def test_null_arguments_are_rejected(cuda_lib):
     assert cuda_lib.rc_render(None, C.byref(p), None, None) == capi.RC_ERR_INVALID
 
 
+@pytest.mark.parametrize("tile", [(0, 0), (16, 8)])
+def test_the_fixed_tile_size_is_accepted(cuda_lib, tile):
+    sh = harness.partition(harness.make_params(40, 20, 1, 1, tile_w=tile[0], tile_h=tile[1], rank=1, world=2), 1, 2)
+    assert (sh["tile_w"], sh["tile_h"], sh["tiles_x"], sh["n_tiles"]) == (16, 8, 3, 4)
+
+
+@pytest.mark.parametrize("tile", [(32, 8), (16, 16), (8, 4), (16, 0), (0, 8), (-16, 8)])
+def test_any_other_tile_size_is_rejected(cuda_lib, tile):
+    """The kernels trace 16 x 8 tiles only: a caller asking for others must not silently get them."""
+    with pytest.raises(capi.RacerCudaError) as e:
+        harness.partition(harness.make_params(40, 20, 1, 1, tile_w=tile[0], tile_h=tile[1]), 0, 1)
+    assert e.value.status == capi.RC_ERR_INVALID and "tile_w" in str(e.value)
+
+
 def test_product_never_touches_the_oracle():
     """Nothing under racer_tracer_b200/ may import, link or open oracle/."""
     pkg = os.path.join(ROOT, "racer_tracer_b200")

@@ -343,6 +343,22 @@ def test_two_devices_in_one_context(renderer, cfg):
         assert r2.stats().n_devices == 2
         two_s = r2.render(harness.make_params(w, h, spp, 20, seed=4, split=capi.RC_SPLIT_SAMPLES))
         assert np.allclose(one, two_s, rtol=1e-5, atol=1e-6)
+        # Shares that leave buffers unwritten, each right after a full render at the same size.  A 1-spp sample split:
+        # sample 0 goes to device 1 and device 0's share is empty, so the reduce must add zeros, not old sums.
+        from test_gpu_shares import tile_mask
+        one1 = renderer.render(harness.make_params(w, h, 1, 20, seed=6))
+        r2.render(harness.make_params(w, h, spp, 20, seed=5, split=capi.RC_SPLIT_SAMPLES))
+        assert np.array_equal(r2.render(harness.make_params(w, h, 1, 20, seed=6, split=capi.RC_SPLIT_SAMPLES)), one1)
+        # rank 1 of world 2 on the two-device context: participants 2 and 3 of 4.  Tile split: tiles k mod 4 in {2, 3}
+        # and zeros elsewhere; sample split at 1 spp: participant 3 traces sample 0, participant 2 nothing.
+        own = tile_mask(w, h, 2, 4) | tile_mask(w, h, 3, 4)
+        r2.render(harness.make_params(w, h, spp, 20, seed=5))
+        share = r2.render(harness.make_params(w, h, spp, 20, seed=4, rank=1, world=2))
+        assert (share[~own] == 0.0).all() and np.array_equal(share[own], one[own])
+        assert r2.stats().samples == int(own.sum()) * spp
+        r2.render(harness.make_params(w, h, spp, 20, seed=5))
+        share = r2.render(harness.make_params(w, h, 1, 20, seed=6, rank=1, world=2, split=capi.RC_SPLIT_SAMPLES))
+        assert np.array_equal(share, one1) and r2.stats().samples == w * h
         wf = r2.render(harness.make_params(w, h, spp, 20, seed=4, variant=capi.RC_VARIANT_WAVEFRONT))
         # a different kernel: FMA contraction differs by an ulp here and there and a path on a reflect / refract
         # threshold may flip (one pixel of 66 933 did, measured) — the same criterion as the one-device comparison

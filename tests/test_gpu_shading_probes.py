@@ -216,22 +216,23 @@ def _tolerance(oracle, job, params, ref):
     return tol + _noise_tolerance(oracle, job, params)
 
 
-def _oracle_linear(oracle, job, q, preview):
+def _oracle_linear(oracle, job, q, preview, sample=0):
+    """The linear radiance of sample `sample` alone (q.samples = 1)."""
     if preview:
-        return oracle.render_preview(job, q, *preview) ** 2 * q.samples
-    return oracle.render(job, q, linear_sum=True)
+        return oracle.render_preview(job, q, *preview, sample_begin=sample, sample_count=1) ** 2 * q.samples
+    return oracle.render(job, q, linear_sum=True, sample_begin=sample, sample_count=1)
 
 
 _REF_CACHE = {}
 
 
-def reference(oracle, job, key, depth, sampler=capi.RC_SAMPLER_DIRECT, rounds=0, preview=None, widen=False):
-    """(linear radiance, per-pixel tolerance, instability mask) of the oracle; cached per key."""
-    ck = (key, depth, sampler, rounds, preview, widen)
+def reference(oracle, job, key, depth, sampler=capi.RC_SAMPLER_DIRECT, rounds=0, preview=None, widen=False, sample=0):
+    """(linear radiance, per-pixel tolerance, instability mask) of the oracle's sample `sample`; cached per key."""
+    ck = (key, depth, sampler, rounds, preview, widen, sample)
     if ck in _REF_CACHE:
         return _REF_CACHE[ck]
     q = harness.make_params(job.width, job.height, 1, depth, seed=SEED, sampler=sampler, rng_rounds=rounds)
-    ref = _oracle_linear(oracle, job, q, preview)
+    ref = _oracle_linear(oracle, job, q, preview, sample)
     tol = _tolerance(oracle, job, q, ref)
     cam = job.camera
     right, up = np.array(list(cam.right)), np.array(list(cam.up))
@@ -239,7 +240,7 @@ def reference(oracle, job, key, depth, sampler=capi.RC_SAMPLER_DIRECT, rounds=0,
     for scale in ((1.0, 4.0) if widen else (1.0,)):
         delta = scale * _delta(job)
         for sx, sy in ((1, 0), (-1, 0), (0, 1), (0, -1), (1, 1), (-1, -1), (1, -1), (-1, 1)):
-            shifted = _oracle_linear(oracle, _with_camera_shift(job, delta * (sx * right + sy * up)), q, preview)
+            shifted = _oracle_linear(oracle, _with_camera_shift(job, delta * (sx * right + sy * up)), q, preview, sample)
             mask |= (np.abs(shifted - ref) > tol).any(axis=2)
     # the fp32 ray direction (upper_left_corner + u horizontal - v vertical - origin) carries 8 ulp of its length: at
     # the horizon of a ground plane that moves the hit point far more than the translation above
@@ -250,7 +251,7 @@ def reference(oracle, job, key, depth, sampler=capi.RC_SAMPLER_DIRECT, rounds=0,
         e = _texture_point_error(job)
         nudged += [_with_translation(job, sign * e * axis) for axis in np.eye(3) for sign in (1.0, -1.0)]
     for j in nudged:
-        mask |= (np.abs(_oracle_linear(oracle, j, q, preview) - ref) > tol).any(axis=2)
+        mask |= (np.abs(_oracle_linear(oracle, j, q, preview, sample) - ref) > tol).any(axis=2)
     _REF_CACHE[ck] = ref, tol, mask
     return _REF_CACHE[ck]
 

@@ -99,6 +99,24 @@ for seed in (21, 22, 23):
     if rank == 0:
         want = r.render(harness.make_params(w, h, spp, 20, seed=seed, specialize=2))
         assert np.allclose(out, want, rtol=2e-6, atol=1e-6), f"sample-split frame seed {seed}: {np.abs(out - want).max()}"
+# ---- fewer samples than ranks: at 1 spp only the last rank has a sample, and every other rank must publish a zeroed
+# slot — not the sums it stored there two frames ago (the frames above left both images' slots non-zero).  Three frames
+# back to back, so that both alternating images are reused.
+kept, seeds = [], (31, 32, 33)
+for seed in seeds:
+    p = harness.make_params(w, h, 1, 20, seed=seed, rank=rank, world=world, specialize=2, split=capi.RC_SPLIT_SAMPLES)
+    dptr = r.render_frame(p, frame, want_device_ptr=(rank == 0))
+    if rank == 0:
+        keep = torch.empty(n, dtype=torch.float32, device="cuda")
+        keep.copy_(harness.device_view(dptr, n), non_blocking=True)
+        kept.append(keep)
+torch.cuda.synchronize()
+dist.barrier()
+if rank == 0:
+    for seed, keep in zip(seeds, kept):
+        got = keep.cpu().numpy().reshape(h, w, 3)
+        want = r.render(harness.make_params(w, h, 1, 20, seed=seed, specialize=2))
+        assert np.allclose(got, want, rtol=3e-7, atol=1e-7), f"1-spp sample-split frame seed {seed}: {np.abs(got - want).max()}"
 r.frame_close(frame)
 r.close()
 if rank == 0:
