@@ -309,6 +309,33 @@ int rc_set_camera(rc_ctx* ctx, const rc_camera* camera);
 int rc_render(rc_ctx* ctx, const rc_params* params, double* out_rgb,
               const volatile int32_t* cancel);
 
+/* Adaptive sampling: every pixel gets as many samples as its noise needs, up to params->samples (S).
+ * Round 0 traces samples [0, min_samples) of every pixel.  After each round every pixel still active is tested; one
+ * that passes stops, the others go from n to min(2n, S) samples.  So each pixel ends with n_p in {n0, 2 n0, 4 n0, ..,
+ * S} (n0 = min_samples), traced as samples [0, n_p) of its own stream with rc_render's seed, jitter and depth: the
+ * pixel equals rc_render's with samples = n_p, up to the order of fp32 sums.
+ * The test, on y = (r + g + b) / 3 of each sample's linear radiance, with S1 = sum y and S2 = sum y^2 over the
+ * pixel's n samples: mu = S1 / n, s^2 = max(0, (S2 - S1^2 / n) / (n - 1)), se = sqrt(s^2 / n), and
+ * err = (sqrt(mu + se) - sqrt(max(mu - se, 0))) / 2 — the half-width of the one-sigma interval of the returned
+ * (gamma'd) value.  The pixel passes when err <= threshold.  S1 comes from the fp32 radiance sums and S2 from fp32
+ * sums of y^2 per round, so err carries their rounding: threshold = 0 stops the pixels whose samples are all equal
+ * where that rounding cancels (samples that are all 0, or exactly representable), and no pixel that has a spread.
+ * out_rgb: width*height*3 doubles, sqrt(sum_p / n_p) as rc_render finalises them with n_p for samples.
+ * out_spp (may be NULL): width*height n_p.  out_err (may be NULL): width*height err at n_p.
+ * rc_get_stats: samples = sum of n_p, segments and kernel_launches of all rounds, gpu_ms of the whole call.
+ * `cancel`: as for rc_render (checked at entry, relayed inside each round, checked between rounds; a cancelled call
+ * writes nothing).  Supported: a one-device context, world <= 1, the megakernel, the direct sampler, 10 Philox rounds;
+ * specialize as for rc_render.  Anything else is RC_ERR_INVALID. */
+typedef struct rc_adaptive {
+    int32_t min_samples;   /* n0 >= 2: samples every pixel gets before its first test            */
+    int32_t reserved;
+    double  threshold;     /* >= 0, finite: stop a pixel once its error estimate is <= threshold   */
+} rc_adaptive;
+
+int rc_render_adaptive(rc_ctx* ctx, const rc_params* params, const rc_adaptive* a,
+                       double* out_rgb, int32_t* out_spp, double* out_err,
+                       const volatile int32_t* cancel);
+
 /* The whole of CpuRendererScaled::render (src/renderer/cpu_scaled.rs:37-121), the preview renderer
  * (`preview_renderer`, src/config.rs:203-207, used while the camera moves, src/main.rs:174-190).
  * params->width/height are the screen; params->samples / max_depth come from config.preview

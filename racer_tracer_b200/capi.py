@@ -91,6 +91,10 @@ class rc_params(C.Structure):
                 ("fixed_jitter", C.c_int32), ("rng_rounds", C.c_int32), ("specialize", C.c_int32)]
 
 
+class rc_adaptive(C.Structure):
+    _fields_ = [("min_samples", C.c_int32), ("reserved", C.c_int32), ("threshold", C.c_double)]
+
+
 class rc_tone_map(C.Structure):
     _fields_ = [("type", C.c_int32), ("reserved", C.c_int32), ("max_white", C.c_double),
                 ("hable", C.c_double * 6), ("exposure_bias", C.c_double),
@@ -110,7 +114,7 @@ ABI_SYMBOLS = [
     "rc_render_preview", "rc_build_lbvh", "rc_get_bvh", "rc_render_tiles_into", "rc_shared_alloc", "rc_shared_open",
     "rc_shared_close", "rc_frame_create", "rc_frame_open", "rc_frame_close", "rc_render_frame",
     "rc_render_accumulate", "rc_finalize", "rc_postprocess", "rc_primary_aov", "rc_get_stats",
-    "rc_last_error", "rc_abi_version", "rc_fp32_peak", "rc_partition", "rc_spec_source",
+    "rc_last_error", "rc_abi_version", "rc_fp32_peak", "rc_partition", "rc_spec_source", "rc_render_adaptive",
 ]
 
 
@@ -141,6 +145,8 @@ def load(path: str | None = None) -> C.CDLL:
     lib.rc_upload_scene.argtypes = [vp, C.POINTER(rc_scene)]
     lib.rc_set_camera.argtypes = [vp, C.POINTER(rc_camera)]
     lib.rc_render.argtypes = [vp, C.POINTER(rc_params), C.POINTER(C.c_double), C.POINTER(C.c_int32)]
+    lib.rc_render_adaptive.argtypes = [vp, C.POINTER(rc_params), C.POINTER(rc_adaptive), C.POINTER(C.c_double),
+                                       C.POINTER(C.c_int32), C.POINTER(C.c_double), C.POINTER(C.c_int32)]
     lib.rc_render_tiles_into.argtypes = [vp, C.POINTER(rc_params), vp, C.POINTER(C.c_int32)]
     lib.rc_shared_alloc.argtypes = [vp, C.c_uint64, C.POINTER(vp), C.POINTER(C.c_uint8)]
     lib.rc_shared_open.argtypes = [vp, C.POINTER(C.c_uint8), C.POINTER(vp)]

@@ -106,9 +106,21 @@ struct DeviceState {
     DevBuf<double> pp_in, pp_mapped;   // rc_postprocess scratch (kept between calls)
     DevBuf<uint8_t> pp_rgba;
     DevBuf<unsigned long long> counter;
+    // rc_render_adaptive, per pixel: still tracing, samples traced, the last round's sum of y^2, running sum of y^2, error
+    DevBuf<uint8_t> ad_active;
+    DevBuf<int> ad_spp;
+    DevBuf<float> ad_m2;
+    DevBuf<double> ad_s2, ad_err;
     WavefrontState wf;
     std::map<std::string, SpecKernel> spec_cache;   // scene-specialised kernels loaded on this device
     int sm_count = 0, clock_khz = 0;
+};
+
+// One round of rc_render_adaptive: the samples [s_begin, s_end) of the pixels flagged in `active`
+struct AdaptiveRound {
+    const uint8_t* active;
+    float* round_m2;
+    int s_begin, s_end;
 };
 
 }  // namespace
@@ -139,13 +151,16 @@ struct rc_ctx {
     int mats_mask = 0xF;         // material kinds the scene uses
     int prims_mask = 0xF;        // primitive kinds the scene uses (bit RT_PRIM_*; moving spheres count as spheres)
     std::string spec_source;     // generated source of the scene-specialised kernel ("" = not generated yet)
-    int spec_rounds = 10;        // Philox rounds spec_source was generated for
+    std::string spec_source_moments;   // the same kernel with second moments, for adaptive rounds ("" = not generated yet)
+    int spec_rounds = 10;        // Philox rounds spec_source and spec_source_moments were generated for
     bool spread_stores = false;  // set by rc_render_frame for a sample-split frame of several ranks (see trace_share)
     std::vector<LbvhObject> objects, objects_next;   // top-level objects of the uploaded scene (rc_build_lbvh)
     std::vector<int> prim_order;       // device primitive i = uploaded primitive prim_order[i] (empty: identity)
     bool lbvh = false;
     bool overwrite = false;            // set for the duration of rc_render_tiles_into
     float final_scale = 0.0f;          // set for the duration of rc_render_frame (KParams::final_scale)
+    const AdaptiveRound* adaptive = nullptr;   // set for each round of rc_render_adaptive, which also owns the call's
+                                               // start event and segment counter
     std::vector<rc_frame*> frames;     // rc_frame_create / rc_frame_open
     bool stats_pending = false;        // the last render's time / counters have not been read back yet
     std::vector<void*> shared_owned, shared_opened;   // rc_shared_alloc / rc_shared_open
@@ -337,9 +352,23 @@ int launch_mega_mode(const KParams& kp, float* accum, int sampler, int rounds, i
     return RC_OK;
 }
 
-int launch_mega(int mode, bool tex, const KParams& kp, float* accum, int sampler, int rounds, int blocks, size_t smem, cudaStream_t st) {
-#define RC_MODE(M) (tex ? launch_mega_mode<M, true>(kp, accum, sampler, rounds, blocks, smem, st) \
-                        : launch_mega_mode<M, false>(kp, accum, sampler, rounds, blocks, smem, st))
+// one adaptive round: the direct sampler and 10 Philox rounds only
+template <int MODE, bool TEX>
+int launch_moments_mode(const KParams& kp, float* accum, int blocks, size_t smem, cudaStream_t st, const uint8_t* active, float* round_m2) {
+    int rc = set_smem(megakernel_moments<MODE, TEX>, smem);
+    if (rc != RC_OK) return rc;
+    megakernel_moments<MODE, TEX><<<blocks, RT_BLOCK, smem, st>>>(kp, accum, active, round_m2);
+    CUDA_TRY(cudaGetLastError());
+    return RC_OK;
+}
+
+// active != NULL: an adaptive round (megakernel_moments)
+int launch_mega(int mode, bool tex, const KParams& kp, float* accum, int sampler, int rounds, int blocks, size_t smem, cudaStream_t st,
+                const uint8_t* active = nullptr, float* round_m2 = nullptr) {
+#define RC_MODE(M) (!active ? (tex ? launch_mega_mode<M, true>(kp, accum, sampler, rounds, blocks, smem, st)          \
+                                   : launch_mega_mode<M, false>(kp, accum, sampler, rounds, blocks, smem, st))        \
+                             : (tex ? launch_moments_mode<M, true>(kp, accum, blocks, smem, st, active, round_m2)     \
+                                    : launch_moments_mode<M, false>(kp, accum, blocks, smem, st, active, round_m2)))
     switch (mode) {
     case RT_MODE_CONST_LINEAR: return RC_MODE(RT_MODE_CONST_LINEAR);
     case RT_MODE_SMEM_BVH: return RC_MODE(RT_MODE_SMEM_BVH);
@@ -426,14 +455,14 @@ int trace_share(rc_ctx* ctx, const rc_params* p, float* accum0, const volatile i
         DeviceState& d = ctx->devs[k];
         CUDA_TRY(cudaSetDevice(d.device));
         if (k == 0) {
-            CUDA_TRY(cudaEventRecord(d.ev0, d.stream));
+            if (!ctx->adaptive) CUDA_TRY(cudaEventRecord(d.ev0, d.stream));
             // fork: whatever device 0's stream holds so far — the zero-fill of the buffer the other devices are about
             // to store into, the previous frame's finalize that still reads it — happens before any of them starts
             if (n_dev > 1) CUDA_TRY(cudaEventRecord(d.ev_traced, d.stream));
         } else {
             CUDA_TRY(cudaStreamWaitEvent(d.stream, ctx->devs[0].ev_traced, 0));
         }
-        CUDA_TRY(cudaMemsetAsync(d.counter.p, 0, sizeof(unsigned long long), d.stream));
+        if (!ctx->adaptive) CUDA_TRY(cudaMemsetAsync(d.counter.p, 0, sizeof(unsigned long long), d.stream));
     }
     // A cancel flag does not change how the frame is launched (one launch per device, sliced if need be): every CTA
     // reads a word in its device's memory before it starts, and this call relays the caller's flag to that word — a
@@ -472,6 +501,12 @@ int trace_share(rc_ctx* ctx, const rc_params* p, float* accum0, const volatile i
         float* accum = (k == 0 || direct) ? accum0 : d.accum.p;
         kp.overwrite = ctx->overwrite ? 1 : 0;
         kp.final_scale = ctx->final_scale;
+        const uint8_t* active = nullptr;
+        float* round_m2 = nullptr;
+        if (ctx->adaptive) {
+            kp.s_begin = ctx->adaptive->s_begin; kp.s_end = ctx->adaptive->s_end;
+            active = ctx->adaptive->active; round_m2 = ctx->adaptive->round_m2;
+        }
         if (kp.n_tiles == 0 || kp.s_end <= kp.s_begin) { if (relay) CUDA_TRY(cudaEventRecord(d.ev_traced, d.stream)); continue; }
         if (p->variant == RC_VARIANT_WAVEFRONT) {
             if (kp.has_motion && rounds != 10) return fail(RC_ERR_INVALID, "the wavefront variant traces moving spheres with 10 Philox rounds only");
@@ -490,11 +525,14 @@ int trace_share(rc_ctx* ctx, const rc_params* p, float* accum0, const volatile i
             std::string err;
             if (!spec_load_api((const void*)&rc_abi_version)) err = spec_api().err;
             else {
-                if (ctx->spec_source.empty() || ctx->spec_rounds != rounds) {
-                    ctx->spec_source = spec_generate(ctx->kp, ctx->has_textures, ctx->mats_mask, ctx->mode, ctx->prims_mask, ctx->instanced, rounds);
+                if (ctx->spec_rounds != rounds) { ctx->spec_source.clear(); ctx->spec_source_moments.clear(); }
+                std::string& source = ctx->adaptive ? ctx->spec_source_moments : ctx->spec_source;
+                if (source.empty()) {
+                    source = spec_generate(ctx->kp, ctx->has_textures, ctx->mats_mask, ctx->mode, ctx->prims_mask, ctx->instanced, rounds,
+                                           ctx->adaptive != nullptr);
                     ctx->spec_rounds = rounds;
                 }
-                spec = spec_build(d.spec_cache, ctx->spec_source, err, ++ctx->spec_clock);
+                spec = spec_build(d.spec_cache, source, err, ++ctx->spec_clock);
             }
             if (!spec && p->specialize == 1) return fail(RC_ERR_STATE, "scene specialisation failed: " + err);
         } else if (p->specialize == 1) {
@@ -506,7 +544,7 @@ int trace_share(rc_ctx* ctx, const rc_params* p, float* accum0, const volatile i
         kp.slices = 1;
         kp.slice_buf = nullptr;
         kp.slice_halving = 0;
-        {
+        if (!ctx->adaptive) {   // (adaptive rounds run unsliced: the round's moments are stored per pixel by the kernel)
             const long long want = 8LL * d.sm_count * 10;
             long long sl = (want + kp.n_tiles - 1) / kp.n_tiles;
             if (sl > (s1 - s0) / 16) sl = (s1 - s0) / 16;
@@ -534,12 +572,13 @@ int trace_share(rc_ctx* ctx, const rc_params* p, float* accum0, const volatile i
         {
             int rc = RC_ERR_CUDA;
             if (spec) {
-                rc = spec_launch(spec, kp, accum, kp.n_tiles * kp.slices, ctx->smem_bytes, d.stream) == 0 ? RC_OK : RC_ERR_CUDA;
+                rc = spec_launch(spec, kp, accum, kp.n_tiles * kp.slices, ctx->smem_bytes, d.stream, active, round_m2) == 0 ? RC_OK : RC_ERR_CUDA;
                 if (rc == RC_OK) used_spec = true;
                 else if (p->specialize == 1) return fail(rc, "launch of the scene-specialised kernel failed");
             }
             if (rc != RC_OK)   // no specialised kernel, or (specialize == 2) it could not be launched: the precompiled one
-                rc = launch_mega(ctx->mode, ctx->has_textures, kp, accum, p->sampler, rounds, kp.n_tiles * kp.slices, ctx->smem_bytes, d.stream);
+                rc = launch_mega(ctx->mode, ctx->has_textures, kp, accum, p->sampler, rounds, kp.n_tiles * kp.slices, ctx->smem_bytes, d.stream,
+                                 active, round_m2);
             if (rc != RC_OK) return rc;
             ++launches;
             if (kp.slices > 1) {
@@ -1129,6 +1168,7 @@ int rc_destroy(rc_ctx* ctx) {
         free_scene(d);
         free_tables(d);
         d.accum.release(); d.slice_buf.release(); d.out64.release(); d.counter.release(); d.cancel_word.release();
+        d.ad_active.release(); d.ad_spp.release(); d.ad_m2.release(); d.ad_s2.release(); d.ad_err.release();
         if (d.cancel_stream) cudaStreamDestroy(d.cancel_stream);
         d.pp_in.release(); d.pp_mapped.release(); d.pp_rgba.release();
         if (d.ev_traced) cudaEventDestroy(d.ev_traced);
@@ -1179,6 +1219,7 @@ int rc_upload_scene(rc_ctx* ctx, const rc_scene* s) {
     ctx->mats_mask = t.mats_mask;
     ctx->prims_mask = t.prims_mask;
     ctx->spec_source.clear();
+    ctx->spec_source_moments.clear();
     ctx->aov.n_prims = s->n_prims; ctx->aov.n_nodes = s->n_nodes;
     // top-level objects = runs of primitives that share an object id (id >> 3; a Box's six sides) and a stored Aabb
     ctx->objects.clear();
@@ -1295,6 +1336,7 @@ int rc_set_camera(rc_ctx* ctx, const rc_camera* c) {
     // the specialised source depends on the camera (lens or pinhole; which pairs of opposite walls enclose it):
     // regenerate it — the text is the cache key, so an unchanged text costs no recompilation
     ctx->spec_source.clear();
+    ctx->spec_source_moments.clear();
     ctx->kp.lens_enabled = c->lens_radius != 0.0;
     DevCamera<double>& g = ctx->aov.cam;
     g.origin = v3d(c->origin); g.upper_left_corner = v3d(c->upper_left_corner); g.right = v3d(c->right); g.up = v3d(c->up);
@@ -1567,6 +1609,76 @@ int rc_render(rc_ctx* ctx, const rc_params* p, double* out_rgb, const volatile i
     return RC_OK;
 }
 
+int rc_render_adaptive(rc_ctx* ctx, const rc_params* p, const rc_adaptive* a, double* out_rgb, int32_t* out_spp, double* out_err,
+                       const volatile int32_t* cancel) {
+    if (!ctx || !a || !out_rgb) return fail(RC_ERR_INVALID, "ctx, adaptive or out_rgb is NULL");
+    int rc = check_params(p);
+    if (rc != RC_OK) return rc;
+    if (ctx->devs.size() != 1 || p->world > 1) return fail(RC_ERR_INVALID, "adaptive rendering needs a one-device context and world <= 1");
+    if (p->variant != RC_VARIANT_MEGAKERNEL || p->sampler != RC_SAMPLER_DIRECT || (p->rng_rounds != 0 && p->rng_rounds != 10))
+        return fail(RC_ERR_INVALID, "adaptive rendering needs the megakernel, the direct sampler and 10 Philox rounds");
+    if (p->specialize == 1 && p->fixed_jitter) return fail(RC_ERR_INVALID, "specialize = 1 needs fixed_jitter = 0");
+    if (a->min_samples < 2 || a->min_samples > p->samples) return fail(RC_ERR_INVALID, "min_samples must be >= 2 and <= samples");
+    if (!(a->threshold >= 0.0) || !std::isfinite(a->threshold)) return fail(RC_ERR_INVALID, "threshold must be finite and >= 0");
+    if (!ctx->has_scene || !ctx->has_camera) return fail(RC_ERR_STATE, "upload a scene and set a camera first");
+    if (cancelled(cancel)) return fail(RC_ERR_CANCELLED, "cancel flag set before the render started");
+    DeviceState& d = ctx->devs[0];
+    CUDA_TRY(cudaSetDevice(d.device));
+    const size_t n_pix = (size_t)p->width * p->height, n = n_pix * 3;
+    CUDA_TRY(d.ad_active.reserve(n_pix));
+    CUDA_TRY(d.ad_spp.reserve(n_pix));
+    CUDA_TRY(d.ad_m2.reserve(n_pix));
+    CUDA_TRY(d.ad_s2.reserve(n_pix));
+    CUDA_TRY(d.ad_err.reserve(n_pix));
+    CUDA_TRY(d.out64.resize(n));
+    // the call's start: the rounds add to one segment counter and are timed together (trace_share leaves both alone)
+    CUDA_TRY(cudaEventRecord(d.ev0, d.stream));
+    CUDA_TRY(cudaMemsetAsync(d.counter.p, 0, sizeof(unsigned long long), d.stream));
+    rc = ensure_accum(ctx, p, true);
+    if (rc != RC_OK) return rc;
+    const unsigned grid = (unsigned)((n_pix + 255) / 256);
+    adaptive_init_kernel<<<grid, 256, 0, d.stream>>>(d.ad_active.p, d.ad_spp.p, d.ad_s2.p, d.ad_err.p, n_pix, a->min_samples);
+    CUDA_TRY(cudaGetLastError());
+    uint64_t launches = 1;
+    int specialized = 0;
+    // every pixel still active after round r has traced the same samples, so a round is one sample range for all
+    for (int lo = 0, hi = a->min_samples;; lo = hi, hi = (int)std::min(2LL * hi, (long long)p->samples)) {
+        const AdaptiveRound round{d.ad_active.p, d.ad_m2.p, lo, hi};
+        bool was_cancelled = false;
+        ctx->adaptive = &round;
+        rc = trace_share(ctx, p, d.accum.p, cancel, was_cancelled);
+        ctx->adaptive = nullptr;
+        if (rc != RC_OK) return rc;
+        if (was_cancelled) return RC_OK;   // a cancelled render writes nothing, cpu.rs:55-62
+        launches += ctx->stats.kernel_launches;
+        specialized = ctx->stats.specialized;
+        adaptive_test_kernel<<<grid, 256, 0, d.stream>>>(d.accum.p, d.ad_m2.p, d.ad_s2.p, d.ad_active.p, d.ad_spp.p, d.ad_err.p, n_pix,
+                                                         p->samples, a->threshold);
+        CUDA_TRY(cudaGetLastError());
+        ++launches;
+        if (hi == p->samples) break;
+        if (cancelled(cancel)) return RC_OK;
+    }
+    finalize_spp_to_f64_kernel<<<(unsigned)((n + 255) / 256), 256, 0, d.stream>>>(d.accum.p, d.ad_spp.p, d.out64.p, n);
+    CUDA_TRY(cudaGetLastError());
+    ++launches;
+    rc = finish_stats(ctx, p);
+    if (rc != RC_OK) return rc;
+    std::vector<int32_t> spp_host;
+    int32_t* spp = out_spp;
+    if (!spp) { spp_host.resize(n_pix); spp = spp_host.data(); }
+    CUDA_TRY(cudaMemcpyAsync(out_rgb, d.out64.p, n * sizeof(double), cudaMemcpyDeviceToHost, d.stream));
+    CUDA_TRY(cudaMemcpyAsync(spp, d.ad_spp.p, n_pix * sizeof(int32_t), cudaMemcpyDeviceToHost, d.stream));
+    if (out_err) CUDA_TRY(cudaMemcpyAsync(out_err, d.ad_err.p, n_pix * sizeof(double), cudaMemcpyDeviceToHost, d.stream));
+    CUDA_TRY(cudaStreamSynchronize(d.stream));
+    uint64_t samples = 0;
+    for (size_t i = 0; i < n_pix; ++i) samples += (uint64_t)spp[i];
+    ctx->stats.samples = samples;
+    ctx->stats.kernel_launches = launches;
+    ctx->stats.specialized = specialized;
+    return RC_OK;
+}
+
 int rc_render_preview(rc_ctx* ctx, const rc_params* p, int32_t scale_w, int32_t scale_h, double* out_rgb,
                       const volatile int32_t* cancel) {
     if (!ctx || !out_rgb) return fail(RC_ERR_INVALID, "ctx or out_rgb is NULL");
@@ -1714,6 +1826,7 @@ int rc_build_lbvh(rc_ctx* ctx) {
     ctx->mode = bvh_bytes + perlin_bytes <= RC_SMEM_STAGE_LIMIT ? RT_MODE_SMEM_BVH : RT_MODE_GLOBAL_BVH;
     ctx->smem_bytes = perlin_bytes + (ctx->mode == RT_MODE_SMEM_BVH ? bvh_bytes : 0);
     ctx->spec_source.clear();
+    ctx->spec_source_moments.clear();
     ctx->lbvh = true;
     CUDA_TRY(cudaSetDevice(ctx->devs[0].device));
     return RC_OK;

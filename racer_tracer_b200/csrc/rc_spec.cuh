@@ -113,10 +113,23 @@ inline std::string spec_float(float v) {
     return s + "f";
 }
 
+// Entry point of a specialised translation unit: the plain megakernel, or (moments) the one of the adaptive rounds.
+// The two are separate sources, hence separate modules in the cache; the plain text is what it always was.
+inline std::string spec_entry(const char* mode, int rounds, bool tex, bool moments) {
+    std::ostringstream o;
+    o << "extern \"C\" __global__ void __launch_bounds__(RT_BLOCK, RT_MIN_BLOCKS)\n"
+         "spec_megakernel(const __grid_constant__ KParams P, float* __restrict__ accum"
+      << (moments ? ", const uint8_t* __restrict__ active, float* __restrict__ round_m2" : "") << ") {\n"
+         "    extern __shared__ __align__(16) unsigned char smem[];\n"
+         "    megakernel_body<" << mode << ", 0, " << rounds << ", " << (tex ? "true" : "false") << (moments ? ", true" : "")
+      << ">(P, accum, smem" << (moments ? ", active, round_m2" : "") << ");\n}\n";
+    return o.str();
+}
+
 // Source of the specialised translation unit for a scene already laid out in KParams
 // (type-sorted constant-bank table).
 inline std::string spec_generate(const KParams& kp, bool tex, int mats_mask, int mode = RT_MODE_CONST_LINEAR, int prims_mask_all = 0xF,
-                                 bool instanced = false, int rounds = 10) {
+                                 bool instanced = false, int rounds = 10, bool moments = false) {
     std::ostringstream o;
     if (mode != RT_MODE_CONST_LINEAR) {
         // BVH paths: the tables stay in memory; what is compiled in is which kinds of primitive, material, wrapper,
@@ -136,11 +149,7 @@ inline std::string spec_generate(const KParams& kp, bool tex, int mats_mask, int
         o << "#define RT_SPEC_MATS " << mats_mask << "\n";
         o << "#define RT_FIXED_JITTER(P) 0\n";
         o << "#include \"rt_kernels.cuh\"\n";
-        o << "extern \"C\" __global__ void __launch_bounds__(RT_BLOCK, RT_MIN_BLOCKS)\n"
-             "spec_megakernel(const __grid_constant__ KParams P, float* __restrict__ accum) {\n"
-             "    extern __shared__ __align__(16) unsigned char smem[];\n"
-             "    megakernel_body<" << (mode == RT_MODE_SMEM_BVH ? "RT_MODE_SMEM_BVH" : "RT_MODE_GLOBAL_BVH") << ", 0, " << rounds << ", "
-          << (tex ? "true" : "false") << ">(P, accum, smem);\n}\n";
+        o << spec_entry(mode == RT_MODE_SMEM_BVH ? "RT_MODE_SMEM_BVH" : "RT_MODE_GLOBAL_BVH", rounds, tex, moments);
         return o.str();
     }
     // primitive kinds present, background, regeneration batching: known before the headers are read
@@ -487,10 +496,7 @@ inline std::string spec_generate(const KParams& kp, bool tex, int mats_mask, int
     o << "#define RT_HAS_MOTION " << (any_motion ? 1 : 0) << "\n";
     o << "#define RT_FIXED_JITTER(P) 0\n";   // renders with fixed jitter (parity checks) use the precompiled kernels
     o << "#include \"rt_kernels.cuh\"\n";
-    o << "extern \"C\" __global__ void __launch_bounds__(RT_BLOCK, RT_MIN_BLOCKS)\n"
-         "spec_megakernel(const __grid_constant__ KParams P, float* __restrict__ accum) {\n"
-         "    extern __shared__ __align__(16) unsigned char smem[];\n"
-         "    megakernel_body<RT_MODE_CONST_LINEAR, 0, " << rounds << ", " << (tex ? "true" : "false") << ">(P, accum, smem);\n}\n";
+    o << spec_entry("RT_MODE_CONST_LINEAR", rounds, tex, moments);
     return o.str();
 }
 
@@ -568,9 +574,11 @@ inline void spec_release(std::map<std::string, SpecKernel>& cache) {
     cache.clear();
 }
 
-inline int spec_launch(SpecKernel* k, const KParams& kp, float* accum, int blocks, size_t smem, cudaStream_t st) {
+// `active` / `round_m2`: the two extra arguments of a moments entry point (spec_entry), NULL for the plain one
+inline int spec_launch(SpecKernel* k, const KParams& kp, float* accum, int blocks, size_t smem, cudaStream_t st,
+                       const uint8_t* active = nullptr, float* round_m2 = nullptr) {
     SpecApi& a = spec_api();
     KParams p = kp;
-    void* args[2] = {&p, &accum};
+    void* args[4] = {&p, &accum, &active, &round_m2};
     return a.cuLaunchKernel(k->function, (unsigned)blocks, 1, 1, RT_BLOCK, 1, 1, (unsigned)smem, (void*)st, args, nullptr);
 }

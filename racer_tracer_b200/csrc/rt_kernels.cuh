@@ -345,13 +345,32 @@ RT_D bool shade_hit(const KParams& P, const TexCtx& X, const Scene& S, const Rng
 #define RT_PHILOX_LATE 0    // 1: the segment's block is drawn after the closest hit in the source (ptxas schedules it either way)
 #endif
 
-template <int MODE, int SAMPLER, int ROUNDS, bool TEX>
-RT_D void megakernel_body(const KParams& P, float* __restrict__ accum, unsigned char* smem) {
-    __shared__ float steal_parked[RT_STEAL ? 3 * RT_BLOCK : 1];   // per lane of the CTA: sums other lanes traced for its pixel
+// channel mean of the radiance a * b that a path adds where it ends
+RT_D float radiance_y(const vec3f& a, const vec3f& b) { return (a.x * b.x + a.y * b.y + a.z * b.z) * (1.0f / 3.0f); }
+
+// MOMENTS (adaptive rounds, rc_render_adaptive): only the pixels flagged in `active` trace [s_begin, s_end); every lane
+// also sums y^2 of each sample it traces (y = channel mean of the sample's radiance) and the pixel's total goes to
+// round_m2.  The launch is unsliced.  Without MOMENTS the kernel is exactly the plain one.  (The two per-pixel buffers
+// are kernel arguments of their own, not KParams fields: a larger KParams would move every kernel argument behind it.)
+template <int MODE, int SAMPLER, int ROUNDS, bool TEX, bool MOMENTS = false>
+RT_D void megakernel_body(const KParams& P, float* __restrict__ accum, unsigned char* smem,
+                          const uint8_t* __restrict__ active_px = nullptr, float* __restrict__ round_m2 = nullptr) {
+    constexpr int PARKED = MOMENTS ? 4 : 3;   // floats parked per lane: the three sums (and the second moment)
+    __shared__ float steal_parked[RT_STEAL ? PARKED * RT_BLOCK : 1];   // per lane of the CTA: sums other lanes traced for its pixel
     // A render the host may cancel (interactive.rs:236-251 always passes a cancel event): CTAs that have not started
     // when the flag is raised do nothing, so a cancelled frame drains in the time of the CTAs already running.
     if (P.cancel_flag != nullptr &&
         __syncthreads_or(threadIdx.x == 0 && *reinterpret_cast<const volatile int*>(P.cancel_flag) != 0)) return;
+    bool active = true;   // (MOMENTS) this lane's pixel traces samples in this round
+    if constexpr (MOMENTS) {
+        // a tile without an active pixel leaves before it stages the scene: later rounds keep the ordinary tile grid
+        const int tile = P.tile_first + (int)blockIdx.x * P.tile_stride;
+        const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
+        const int x = (tile % P.tiles_x) * RT_TILE_W + (w & 1) * 8 + (l & 7);
+        const int y = (tile / P.tiles_x) * RT_TILE_H + (w >> 1) * 4 + (l >> 3);
+        active = x < P.width && y < P.height && active_px[y * P.width + x] != 0;
+        if (!__syncthreads_or(active ? 1 : 0)) return;
+    }
     __shared__ float reg_consts[7];
     if (threadIdx.x == 0) {
         reg_consts[0] = 2.0f; reg_consts[1] = 6.283185307179586f / 16777216.0f; reg_consts[2] = 1.0f;
@@ -412,17 +431,22 @@ RT_D void megakernel_body(const KParams& P, float* __restrict__ accum, unsigned 
         vj_bits = __byte_perm(w.y, w.x, 0x0040);
     }
     int owner = lane;          // the lane of this warp whose pixel `sum` is being traced for
-    float* const parked = steal_parked + 96 * warp;
-    if (RT_STEAL) { parked[lane] = 0.0f; parked[lane + 32] = 0.0f; parked[lane + 64] = 0.0f; __syncwarp(); }
+    float* const parked = steal_parked + 32 * PARKED * warp;
+    if (RT_STEAL) {
+        parked[lane] = 0.0f; parked[lane + 32] = 0.0f; parked[lane + 64] = 0.0f;
+        if constexpr (MOMENTS) parked[lane + 96] = 0.0f;
+        __syncwarp();
+    }
 
     // Path state.  Radiance is only ever picked up where a path ENDS (escape, light, depth
     // exhaustion): lights do not scatter and nothing else emits (src/material/*.rs), so
     // ray_color's `emitted + attenuation * recurse` collapses to throughput x terminal radiance.
     vec3f sum = mk3(0.0f, 0.0f, 0.0f);
+    float m2 = 0.0f;           // (MOMENTS) sum of y^2 over the samples in `sum`: one path adds radiance once, where it ends
     vec3f o = mk3(0.0f, 0.0f, 0.0f), d = o, T = o;
     const vec3f T_ONE = mk3(1.0f, 1.0f, 1.0f);
     float time = 0.0f;         // Ray::time of the path (scattered rays inherit it, lambertian.rs:36 etc.)
-    int s = valid ? s_first : s_last;
+    int s = valid && active ? s_first : s_last;   // a pixel with nothing to trace starts idle (and may steal)
     // > 0: this lane is on a path that may still trace that many segments; 0: no path.  A float (max_depth <= 63
     // is exact): counting down and the "budget spent" weight are then FADD / FADD.SAT on the FMA pipe instead
     // of integer add + compare + select on the ALU pipe, which is the saturated one in this kernel.
@@ -436,6 +460,7 @@ RT_D void megakernel_body(const KParams& P, float* __restrict__ accum, unsigned 
     if (P.max_depth <= 0) {    // renderer.rs:48-56: depth 0 is white, for every sample
         const float n = (float)(s_last - s);
         sum = mk3(n, n, n);
+        if constexpr (MOMENTS) m2 = n;   // y = 1
         s = s_last;
     }
 
@@ -455,6 +480,7 @@ RT_D void megakernel_body(const KParams& P, float* __restrict__ accum, unsigned 
                         bg = background_color(P, d);
                     } else bg = mk3(P.bg_a.x, P.bg_a.y, P.bg_a.z);
                     sum = mk3(fmaf(T_ONE.x, bg.x, sum.x), fmaf(T_ONE.y, bg.y, sum.y), fmaf(T_ONE.z, bg.z, sum.z));
+                    if constexpr (MOMENTS) { const float y = radiance_y(T_ONE, bg); m2 = fmaf(y, y, m2); }
                 }
             }
             s = s_last;
@@ -516,6 +542,7 @@ RT_D void megakernel_body(const KParams& P, float* __restrict__ accum, unsigned 
             if (!RT_SPEC_BG_BLACK) {
                 const vec3f bg = background_color(P, d);
                 sum = mk3(fmaf(T.x, bg.x, sum.x), fmaf(T.y, bg.y, sum.y), fmaf(T.z, bg.z, sum.z));
+                if constexpr (MOMENTS) { const float y = radiance_y(T, bg); m2 = fmaf(y, y, m2); }
             }
             depth_left = 0.0f;
         } else {
@@ -527,6 +554,7 @@ RT_D void megakernel_body(const KParams& P, float* __restrict__ accum, unsigned 
             else { PtrScene S; S.prims = L.prims; S.nodes = L.nodes; S.inst = P.instances; S.ref_aabb = P.ref_aabb; cont = shade_hit<SAMPLER, ROUNDS, TEX>(P, X, S, R, prim, r, t, seg, rnd, o, d, T, X_end); }
             if (!cont) {                 // absorbed (X_end = 0) or a light (X_end = emission)
                 sum = sum + T * X_end;
+                if constexpr (MOMENTS) { const float y = radiance_y(T, X_end); m2 = fmaf(y, y, m2); }
                 depth_left = 0.0f;
             } else {
                 last_prim = prim;
@@ -535,6 +563,7 @@ RT_D void megakernel_body(const KParams& P, float* __restrict__ accum, unsigned 
                 const float w = __saturatef(1.0f - depth_left);   // 1 when the budget is spent (depth_left == 0), else 0
                 fma2_bcast(w, T.x, T.y, sum.x, sum.y, sum.x, sum.y);
                 sum.z = fmaf(w, T.z, sum.z);
+                if constexpr (MOMENTS) { const float y = radiance_y(T_ONE, T); m2 = fmaf(w, y * y, m2); }   // w is 0 or 1
             }
         }
         };
@@ -569,6 +598,7 @@ RT_D void megakernel_body(const KParams& P, float* __restrict__ accum, unsigned 
                         // what this lane has summed belongs to `owner`'s pixel: park it (only this lane is active here)
                         parked[owner] += sum.x; parked[owner + 32] += sum.y; parked[owner + 64] += sum.z;
                         sum = mk3(0.0f, 0.0f, 0.0f);
+                        if constexpr (MOMENTS) { parked[owner + 96] += m2; m2 = 0.0f; }
                         owner = v_owner;
                         pc.pixel = v_pixel; pc.dir0 = mk3(vx, vy, vz);
                         R.pixel = v_pixel;
@@ -606,13 +636,24 @@ RT_D void megakernel_body(const KParams& P, float* __restrict__ accum, unsigned 
         while (pending) {
             const int l = __ffs(pending) - 1;
             pending &= pending - 1;
-            if (lane == l) { parked[owner] += sum.x; parked[owner + 32] += sum.y; parked[owner + 64] += sum.z; }
+            if (lane == l) {
+                parked[owner] += sum.x; parked[owner + 32] += sum.y; parked[owner + 64] += sum.z;
+                if constexpr (MOMENTS) parked[owner + 96] += m2;
+            }
             __syncwarp();
         }
-        if (owner != lane) sum = mk3(0.0f, 0.0f, 0.0f);
+        if (owner != lane) { sum = mk3(0.0f, 0.0f, 0.0f); m2 = 0.0f; }
         sum = mk3(sum.x + parked[lane], sum.y + parked[lane + 32], sum.z + parked[lane + 64]);
+        if constexpr (MOMENTS) m2 += parked[lane + 96];
     }
-    if (P.slices > 1) {
+    if constexpr (MOMENTS) {
+        // unsliced, added to the running sums; nothing to write for a pixel outside this round
+        if (valid && active) {
+            float* a = accum + 3 * (size_t)own_pixel;
+            a[0] += sum.x; a[1] += sum.y; a[2] += sum.z;
+            round_m2[own_pixel] = m2;
+        }
+    } else if (P.slices > 1) {
         // partial sum of this slice; reduce_slices_kernel adds the slices in order (deterministic)
         float* a = P.slice_buf + 3 * ((size_t)slice * ((size_t)P.n_tiles * RT_BLOCK) + (size_t)tile_k * RT_BLOCK + threadIdx.x);
         a[0] = sum.x; a[1] = sum.y; a[2] = sum.z;
@@ -656,6 +697,41 @@ __global__ void __launch_bounds__(RT_BLOCK, MODE == RT_MODE_GLOBAL_BVH ? RT_MIN_
 megakernel_render(const __grid_constant__ KParams P, float* __restrict__ accum) {
     extern __shared__ __align__(16) unsigned char smem[];
     megakernel_body<MODE, SAMPLER, ROUNDS, TEX>(P, accum, smem);
+}
+
+// One adaptive round (rc_render_adaptive): the megakernel with second moments, over the active pixels only
+template <int MODE, bool TEX>
+__global__ void __launch_bounds__(RT_BLOCK, MODE == RT_MODE_GLOBAL_BVH ? RT_MIN_BLOCKS_GLOBAL_BVH : RT_MIN_BLOCKS)
+megakernel_moments(const __grid_constant__ KParams P, float* __restrict__ accum, const uint8_t* __restrict__ active,
+                   float* __restrict__ round_m2) {
+    extern __shared__ __align__(16) unsigned char smem[];
+    megakernel_body<MODE, 0, 10, TEX, true>(P, accum, smem, active, round_m2);
+}
+
+// After an adaptive round, for every pixel that traced it: S2 += the round's sum of y^2; S1 = the channel mean of the
+// radiance sums; the error estimate of sqrt(mean) (include/racer_cuda.h, rc_adaptive) decides whether the pixel stops
+// or doubles its sample count, up to `max_spp`.  spp holds the samples traced so far.
+__global__ void adaptive_test_kernel(const float* __restrict__ accum, const float* __restrict__ round_m2, double* __restrict__ s2,
+                                     uint8_t* __restrict__ active, int* __restrict__ spp, double* __restrict__ err,
+                                     size_t n_pixels, int max_spp, double threshold) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_pixels || !active[i]) return;
+    const int n = spp[i];
+    const double S2 = s2[i] + (double)round_m2[i];
+    const double S1 = ((double)accum[3 * i] + (double)accum[3 * i + 1] + (double)accum[3 * i + 2]) / 3.0;
+    const double mu = S1 / n, se = sqrt(fmax(0.0, (S2 - S1 * S1 / n) / (n - 1)) / n);
+    const double e = 0.5 * (sqrt(mu + se) - sqrt(fmax(mu - se, 0.0)));
+    s2[i] = S2;
+    err[i] = e;
+    if (e <= threshold || n >= max_spp) active[i] = 0;
+    else spp[i] = min(2 * n, max_spp);
+}
+
+__global__ void adaptive_init_kernel(uint8_t* __restrict__ active, int* __restrict__ spp, double* __restrict__ s2,
+                                     double* __restrict__ err, size_t n_pixels, int n0) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_pixels) return;
+    active[i] = 1; spp[i] = n0; s2[i] = 0.0; err[i] = 0.0;
 }
 
 
@@ -935,6 +1011,12 @@ __global__ void widen_kernel(const float* __restrict__ in, double* __restrict__ 
 __global__ void finalize_to_f64_kernel(const float* __restrict__ accum, double* __restrict__ rgb, size_t n, double scale) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) rgb[i] = sqrt(scale * (double)accum[i]);
+}
+
+// finalize_to_f64_kernel with each pixel's own sample count (rc_render_adaptive); n = width * height * 3
+__global__ void finalize_spp_to_f64_kernel(const float* __restrict__ accum, const int* __restrict__ spp, double* __restrict__ rgb, size_t n) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) rgb[i] = sqrt(1.0 / (double)spp[i / 3] * (double)accum[i]);
 }
 
 // ---------------------------------------------------------------------------

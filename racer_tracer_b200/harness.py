@@ -948,6 +948,22 @@ class CudaRenderer:
                                                 out.ctypes.data_as(C.POINTER(C.c_double)), cptr))
         return out
 
+    def render_adaptive(self, params: rc_params, threshold: float, min_samples: int, cancel=None):
+        """rc_render_adaptive -> (rgb (H, W, 3) float64, spp (H, W) int32, err (H, W) float64): every pixel traces
+        samples [0, n_p), n_p doubling from min_samples up to params.samples until its error estimate is <= threshold."""
+        h, w = params.height, params.width
+        rgb = np.empty((h, w, 3), dtype=np.float64)
+        spp = np.empty((h, w), dtype=np.int32)
+        err = np.empty((h, w), dtype=np.float64)
+        a = capi.rc_adaptive()
+        a.min_samples, a.threshold = min_samples, threshold
+        cptr = C.cast(C.pointer(cancel), C.POINTER(C.c_int32)) if cancel is not None else None
+        capi.check(self.lib, self.lib.rc_render_adaptive(self.ctx, C.byref(params), C.byref(a),
+                                                         rgb.ctypes.data_as(C.POINTER(C.c_double)),
+                                                         spp.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                         err.ctypes.data_as(C.POINTER(C.c_double)), cptr))
+        return rgb, spp, err
+
     def render_preview(self, params: rc_params, scale_w: int, scale_h: int, cancel=None) -> np.ndarray:
         """rc_render_preview: what CpuRendererScaled sends (cpu_scaled.rs); params = screen size + config.preview."""
         out = np.empty((params.height, params.width, 3), dtype=np.float64)

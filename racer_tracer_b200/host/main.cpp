@@ -6,6 +6,7 @@
 //
 //   racer_render --config config.yml --scene scene.yml [--width W --height H] [--samples N]
 //                [--max-depth D] [--seed S] [--preview] [--out image.png] [--image-dir DIR]
+//                [--adaptive T [--min-samples N]]   (adaptive sampling up to --samples per pixel: gpu.adaptive)
 //                [--dump-flat scene.json]      (flat tables as JSON; needs no GPU)
 #include <chrono>
 #include <cstdio>
@@ -46,6 +47,9 @@ int main(int argc, char** argv) {
     long width = 0, height = 0, samples = -1, max_depth = -1;
     unsigned long long seed = 0;
     bool have_seed = false, preview = false;
+    bool have_adaptive = false;
+    double adaptive = 0.0;
+    long min_samples = -1;
     try {
         for (int i = 1; i < argc; ++i) {
             const std::string a = argv[i];
@@ -80,6 +84,8 @@ int main(int argc, char** argv) {
             else if (a == "--max-depth") max_depth = std::atol(next().c_str());
             else if (a == "--seed") { seed = std::strtoull(next().c_str(), nullptr, 10); have_seed = true; }
             else if (a == "--preview") preview = true;
+            else if (a == "--adaptive") { adaptive = std::atof(next().c_str()); have_adaptive = true; }
+            else if (a == "--min-samples") min_samples = std::atol(next().c_str());
             else throw TracerError(TracerError::ArgumentParsingError, "Argument parsing Error: unknown argument " + a);
         }
         Config config = config_path.empty() ? Config() : Config::from_file(config_path);
@@ -88,6 +94,11 @@ int main(int argc, char** argv) {
         if (samples >= 0) (preview ? config.preview : config.render).samples = (size_t)samples;
         if (max_depth >= 0) (preview ? config.preview : config.render).max_depth = (size_t)max_depth;
         if (have_seed) config.gpu.seed = seed;
+        if (have_adaptive) { config.gpu.adaptive = true; config.gpu.adaptive_threshold = adaptive; }
+        if (min_samples >= 0) {
+            if (!config.gpu.adaptive) throw TracerError(TracerError::ArgumentParsingError, "Argument parsing Error: --min-samples needs --adaptive");
+            config.gpu.adaptive_min_samples = (int32_t)min_samples;
+        }
         if (scene_path.empty() && config.loader.kind == SceneLoaderConfig::Yml) scene_path = config.loader.path;
         if (scene_path.empty() && config.loader.kind == SceneLoaderConfig::Random) scene_path = "random";
         if (scene_path.empty() && config.loader.kind == SceneLoaderConfig::Sandbox) scene_path = "sandbox:../resources/scenes/cornell_box.yml";   // sandbox.rs:41-42

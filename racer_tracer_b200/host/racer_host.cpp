@@ -428,6 +428,11 @@ Config Config::from_file(const std::string& file) {
             if (g->has("specialize")) cfg.gpu.specialize = (int)g->at("specialize").as_int();
             if (g->has("devices") && g->at("devices").is_seq())
                 for (auto& d : g->at("devices").seq) cfg.gpu.devices.push_back((int32_t)d.as_int());
+            if (const Node* a = g->find("adaptive")) {
+                cfg.gpu.adaptive = true;
+                if (a->has("threshold")) cfg.gpu.adaptive_threshold = a->at("threshold").as_double();
+                if (a->has("min_samples")) cfg.gpu.adaptive_min_samples = (int32_t)a->at("min_samples").as_int();
+            }
         }
     } catch (const yaml_lite::ParseError& e) {
         throw TracerError(TracerError::Configuration, "Config Error (" + file + "): " + e.what());
@@ -961,7 +966,16 @@ void CudaRenderer::render(const RenderData& rd, const DataWriter<ImageBufferEven
     ImageBufferEvent ev;
     ev.rgb.resize(n);
     static_assert(sizeof(Color) == 3 * sizeof(double), "Color is three packed doubles");
-    check(rc_render(ctx_, &p, reinterpret_cast<double*>(ev.rgb.data()), rd.cancel_event), "rc_render");
+    if (gpu_.adaptive) {
+        rc_adaptive a;
+        std::memset(&a, 0, sizeof(a));
+        a.min_samples = gpu_.adaptive_min_samples;
+        a.threshold = gpu_.adaptive_threshold;
+        check(rc_render_adaptive(ctx_, &p, &a, reinterpret_cast<double*>(ev.rgb.data()), nullptr, nullptr, rd.cancel_event),
+              "rc_render_adaptive");
+    } else {
+        check(rc_render(ctx_, &p, reinterpret_cast<double*>(ev.rgb.data()), rd.cancel_event), "rc_render");
+    }
     if (rd.cancel_event && *rd.cancel_event) return;   // cancelled midway: nothing is written, cpu.rs:55-62
     ev.r = 0; ev.c = 0; ev.width = rd.image->width; ev.height = rd.image->height;   // one message for the whole image
     writer.write(std::move(ev));

@@ -72,6 +72,11 @@ struct GpuConfig {      // new optional `gpu:` block
     uint64_t seed = 0;
     int variant = RC_VARIANT_MEGAKERNEL, sampler = RC_SAMPLER_DIRECT, split = RC_SPLIT_TILES, specialize = 2;
     std::vector<int32_t> devices;
+    // optional `adaptive: {threshold, min_samples}`: the full renderer samples adaptively (rc_render_adaptive) with
+    // render.samples as the per-pixel maximum
+    bool adaptive = false;
+    double adaptive_threshold = 0.0;
+    int32_t adaptive_min_samples = 16;
 };
 struct Config {         // config.rs:183-215
     RenderConfig preview, render;

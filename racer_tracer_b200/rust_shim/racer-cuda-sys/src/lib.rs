@@ -93,6 +93,12 @@ pub struct rc_stats {
     pub n_devices: i32, pub sm_count: i32, pub sm_clock_khz: i32, pub specialized: i32,
 }
 
+/// rc_render_adaptive: samples every pixel gets before its first test, and the error estimate that stops it.
+#[repr(C)] #[derive(Clone, Copy)]
+pub struct rc_adaptive {
+    pub min_samples: i32, pub reserved: i32, pub threshold: f64,
+}
+
 #[repr(C)] #[derive(Clone, Copy)]
 pub struct rc_tone_map {
     pub type_: i32, pub reserved: i32, pub max_white: f64, pub hable: [f64; 6], pub exposure_bias: f64,
@@ -115,6 +121,8 @@ extern "C" {
     pub fn rc_build_lbvh(ctx: *mut rc_ctx) -> c_int;
     pub fn rc_get_bvh(ctx: *mut rc_ctx, nodes: *mut rc_bvh_node, node_capacity: i32, prim_order: *mut i32, prim_capacity: i32) -> c_int;
     pub fn rc_render(ctx: *mut rc_ctx, params: *const rc_params, out_rgb: *mut f64, cancel: *const i32) -> c_int;
+    pub fn rc_render_adaptive(ctx: *mut rc_ctx, params: *const rc_params, a: *const rc_adaptive, out_rgb: *mut f64, out_spp: *mut i32,
+                              out_err: *mut f64, cancel: *const i32) -> c_int;
     pub fn rc_render_preview(ctx: *mut rc_ctx, params: *const rc_params, scale_w: i32, scale_h: i32, out_rgb: *mut f64,
                              cancel: *const i32) -> c_int;
     pub fn rc_render_tiles_into(ctx: *mut rc_ctx, params: *const rc_params, d_image: *mut f32, cancel: *const i32) -> c_int;
