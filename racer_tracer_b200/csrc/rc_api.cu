@@ -116,13 +116,6 @@ struct DeviceState {
     int sm_count = 0, clock_khz = 0;
 };
 
-// One round of rc_render_adaptive: the samples [s_begin, s_end) of the pixels flagged in `active`
-struct AdaptiveRound {
-    const uint8_t* active;
-    float* round_m2;
-    int s_begin, s_end;
-};
-
 }  // namespace
 
 // One image shared by the ranks of a box (rc_frame_create / rc_frame_open): [image 0][image 1][progress words],
@@ -144,7 +137,6 @@ struct rc_ctx {
     KParams kp;             // scene part filled at upload (device pointers of device 0 patched per launch)
     AovParamsD aov;
     int mode = RT_MODE_CONST_LINEAR;
-    int preview_sw = 0, preview_sh = 0, preview_w = 0, preview_h = 0;   // set for the duration of rc_render_preview
     size_t smem_bytes = 0;
     bool has_scene = false, has_camera = false;
     bool has_textures = false;   // any primitive whose texture is not a solid colour
@@ -153,14 +145,9 @@ struct rc_ctx {
     std::string spec_source;     // generated source of the scene-specialised kernel ("" = not generated yet)
     std::string spec_source_moments;   // the same kernel with second moments, for adaptive rounds ("" = not generated yet)
     int spec_rounds = 10;        // Philox rounds spec_source and spec_source_moments were generated for
-    bool spread_stores = false;  // set by rc_render_frame for a sample-split frame of several ranks (see trace_share)
     std::vector<LbvhObject> objects, objects_next;   // top-level objects of the uploaded scene (rc_build_lbvh)
     std::vector<int> prim_order;       // device primitive i = uploaded primitive prim_order[i] (empty: identity)
     bool lbvh = false;
-    bool overwrite = false;            // set for the duration of rc_render_tiles_into
-    float final_scale = 0.0f;          // set for the duration of rc_render_frame (KParams::final_scale)
-    const AdaptiveRound* adaptive = nullptr;   // set for each round of rc_render_adaptive, which also owns the call's
-                                               // start event and segment counter
     std::vector<rc_frame*> frames;     // rc_frame_create / rc_frame_open
     bool stats_pending = false;        // the last render's time / counters have not been read back yet
     std::vector<void*> shared_owned, shared_opened;   // rc_shared_alloc / rc_shared_open
@@ -441,35 +428,56 @@ bool direct_tiles(const rc_ctx* ctx, const rc_params* p) {
     return ctx->devs.size() > 1 && p->split == RC_SPLIT_TILES && ctx->multi.peer_write_ok && p->variant == RC_VARIANT_MEGAKERNEL;
 }
 
-// Trace this context's share into each device's own accumulation buffer
-// (device 0 uses `accum0`).  Does not gather.
-int trace_share(rc_ctx* ctx, const rc_params* p, float* accum0, const volatile int32_t* cancel, bool& was_cancelled) {
+// One round of rc_render_adaptive: the samples [s_begin, s_end) of the pixels flagged in `active`
+struct AdaptiveRound {
+    const uint8_t* active;
+    float* round_m2;
+    int s_begin, s_end;
+};
+
+// What one render call asks of trace_share besides its rc_params
+struct ShareCall {
+    float* accum0;                       // device 0's destination buffer
+    const volatile int32_t* cancel;      // the caller's cancel flag (may be null)
+    bool store = false;                  // KParams::overwrite: store the pixel sums instead of adding them
+    float final_scale = 0.0f;            // KParams::final_scale
+    bool spread_stores = false;          // a sample-split rc_render_frame of several ranks: no forced tail slicing
+    int preview_sw = 0, preview_sh = 0, preview_w = 0, preview_h = 0;   // preview scale and screen size (0: no preview)
+    const AdaptiveRound* round = nullptr;   // a round of rc_render_adaptive, which owns the call's start event and
+                                            // segment counter
+};
+
+// Trace this context's share into each device's own accumulation buffer (device 0 uses `call.accum0`), then,
+// unless the render was cancelled, join or gather the other devices' pixels onto device 0.
+int trace_share(rc_ctx* ctx, const rc_params* p, const ShareCall& call, bool& was_cancelled) {
     was_cancelled = false;
     const int n_dev = (int)ctx->devs.size();
     const int world = p->world > 0 ? p->world : 1;
     const int parts = world * n_dev;
     const int rounds = p->rng_rounds ? p->rng_rounds : 10;
+    // direct tile split: every device stores its pixels into device 0's buffer (peer memory) itself
+    const bool direct = direct_tiles(ctx, p);
     uint64_t launches = 0;
     bool used_spec = false;
     for (int k = 0; k < n_dev; ++k) {
         DeviceState& d = ctx->devs[k];
         CUDA_TRY(cudaSetDevice(d.device));
         if (k == 0) {
-            if (!ctx->adaptive) CUDA_TRY(cudaEventRecord(d.ev0, d.stream));
+            if (!call.round) CUDA_TRY(cudaEventRecord(d.ev0, d.stream));
             // fork: whatever device 0's stream holds so far — the zero-fill of the buffer the other devices are about
             // to store into, the previous frame's finalize that still reads it — happens before any of them starts
             if (n_dev > 1) CUDA_TRY(cudaEventRecord(d.ev_traced, d.stream));
         } else {
             CUDA_TRY(cudaStreamWaitEvent(d.stream, ctx->devs[0].ev_traced, 0));
         }
-        if (!ctx->adaptive) CUDA_TRY(cudaMemsetAsync(d.counter.p, 0, sizeof(unsigned long long), d.stream));
+        if (!call.round) CUDA_TRY(cudaMemsetAsync(d.counter.p, 0, sizeof(unsigned long long), d.stream));
     }
     // A cancel flag does not change how the frame is launched (one launch per device, sliced if need be): every CTA
     // reads a word in its device's memory before it starts, and this call relays the caller's flag to that word — a
     // 4-byte copy on a second stream — while it waits (do_cancel per row, src/renderer/cpu.rs:55-62).  (The word used to
     // be mapped HOST memory: ten thousand CTAs per GPU then each read it over PCIe, which cost 0.7 ms per frame on one
     // GPU and 7 ms with eight processes on one host.)  The wavefront variant is not interruptible.
-    const bool relay = cancel != nullptr && p->variant == RC_VARIANT_MEGAKERNEL;
+    const bool relay = call.cancel != nullptr && p->variant == RC_VARIANT_MEGAKERNEL;
     if (relay)
         for (int k = 0; k < n_dev; ++k) {
             DeviceState& d = ctx->devs[k];
@@ -490,22 +498,20 @@ int trace_share(rc_ctx* ctx, const rc_params* p, float* accum0, const volatile i
         partition(kp, p, p->rank * n_dev + k, parts);
         // tile culling needs one ray origin per tile (no lens), primitives that stay where they are, and a linear mode
         kp.tile_cull = (!kp.lens_enabled && !kp.has_motion && !p->fixed_jitter && std::getenv("RC_NO_TILE_CULL") == nullptr) ? 1 : 0;
-        if (ctx->preview_sw > 0) {   // scaled preview: p->width/height is the block grid, u and v refer to the screen
-            kp.px_scale_x = ctx->preview_sw; kp.px_scale_y = ctx->preview_sh;
-            kp.wm1 = (float)(ctx->preview_w - 1);
-            kp.inv_wm1 = 1.0f / (float)(ctx->preview_w - 1); kp.inv_hm1 = 1.0f / (float)(ctx->preview_h - 1);
-            set_vstep(kp, ctx->preview_h);
+        if (call.preview_sw > 0) {   // scaled preview: p->width/height is the block grid, u and v refer to the screen
+            kp.px_scale_x = call.preview_sw; kp.px_scale_y = call.preview_sh;
+            kp.wm1 = (float)(call.preview_w - 1);
+            kp.inv_wm1 = 1.0f / (float)(call.preview_w - 1); kp.inv_hm1 = 1.0f / (float)(call.preview_h - 1);
+            set_vstep(kp, call.preview_h);
         }
-        // direct tile split: every device stores its pixels into device 0's buffer (peer memory) itself
-        const bool direct = n_dev > 1 && p->split == RC_SPLIT_TILES && ctx->multi.peer_write_ok && p->variant == RC_VARIANT_MEGAKERNEL;
-        float* accum = (k == 0 || direct) ? accum0 : d.accum.p;
-        kp.overwrite = ctx->overwrite ? 1 : 0;
-        kp.final_scale = ctx->final_scale;
+        float* accum = (k == 0 || direct) ? call.accum0 : d.accum.p;
+        kp.overwrite = call.store ? 1 : 0;
+        kp.final_scale = call.final_scale;
         const uint8_t* active = nullptr;
         float* round_m2 = nullptr;
-        if (ctx->adaptive) {
-            kp.s_begin = ctx->adaptive->s_begin; kp.s_end = ctx->adaptive->s_end;
-            active = ctx->adaptive->active; round_m2 = ctx->adaptive->round_m2;
+        if (call.round) {
+            kp.s_begin = call.round->s_begin; kp.s_end = call.round->s_end;
+            active = call.round->active; round_m2 = call.round->round_m2;
         }
         if (kp.n_tiles == 0 || kp.s_end <= kp.s_begin) { if (relay) CUDA_TRY(cudaEventRecord(d.ev_traced, d.stream)); continue; }
         if (p->variant == RC_VARIANT_WAVEFRONT) {
@@ -526,10 +532,10 @@ int trace_share(rc_ctx* ctx, const rc_params* p, float* accum0, const volatile i
             if (!spec_load_api((const void*)&rc_abi_version)) err = spec_api().err;
             else {
                 if (ctx->spec_rounds != rounds) { ctx->spec_source.clear(); ctx->spec_source_moments.clear(); }
-                std::string& source = ctx->adaptive ? ctx->spec_source_moments : ctx->spec_source;
+                std::string& source = call.round ? ctx->spec_source_moments : ctx->spec_source;
                 if (source.empty()) {
                     source = spec_generate(ctx->kp, ctx->has_textures, ctx->mats_mask, ctx->mode, ctx->prims_mask, ctx->instanced, rounds,
-                                           ctx->adaptive != nullptr);
+                                           call.round != nullptr);
                     ctx->spec_rounds = rounds;
                 }
                 spec = spec_build(d.spec_cache, source, err, ++ctx->spec_clock);
@@ -544,7 +550,7 @@ int trace_share(rc_ctx* ctx, const rc_params* p, float* accum0, const volatile i
         kp.slices = 1;
         kp.slice_buf = nullptr;
         kp.slice_halving = 0;
-        if (!ctx->adaptive) {   // (adaptive rounds run unsliced: the round's moments are stored per pixel by the kernel)
+        if (!call.round) {   // (adaptive rounds run unsliced: the round's moments are stored per pixel by the kernel)
             const long long want = 8LL * d.sm_count * 10;
             long long sl = (want + kp.n_tiles - 1) / kp.n_tiles;
             if (sl > (s1 - s0) / 16) sl = (s1 - s0) / 16;
@@ -554,7 +560,7 @@ int trace_share(rc_ctx* ctx, const rc_params* p, float* accum0, const volatile i
             // cost more in per-CTA set-up than they save.
             // (not for a sample-split frame of several ranks: there the kernel's own stores go to rank 0 over NVLink and
             // should be spread over the frame, not issued by reduce_slices_kernel in one burst at its end)
-            if (sl < 2 && s1 - s0 >= 512 && !ctx->spread_stores) sl = 2;
+            if (sl < 2 && s1 - s0 >= 512 && !call.spread_stores) sl = 2;
             if (const char* e = std::getenv("RC_SLICES")) sl = std::atoll(e);
             // Slice lengths: halving (n/2, n/4, .., the last two equal) from five slices on, linearly decreasing below —
             // with two or three slices the halving scheme's last slice is too long a tail.  One rank's share of the
@@ -600,7 +606,7 @@ int trace_share(rc_ctx* ctx, const rc_params* p, float* accum0, const volatile i
                 if (e == cudaErrorNotReady) done = false;
                 else if (e != cudaSuccess) return fail(RC_ERR_CUDA, std::string("cudaEventQuery: ") + cudaGetErrorString(e));
             }
-            if (!was_cancelled && cancelled(cancel)) {
+            if (!was_cancelled && cancelled(call.cancel)) {
                 was_cancelled = true;
                 for (int k = 0; k < n_dev; ++k) {
                     DeviceState& d = ctx->devs[k];
@@ -615,6 +621,17 @@ int trace_share(rc_ctx* ctx, const rc_params* p, float* accum0, const volatile i
         }
         CUDA_TRY(cudaSetDevice(ctx->devs[0].device));
     }
+    if (was_cancelled || n_dev == 1) return RC_OK;
+    auto stream_of = [&](size_t k) { return ctx->devs[k].stream; };
+    auto device_of = [&](size_t k) { return ctx->devs[k].device; };
+    if (direct) {
+        if (multi_join(ctx->multi, stream_of, device_of) != 0)
+            return fail(RC_ERR_CUDA, std::string("multi-device join failed: ") + multi_error(ctx->multi));
+        return RC_OK;
+    }
+    const int rc = multi_gather(ctx->multi, p->split, (size_t)p->width * p->height * 3, call.accum0,
+                                [&](size_t k) { return ctx->devs[k].accum.p; }, stream_of, device_of);
+    if (rc != RC_OK) return fail(rc, std::string("multi-device gather failed: ") + multi_error(ctx->multi));
     return RC_OK;
 }
 
@@ -1346,28 +1363,23 @@ int rc_set_camera(rc_ctx* ctx, const rc_camera* c) {
     return RC_OK;
 }
 
+// rc_render_accumulate (store = false) and rc_render_tiles_into (store = true) once their arguments are checked
+static int render_into(rc_ctx* ctx, const rc_params* p, float* dst, const volatile int32_t* cancel, bool store) {
+    if (!ctx->has_scene || !ctx->has_camera) return fail(RC_ERR_STATE, "upload a scene and set a camera first");
+    if (cancelled(cancel)) return fail(RC_ERR_CANCELLED, "cancel flag set before the render started");
+    int rc = ensure_accum(ctx, p, false);
+    if (rc != RC_OK) return rc;
+    bool was_cancelled = false;
+    rc = trace_share(ctx, p, ShareCall{dst, cancel, store}, was_cancelled);
+    if (rc != RC_OK) return rc;
+    return finish_stats(ctx, p);
+}
+
 int rc_render_accumulate(rc_ctx* ctx, const rc_params* p, float* d_accum, const volatile int32_t* cancel) {
     if (!ctx || !d_accum) return fail(RC_ERR_INVALID, "ctx or d_accum is NULL");
     int rc = check_params(p);
     if (rc != RC_OK) return rc;
-    if (!ctx->has_scene || !ctx->has_camera) return fail(RC_ERR_STATE, "upload a scene and set a camera first");
-    if (cancelled(cancel)) return fail(RC_ERR_CANCELLED, "cancel flag set before the render started");
-    rc = ensure_accum(ctx, p, false);
-    if (rc != RC_OK) return rc;
-    bool was_cancelled = false;
-    rc = trace_share(ctx, p, d_accum, cancel, was_cancelled);
-    if (rc != RC_OK) return rc;
-    if (!was_cancelled && ctx->devs.size() > 1 && direct_tiles(ctx, p)) {
-        if (multi_join(ctx->multi, [&](size_t k) { return ctx->devs[k].stream; }, [&](size_t k) { return ctx->devs[k].device; }) != 0)
-            return fail(RC_ERR_CUDA, std::string("multi-device join failed: ") + multi_error(ctx->multi));
-    } else if (!was_cancelled && ctx->devs.size() > 1) {
-        rc = multi_gather(ctx->multi, p->split, (size_t)p->width * p->height * 3, d_accum,
-                          [&](size_t k) { return ctx->devs[k].accum.p; },
-                          [&](size_t k) { return ctx->devs[k].stream; },
-                          [&](size_t k) { return ctx->devs[k].device; });
-        if (rc != RC_OK) return fail(rc, std::string("multi-device gather failed: ") + multi_error(ctx->multi));
-    }
-    return finish_stats(ctx, p);
+    return render_into(ctx, p, d_accum, cancel, false);
 }
 
 int rc_render_tiles_into(rc_ctx* ctx, const rc_params* p, float* d_image, const volatile int32_t* cancel) {
@@ -1377,10 +1389,7 @@ int rc_render_tiles_into(rc_ctx* ctx, const rc_params* p, float* d_image, const 
     if (p->split != RC_SPLIT_TILES || p->variant != RC_VARIANT_MEGAKERNEL)
         return fail(RC_ERR_INVALID, "rc_render_tiles_into needs the tile split and the megakernel (pixels are stored, not added)");
     if (ctx->devs.size() > 1 && !ctx->multi.peer_write_ok) return fail(RC_ERR_INVALID, "rc_render_tiles_into over several devices needs peer access");
-    ctx->overwrite = true;
-    rc = rc_render_accumulate(ctx, p, d_image, cancel);
-    ctx->overwrite = false;
-    return rc;
+    return render_into(ctx, p, d_image, cancel, true);
 }
 
 // ---- a device buffer shared by the processes of one box (CUDA IPC over NVLink / PCIe peer mappings) ----
@@ -1518,13 +1527,10 @@ int rc_render_frame(rc_ctx* ctx, const rc_params* p, rc_frame* f, const float** 
         CUDA_TRY(cudaGetLastError());
     }
     bool was_cancelled = false;
-    ctx->overwrite = true;
-    ctx->final_scale = by_samples ? 0.0f : 1.0f / (float)p->samples;   // sample split: raw sums, the square root comes after the slots are added
-    ctx->spread_stores = by_samples && world > 1;
-    rc = trace_share(ctx, p, target, cancel, was_cancelled);
-    ctx->spread_stores = false;
-    ctx->overwrite = false;
-    ctx->final_scale = 0.0f;
+    ShareCall call{target, cancel, true};
+    call.final_scale = by_samples ? 0.0f : 1.0f / (float)p->samples;   // sample split: raw sums, the square root comes after the slots are added
+    call.spread_stores = by_samples && world > 1;
+    rc = trace_share(ctx, p, call, was_cancelled);
     if (rc != RC_OK) return rc;
     if (by_samples && (long long)p->samples * (f->rank + 1) / world <= (long long)p->samples * f->rank / world) {
         // fewer samples than ranks and none for this one: its slot still holds frame n - 2's sums, and rank 0 adds it
@@ -1583,21 +1589,9 @@ int rc_render(rc_ctx* ctx, const rc_params* p, double* out_rgb, const volatile i
     rc = ensure_accum(ctx, p, true, !store);
     if (rc != RC_OK) return rc;
     bool was_cancelled = false;
-    ctx->overwrite = store;
-    rc = trace_share(ctx, p, d0.accum.p, cancel, was_cancelled);
-    ctx->overwrite = false;
+    rc = trace_share(ctx, p, ShareCall{d0.accum.p, cancel, store}, was_cancelled);
     if (rc != RC_OK) return rc;
     if (was_cancelled) return RC_OK;  // a cancelled render writes nothing, cpu.rs:55-62
-    if (ctx->devs.size() > 1 && direct_tiles(ctx, p)) {
-        if (multi_join(ctx->multi, [&](size_t k) { return ctx->devs[k].stream; }, [&](size_t k) { return ctx->devs[k].device; }) != 0)
-            return fail(RC_ERR_CUDA, std::string("multi-device join failed: ") + multi_error(ctx->multi));
-    } else if (ctx->devs.size() > 1) {
-        rc = multi_gather(ctx->multi, p->split, n, d0.accum.p,
-                          [&](size_t k) { return ctx->devs[k].accum.p; },
-                          [&](size_t k) { return ctx->devs[k].stream; },
-                          [&](size_t k) { return ctx->devs[k].device; });
-        if (rc != RC_OK) return fail(rc, std::string("multi-device gather failed: ") + multi_error(ctx->multi));
-    }
     CUDA_TRY(cudaSetDevice(d0.device));
     CUDA_TRY(d0.out64.resize(n));
     finalize_to_f64_kernel<<<(unsigned)((n + 255) / 256), 256, 0, d0.stream>>>(d0.accum.p, d0.out64.p, n, 1.0 / (double)p->samples);
@@ -1644,10 +1638,10 @@ int rc_render_adaptive(rc_ctx* ctx, const rc_params* p, const rc_adaptive* a, do
     // every pixel still active after round r has traced the same samples, so a round is one sample range for all
     for (int lo = 0, hi = a->min_samples;; lo = hi, hi = (int)std::min(2LL * hi, (long long)p->samples)) {
         const AdaptiveRound round{d.ad_active.p, d.ad_m2.p, lo, hi};
+        ShareCall call{d.accum.p, cancel};
+        call.round = &round;
         bool was_cancelled = false;
-        ctx->adaptive = &round;
-        rc = trace_share(ctx, p, d.accum.p, cancel, was_cancelled);
-        ctx->adaptive = nullptr;
+        rc = trace_share(ctx, p, call, was_cancelled);
         if (rc != RC_OK) return rc;
         if (was_cancelled) return RC_OK;   // a cancelled render writes nothing, cpu.rs:55-62
         launches += ctx->stats.kernel_launches;
@@ -1703,24 +1697,12 @@ int rc_render_preview(rc_ctx* ctx, const rc_params* p, int32_t scale_w, int32_t 
     const bool store = can_store(ctx, &q);
     rc = ensure_accum(ctx, &q, true, !store);
     if (rc != RC_OK) return rc;
-    ctx->preview_sw = scale_w; ctx->preview_sh = scale_h; ctx->preview_w = p->width; ctx->preview_h = p->height;
+    ShareCall call{d0.accum.p, cancel, store};
+    call.preview_sw = scale_w; call.preview_sh = scale_h; call.preview_w = p->width; call.preview_h = p->height;
     bool was_cancelled = false;
-    ctx->overwrite = store;
-    rc = trace_share(ctx, &q, d0.accum.p, cancel, was_cancelled);
-    ctx->overwrite = false;
-    ctx->preview_sw = ctx->preview_sh = ctx->preview_w = ctx->preview_h = 0;
+    rc = trace_share(ctx, &q, call, was_cancelled);
     if (rc != RC_OK) return rc;
     if (was_cancelled) return RC_OK;
-    if (ctx->devs.size() > 1 && direct_tiles(ctx, &q)) {
-        if (multi_join(ctx->multi, [&](size_t k) { return ctx->devs[k].stream; }, [&](size_t k) { return ctx->devs[k].device; }) != 0)
-            return fail(RC_ERR_CUDA, std::string("multi-device join failed: ") + multi_error(ctx->multi));
-    } else if (ctx->devs.size() > 1) {
-        rc = multi_gather(ctx->multi, q.split, (size_t)q.width * q.height * 3, d0.accum.p,
-                          [&](size_t k) { return ctx->devs[k].accum.p; },
-                          [&](size_t k) { return ctx->devs[k].stream; },
-                          [&](size_t k) { return ctx->devs[k].device; });
-        if (rc != RC_OK) return fail(rc, std::string("multi-device gather failed: ") + multi_error(ctx->multi));
-    }
     CUDA_TRY(cudaSetDevice(d0.device));
     preview_expand_kernel<<<(unsigned)((n_out + 255) / 256), 256, 0, d0.stream>>>(
         d0.accum.p, d0.out64.p, p->width, p->height, q.width, q.height, scale_w, scale_h, 1.0 / (double)p->samples);

@@ -141,7 +141,7 @@ int multi_nccl_init(MultiState& m, DevOf device_of) {
     return 0;
 }
 
-// Direct tile split: the other devices wrote into device 0's buffer themselves; its stream waits for them.
+// Device 0's stream waits for the other devices' (all a direct tile split needs: they stored into its buffer themselves).
 template <class StreamOf, class DevOf>
 int multi_join(MultiState& m, StreamOf stream_of, DevOf device_of) {
     for (size_t k = 1; k < m.n_dev; ++k) {
@@ -176,13 +176,8 @@ int multi_gather(MultiState& m, int split, size_t n, float* dst0, AccumOf accum_
         return 0;
     }
     // tile split: device 0 waits for the others, then pulls their buffers
-    for (size_t k = 1; k < m.n_dev; ++k) {
-        cudaSetDevice(device_of(k));
-        if (cudaEventRecord(m.done[k], stream_of(k)) != cudaSuccess) { m.err = "event record failed"; return -3; }
-    }
-    cudaSetDevice(device_of(0));
-    for (size_t k = 1; k < m.n_dev; ++k)
-        if (cudaStreamWaitEvent(stream_of(0), m.done[k], 0) != cudaSuccess) { m.err = "stream wait failed"; return -3; }
+    int rc = multi_join(m, stream_of, device_of);
+    if (rc != 0) return rc;
     PeerList pl;
     pl.n = 0;
     if (m.peer_ok) {
