@@ -526,7 +526,7 @@ int trace_share(rc_ctx* ctx, const rc_params* p, const ShareCall& call, bool& wa
         // primitive, material and wrapper compiled in or out — 48 KB of dynamic shared memory without opt-in)
         const bool spec_mode_ok = ctx->smem_bytes <= 48 * 1024 &&
                                   (ctx->mode == RT_MODE_CONST_LINEAR ||
-                                   ((ctx->mode == RT_MODE_SMEM_BVH || ctx->mode == RT_MODE_GLOBAL_BVH) && std::getenv("RC_NO_BVH_SPEC") == nullptr));
+                                   ctx->mode == RT_MODE_SMEM_BVH || ctx->mode == RT_MODE_GLOBAL_BVH);
         if (p->specialize && spec_mode_ok && p->sampler == RC_SAMPLER_DIRECT && !p->fixed_jitter) {
             std::string err;
             if (!spec_load_api((const void*)&rc_abi_version)) err = spec_api().err;

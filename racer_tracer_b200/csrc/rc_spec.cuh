@@ -16,8 +16,9 @@
 // are one rectangle test (slab pairs), the origin the kernel traces relative to (RT_SPEC_SHIFT: the most common
 // rectangle centre per axis), which literals are handed over as register constants (spec_reg_consts), the layout of
 // the staged table's rows for the hit record's plane snap (spec_snap_row), and where packed two-lane arithmetic pays
-// (operands already in register pairs).  Each of these has an environment switch that turns it off, so that the
-// equivalence tests and the measurements in DESIGN.md can be repeated (appendix there).
+// (operands already in register pairs).  Each was measured against the form it replaced (DESIGN.md §3.1).  Slab pairs
+// alone keep a switch that turns them off (RC_SPEC_NO_SLAB), because the tests trace the kernel without them as the
+// reference the slab pairs must match.
 #pragma once
 #include <cuda_runtime.h>
 #include <dlfcn.h>
@@ -140,8 +141,7 @@ inline std::string spec_generate(const KParams& kp, bool tex, int mats_mask, int
         o << "#define RT_HAS_INSTANCES " << (instanced ? 1 : 0) << "\n";
         o << "#define RT_HAS_LENS " << (kp.lens_enabled ? 1 : 0) << "\n";
         o << "#define RT_HAS_MOTION " << (kp.has_motion ? 1 : 0) << "\n";
-        if (const char* e = std::getenv("RC_MIN_BLOCKS")) o << "#define RT_MIN_BLOCKS " << std::atoi(e) << "\n";
-        else if (mode == RT_MODE_GLOBAL_BVH) o << "#define RT_MIN_BLOCKS RT_MIN_BLOCKS_GLOBAL_BVH\n";   // see rt_kernels.cuh
+        if (mode == RT_MODE_GLOBAL_BVH) o << "#define RT_MIN_BLOCKS RT_MIN_BLOCKS_GLOBAL_BVH\n";   // see rt_kernels.cuh
         o << "#include \"rt_scene.cuh\"\n";
         o << "RT_D int spec_closest_hit(const RayT<float>&, int, float&, const TexCtx&) { return -1; }   // constant-table scenes only\n";
         o << "#define RT_SPEC_REG_CONSTS 0\nRT_D void spec_reg_consts(float*) {}\n";
@@ -152,7 +152,7 @@ inline std::string spec_generate(const KParams& kp, bool tex, int mats_mask, int
         o << spec_entry(mode == RT_MODE_SMEM_BVH ? "RT_MODE_SMEM_BVH" : "RT_MODE_GLOBAL_BVH", rounds, tex, moments);
         return o.str();
     }
-    // primitive kinds present, background, regeneration batching: known before the headers are read
+    // primitive kinds present, background: known before the headers are read
     int prims_mask = 0;   // bit RT_PRIM_* (moving spheres count as spheres), instanced primitives included
     for (int i = 0; i < kp.n_prims && i < RT_MAX_CONST_PRIMS; ++i) {
         const int type = __float_as_int_host(kp.cprims[i].b.z) & 15;
@@ -170,8 +170,7 @@ inline std::string spec_generate(const KParams& kp, bool tex, int mats_mask, int
     // and ray.  Camera origin, plane constants (tests and the staged table's, from the same literal) and centres are
     // shifted; directions, distances and colours are what they were up to fp32 rounding.
     double shift[3] = {0.0, 0.0, 0.0};
-    const bool shift_ok = (prims_mask & 1) == 0 && kp.n_cobj == 0 && !tex && std::getenv("RC_SPEC_NO_SHIFT") == nullptr &&
-                          std::getenv("RC_SPEC_SELECT") == nullptr && std::getenv("RC_SPEC_INT_INDEX") == nullptr;
+    const bool shift_ok = (prims_mask & 1) == 0 && kp.n_cobj == 0 && !tex;
     if (shift_ok) o << "#define RT_SPEC_SNAP_TABLE 1\n";    // (see spec_snap_row below)
     if (shift_ok) {
         std::map<float, int> votes[3];
@@ -194,16 +193,11 @@ inline std::string spec_generate(const KParams& kp, bool tex, int mats_mask, int
     auto centre_a = [&](float c, int g) { return (float)((double)c - shift[g == 2 ? 1 : 0]); };
     auto centre_b = [&](float c, int g) { return (float)((double)c - shift[g == 0 ? 1 : 2]); };
     if (const char* e = std::getenv("RC_STEAL")) o << "#define RT_STEAL " << std::atoi(e) << "\n";
-    if (const char* e = std::getenv("RC_STEAL_MIN")) o << "#define RT_STEAL_MIN " << std::atoi(e) << "\n";
-    if (const char* e = std::getenv("RC_FIRST_TEST_RANGE")) o << "#define RT_FIRST_TEST_RANGE " << std::atoi(e) << "\n";
-    if (const char* e = std::getenv("RC_KCONST_MASK")) o << "#define RT_KCONST_MASK " << std::atoi(e) << "\n";
-    if (const char* e = std::getenv("RC_PHILOX_LATE")) o << "#define RT_PHILOX_LATE " << std::atoi(e) << "\n";
-    if (const char* e = std::getenv("RC_MIN_BLOCKS")) o << "#define RT_MIN_BLOCKS " << std::atoi(e) << "\n";
     o << "#include \"rt_scene.cuh\"\n";
     // rectangle-only scenes keep the index of the best hit as a FLOAT, so that both conditional moves of the
     // closest-hit update are predicated FFMAs on the FMA pipe (rect_closest_fma); with spheres around, the
     // index stays an integer (rect_closest)
-    const bool fidx = (prims_mask & 1) == 0 && std::getenv("RC_SPEC_SELECT") == nullptr && std::getenv("RC_SPEC_INT_INDEX") == nullptr;
+    const bool fidx = (prims_mask & 1) == 0;
     o << "RT_D int spec_closest_hit(const RayT<float>& r, int last_prim, float& best_t, const TexCtx& X) {\n";
     o << "    (void)X;\n";
     // literals handed to the kernel as register constants (TexCtx::k_spec): the plane pairs of slab pairs
@@ -211,7 +205,7 @@ inline std::string spec_generate(const KParams& kp, bool tex, int mats_mask, int
     auto reg_pair = [&](float k1, float k2) {   // -> the two operand expressions
         for (size_t j = 0; j + 1 < reg_consts.size(); j += 2)
             if (reg_consts[j] == k1 && reg_consts[j + 1] == k2) return std::make_pair("X.k_spec[" + std::to_string(j) + "]", "X.k_spec[" + std::to_string(j + 1) + "]");
-        if (reg_consts.size() + 2 > 4 || std::getenv("RC_SPEC_NO_REG_CONSTS") != nullptr) return std::make_pair(spec_float(k1), spec_float(k2));
+        if (reg_consts.size() + 2 > 4) return std::make_pair(spec_float(k1), spec_float(k2));
         reg_consts.push_back(k1); reg_consts.push_back(k2);
         const size_t j = reg_consts.size() - 2;
         return std::make_pair("X.k_spec[" + std::to_string(j) + "]", "X.k_spec[" + std::to_string(j + 1) + "]");
@@ -260,10 +254,9 @@ inline std::string spec_generate(const KParams& kp, bool tex, int mats_mask, int
     // The two in-plane coordinates of ONE rectangle, t * (d_a, d_b) + (oc_a, oc_b): one packed multiply-add when the
     // operands already sit in register pairs — the ray direction is held as (x, y), z, so that is the xy group —
     // and two scalar ones otherwise: building a pair costs a MOV per operand on the ALU pipe, which made the packed
-    // form of the xz / yz groups 2.5 - 3 instructions against 2 (RC_SPEC_PACK_ALL=1: packed everywhere, as before).
-    const bool pack_all = std::getenv("RC_SPEC_PACK_ALL") != nullptr;
+    // form of the xz / yz groups 2.5 - 3 instructions against 2.
     auto coords = [&](const std::string& t, int g, const std::string& oca, const std::string& ocb, const std::string& xa, const std::string& xb) {
-        if (g == 0 || pack_all)
+        if (g == 0)
             o << "        fma2_bcast(" << t << ", " << da[g] << ", " << db[g] << ", " << oca << ", " << ocb << ", " << xa << ", " << xb << ");\n";
         else
             o << "        " << xa << " = fmaf(" << t << ", " << da[g] << ", " << oca << "); " << xb << " = fmaf(" << t << ", " << db[g] << ", " << ocb << ");\n";
@@ -281,13 +274,11 @@ inline std::string spec_generate(const KParams& kp, bool tex, int mats_mask, int
             vb[i - begin] = rel_origin(ob[g], centre_b(c.z, g));
         }
         o << "    {\n";
-        const bool chain = std::getenv("RC_SPEC_SELECT") == nullptr;   // predicate chain (default) or candidate + select reduction
-        const bool packed = chain && std::getenv("RC_SPEC_SCALAR") == nullptr;   // FFMA2 pairs (default) or scalar arithmetic
         // Slab pair: two rectangles of this group with the same bounds (opposite walls) between which every ray of
         // the scene starts — all geometry and the pinhole lie inside the slab.  Exactly one of the two planes is
         // then in front of a ray, max(t_i, t_j), and ONE rectangle test serves both walls.
         int s0 = -1, s1 = -1;
-        if (packed && fidx && slab_scene_ok) {
+        if (fidx && slab_scene_ok) {
             const int n_axis = 2 - g;   // plane axis of the group: xy -> z, xz -> y, yz -> x
             for (int i = begin; i < end && s0 < 0; ++i)
                 for (int j = i + 1; j < end && s0 < 0; ++j) {
@@ -314,10 +305,7 @@ inline std::string spec_generate(const KParams& kp, bool tex, int mats_mask, int
         for (int i = begin; i < end; ++i)
             if (i != s0 && i != s1) rest.push_back(i);
         if (s0 >= 0) {
-            const DevPrim& p = kp.cprims[s0];
-            const DevPrim& q = kp.cprims[s1];
             o << "        float t" << s0 << ", t" << s1 << ", xa" << s0 << ", xb" << s0 << ";\n";
-            (void)p; (void)q;
             const auto kk = reg_pair(plane(s0, g), plane(s1, g));
             o << "        pair_t(" << kk.first << ", " << kk.second << ", " << on[g] << ", " << in[g] << ", t" << s0 << ", t" << s1 << ");   // planes "
               << spec_float(plane(s0, g)) << ", " << spec_float(plane(s1, g)) << "\n";
@@ -326,14 +314,10 @@ inline std::string spec_generate(const KParams& kp, bool tex, int mats_mask, int
         }
         for (size_t u = 0; u < rest.size(); ++u) {
             const int i = rest[u];
-            const DevPrim& p = kp.cprims[i];
-            const float4 c = kp.crect_bounds[g][i - begin];
-            if (packed && u + 1 < rest.size()) {   // two rectangles of this axis group per packed instruction
+            if (u + 1 < rest.size()) {   // two rectangles of this axis group per packed instruction
                 const int j = rest[u + 1];
-                const DevPrim& q = kp.cprims[j];
-                const float4 c2 = kp.crect_bounds[g][j - begin];
+                const float4 c = kp.crect_bounds[g][i - begin], c2 = kp.crect_bounds[g][j - begin];
                 o << "        float t" << i << ", t" << j << ", xa" << i << ", xa" << j << ", xb" << i << ", xb" << j << ";\n";
-                (void)q;
                 o << "        pair_t(" << spec_float(plane(i, g)) << ", " << spec_float(plane(j, g)) << ", " << on[g] << ", " << in[g] << ", t" << i << ", t" << j << ");\n";
                 auto centres = [&](const char* axis, float ca1, float ca2, const std::string& v1, const std::string& v2, const char* tag) {
                     if (ca1 == ca2) return std::make_pair(v1, v2);      // one shared scalar, broadcast
@@ -349,20 +333,10 @@ inline std::string spec_generate(const KParams& kp, bool tex, int mats_mask, int
                 ++u;
                 continue;
             }
-            (void)p;
+            // one rectangle: its two in-plane coordinates are the two lanes
             o << "        const float t" << i << " = (" << spec_float(plane(i, g)) << " - " << on[g] << ") * " << in[g] << ";\n";
-            if (packed) {   // one rectangle: its two in-plane coordinates are the two lanes
-                o << "        float xa" << i << ", xb" << i << ";\n";
-                coords("t" + std::to_string(i), g, va[i - begin], vb[i - begin], "xa" + std::to_string(i), "xb" + std::to_string(i));
-                continue;
-            }
-            if (chain) {
-                o << "        const float xa" << i << " = fmaf(t" << i << ", " << da[g] << ", " << va[i - begin] << "), xb" << i << " = fmaf(t" << i
-                  << ", " << db[g] << ", " << vb[i - begin] << ");\n";
-                continue;
-            }
-            o << "        const float c" << i << " = rect_candidate(t" << i << ", fmaf(t" << i << ", " << da[g] << ", " << va[i - begin]
-              << "), fmaf(t" << i << ", " << db[g] << ", " << vb[i - begin] << "), " << spec_float(c.y) << ", " << spec_float(c.w) << ");\n";
+            o << "        float xa" << i << ", xb" << i << ";\n";
+            coords("t" + std::to_string(i), g, va[i - begin], vb[i - begin], "xa" + std::to_string(i), "xb" + std::to_string(i));
         }
         if (s0 >= 0) {
             const float4 c = kp.crect_bounds[g][s0 - begin];
@@ -372,22 +346,19 @@ inline std::string spec_generate(const KParams& kp, bool tex, int mats_mask, int
         if (s0 >= 0) nothing_yet = false;
         for (int i : rest) {
             const float4 c = kp.crect_bounds[g][i - begin];
-            if (chain && fidx && nothing_yet) {   // the first test of the function: selects between literals
+            if (fidx && nothing_yet) {   // the first test of the function: selects between literals
                 o << "        rect_closest_first(t" << i << ", xa" << i << ", xb" << i << ", " << spec_float(c.y) << ", " << spec_float(c.w) << ", "
                   << spec_float((float)i) << ", best_t, bestf);\n";
                 nothing_yet = false;
                 continue;
             }
             nothing_yet = false;
-            if (chain && fidx)
+            if (fidx)
                 o << "        rect_closest_fma(t" << i << ", xa" << i << ", xb" << i << ", " << spec_float(c.y) << ", " << spec_float(c.w) << ", "
                   << spec_float((float)i) << ", best_t, bestf);\n";
-            else if (chain)
+            else
                 o << "        rect_closest(t" << i << ", xa" << i << ", xb" << i << ", " << spec_float(c.y) << ", " << spec_float(c.w) << ", " << i
                   << ", best_t, best);\n";
-            else
-                o << "        { const bool hit = c" << i << " <= best_t; best_t = hit ? c" << i << " : best_t; best = hit ? " << i
-                  << " : best; }\n";
         }
         o << "    }\n";
     }
@@ -423,7 +394,7 @@ inline std::string spec_generate(const KParams& kp, bool tex, int mats_mask, int
             const double ca = 0.5 * ((double)p.a.x + p.a.y), ha = 0.5 * ((double)p.a.y - p.a.x);
             const double cb = 0.5 * ((double)p.a.z + p.a.w), hb = 0.5 * ((double)p.a.w - p.a.z);
             // two consecutive sides on the same axis (a Box's opposite faces): packed arithmetic, as for the plain groups
-            if (std::getenv("RC_SPEC_SCALAR") == nullptr && i + 1 < first + count && (__float_as_int_host(kp.cprims[i + 1].b.z) & 15) == type) {
+            if (i + 1 < first + count && (__float_as_int_host(kp.cprims[i + 1].b.z) & 15) == type) {
                 const DevPrim& q = kp.cprims[i + 1];
                 const int j = i + 1;
                 const double ca2 = 0.5 * ((double)q.a.x + q.a.y), cb2 = 0.5 * ((double)q.a.z + q.a.w);

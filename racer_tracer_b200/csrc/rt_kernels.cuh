@@ -333,17 +333,6 @@ RT_D bool shade_hit(const KParams& P, const TexCtx& X, const Scene& S, const Rng
 #ifndef RT_STEAL
 #define RT_STEAL 1
 #endif
-#ifndef RT_STEAL_MIN
-#define RT_STEAL_MIN 4      // a victim keeps at least half of >= 4 unstarted samples; below that the tail is left alone
-#endif
-
-
-#ifndef RT_KCONST_MASK
-#define RT_KCONST_MASK 7
-#endif
-#ifndef RT_PHILOX_LATE
-#define RT_PHILOX_LATE 0    // 1: the segment's block is drawn after the closest hit in the source (ptxas schedules it either way)
-#endif
 
 // channel mean of the radiance a * b that a path adds where it ends
 RT_D float radiance_y(const vec3f& a, const vec3f& b) { return (a.x * b.x + a.y * b.y + a.z * b.z) * (1.0f / 3.0f); }
@@ -382,10 +371,10 @@ RT_D void megakernel_body(const KParams& P, float* __restrict__ accum, unsigned 
     TexCtx X; X.perlin = L.perlin; X.perm = L.perm;
     {   // volatile: a plain load would be folded back into the literal (the only value ever stored there)
         const volatile float* rc = reg_consts;
-        // held in registers across the path loop, see TexCtx (RT_KCONST_MASK: which of the three; experiments)
-        if (RT_KCONST_MASK & 1) X.k_two = rc[0];
-        if (RT_KCONST_MASK & 2) X.k_phi = rc[1];
-        if (RT_KCONST_MASK & 4) X.k_one = rc[2];
+        // held in registers across the path loop, see TexCtx
+        X.k_two = rc[0];
+        X.k_phi = rc[1];
+        X.k_one = rc[2];
 #ifdef RT_SPECIALIZED
 #pragma unroll
         for (int j = 0; j < RT_SPEC_REG_CONSTS; ++j) X.k_spec[j] = rc[3 + j];
@@ -524,19 +513,13 @@ RT_D void megakernel_body(const KParams& P, float* __restrict__ accum, unsigned 
         // ---- the segment's random block: drawn here, by all lanes together.  Nothing before the hit record needs
         // it (the spare bytes of a sample's block 0 are the NEXT sample's v jitter, DESIGN §4), so its ten dependent
         // multiply-xor rounds are scheduled between the instructions of the closest hit instead of in front of them.
-#if !RT_PHILOX_LATE
         const uint2 rnd = philox2x32_from<ROUNDS>(ppre, ctr1, P.ks);   // == philox2x32_ks(pc.pixel, rt_ctr1(R.sample, seg, RT_TAG_PATH))
         if (fresh) vj_bits = __byte_perm(rnd.y, rnd.x, 0x0040);
-#endif
         RayT<float> r = make_ray(o, d, time);
         float t;
         int prim;
         if (MODE == RT_MODE_CONST_LINEAR) { ConstScene S(P, sh_prims); prim = closest_hit<MODE>(P, S, r, last_prim, t, X); }
         else { PtrScene S; S.prims = L.prims; S.nodes = L.nodes; S.inst = P.instances; S.ref_aabb = P.ref_aabb; prim = closest_hit<MODE>(P, S, r, last_prim, t, X); }
-#if RT_PHILOX_LATE
-        const uint2 rnd = philox2x32_from<ROUNDS>(ppre, ctr1, P.ks);
-        if (fresh) vj_bits = __byte_perm(rnd.y, rnd.x, 0x0040);
-#endif
         ++nseg;
         if (prim < 0) {  // renderer.rs:78-88
             if (!RT_SPEC_BG_BLACK) {
@@ -586,7 +569,9 @@ RT_D void megakernel_body(const KParams& P, float* __restrict__ accum, unsigned 
                     const unsigned idle = __ballot_sync(m, !(RT_LANE_BUSY));
                     if (idle == 0u) break;
                     const int most = __reduce_max_sync(m, rem);
-                    if (most < RT_STEAL_MIN) break;      // unstarted samples only ever shrink: nothing worth taking, now or later
+                    // a victim keeps at least half of >= 4 unstarted samples; below that the tail is left alone.  Unstarted
+                    // samples only ever shrink: nothing worth taking, now or later
+                    if (most < 4) break;
                     const int victim = __ffs(__ballot_sync(m, rem == most)) - 1, thief = __ffs(idle) - 1;
                     const int take = most >> 1;
                     const int v_last = __shfl_sync(m, s_last, victim), v_owner = __shfl_sync(m, owner, victim);

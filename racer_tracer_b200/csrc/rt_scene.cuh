@@ -420,23 +420,18 @@ RT_D void rect_closest_fma(float t, float xa, float xb, float ha, float hb, floa
 
 // The FIRST test of a generated closest hit: nothing has been hit yet (best_t = RT_NO_HIT, index -1), so the two
 // results are selects between literals instead of updates of running values — two instructions fewer than the
-// general form, whose multiply-adds with the known start values ptxas does not fold.  `t <= RT_NO_HIT` could go as
-// well: a ray parallel to the plane has t = +-inf or NaN, and then the in-plane coordinates t * d + o are +-inf or
-// NaN too, which the bounds tests at the head of the chain reject (RT_FIRST_TEST_RANGE, above).
-// (1: the first test also compares t <= RT_NO_HIT.  The compare is redundant — see below — but the kernel WITHOUT
-// it measured 2.1 % slower, 33.39 against 32.71 ms on the same GPU, profiles/r02_v26_sweeps.txt: one instruction
-// fewer, another ptxas schedule.  At 142 instructions the schedule's luck is worth more than an instruction.)
-#ifndef RT_FIRST_TEST_RANGE
-#define RT_FIRST_TEST_RANGE 1
-#endif
+// general form, whose multiply-adds with the known start values ptxas does not fold.
+// The compare t <= RT_NO_HIT is redundant: a ray parallel to the plane has t = +-inf or NaN, and then the in-plane
+// coordinates t * d + o are +-inf or NaN too, which the bounds tests at the head of the chain reject.  But the
+// kernel WITHOUT it measured 2.1 % slower, 33.39 against 32.71 ms on the same GPU (profiles/r02_v26_sweeps.txt):
+// one instruction fewer, another ptxas schedule.  At 142 instructions the schedule's luck is worth more than an
+// instruction.
 RT_D void rect_closest_first(float t, float xa, float xb, float ha, float hb, float index, float& best_t, float& best_index) {
     asm("{\n\t.reg .pred p;\n\t"
         "setp.le.f32 p, %2, %4;\n\t"
         "setp.le.and.f32 p, %3, %5, p;\n\t"
         "setp.ge.and.f32 p, %6, 0f3A83126F, p;\n\t"   /* t >= 0.001f */
-#if RT_FIRST_TEST_RANGE
         "setp.le.and.f32 p, %6, 0f7F61B1E6, p;\n\t"   /* t <= RT_NO_HIT (3e38f) */
-#endif
         "selp.f32 %0, %6, 0f7F61B1E6, p;\n\t"
         "selp.f32 %1, %7, 0fBF800000, p;\n\t}"
         : "=f"(best_t), "=f"(best_index) : "f"(fabsf(xa)), "f"(fabsf(xb)), "f"(ha), "f"(hb), "f"(t), "f"(index));
@@ -671,23 +666,12 @@ RT_D bool aabb_hit_reference(float4 lo, float4 hi, const RayT<float>& r, float t
     return true;
 }
 
-// Entry distance of the slab test (aabb_hit above) when the box is hit within [t_min, t_max], else -1.
-RT_D float aabb_entry(float4 lo, float4 hi, const RayT<float>& r, float t_max) {
-    float tx0 = (lo.x - r.o.x) * r.inv_d.x, tx1 = (hi.x - r.o.x) * r.inv_d.x;
-    float ty0 = (lo.y - r.o.y) * r.inv_d.y, ty1 = (hi.y - r.o.y) * r.inv_d.y;
-    float tz0 = (lo.z - r.o.z) * r.inv_d.z, tz1 = (hi.z - r.o.z) * r.inv_d.z;
-    float tn = fmaxf(fmaxf(fminf(tx0, tx1), fminf(ty0, ty1)), fmaxf(fminf(tz0, tz1), (float)RT_T_MIN));
-    float tf = fminf(fminf(fmaxf(tx0, tx1), fmaxf(ty0, ty1)), fminf(fmaxf(tz0, tz1), t_max));
-    return tn <= tf ? tn : -1.0f;
-}
-
 // The primitives of one leaf (one top-level object: a single primitive, or the six sides of a Box
 // tested in order, src/geometry/box.rs:82-101; they share the object's instance transform, applied
-// to the ray once per leaf).  ORDERED = the traversal may reach leaves in any order: a candidate
-// then replaces the best hit if it is nearer, or equally near with a higher primitive index — which
-// is what the reference's left-to-right walk with `t <= closest` (bvh_node.rs:124-129, sphere.rs:53)
-// ends up with, since primitives are stored in its visiting order.
-template <bool ORDERED, class Scene>
+// to the ray once per leaf).  The walk reaches the leaves in the reference's order and a primitive
+// only reports a hit within best_t, so every hit replaces the best one: a later primitive wins an
+// exact tie, as with the reference's `t <= closest` (bvh_node.rs:124-129, sphere.rs:53).
+template <class Scene>
 RT_D void leaf_test(const Scene& S, int leaf, const RayT<float>& r, int last_prim, float& best_t, int& best) {
     const int first = leaf & 0xffffff, count = leaf >> 24;
     const int inst = RT_HAS_INSTANCES ? kinds_inst(S.pb(first).z) : -1;
@@ -695,24 +679,21 @@ RT_D void leaf_test(const Scene& S, int leaf, const RayT<float>& r, int last_pri
         const RayT<float> lr = to_local(S.instances()[inst], r);
         for (int p = first; p < first + count; ++p) {
             const float t = prim_test_local(S, p, S.pa(p), S.pb(p), lr, p == last_prim, true, best_t);
-            if (t >= 0.0f && (!ORDERED || t < best_t || p > best)) { best_t = t; best = p; }
+            if (t >= 0.0f) { best_t = t; best = p; }
         }
     } else {
         for (int p = first; p < first + count; ++p) {
             const float t = prim_test_local(S, p, S.pa(p), S.pb(p), r, p == last_prim, false, best_t);
-            if (t >= 0.0f && (!ORDERED || t < best_t || p > best)) { best_t = t; best = p; }
+            if (t >= 0.0f) { best_t = t; best = p; }
         }
     }
 }
 
-#ifndef RT_BVH_DEFER_LEAF
-#define RT_BVH_DEFER_LEAF 0
-#endif
 // Threaded pre-order BVH: left child = i + 1, `skip` = next node when this
 // subtree is done.  Visits left before right with a shrinking t_max, exactly
 // the order of Node::hit (src/bvh_node.rs:112-132), over the node range
 // [i, end) (the whole tree, or one subtree).
-template <bool ORDERED, class Scene>
+template <class Scene>
 RT_D void closest_hit_threaded(const Scene& S, int i, int end, const RayT<float>& r, int last_prim, float& best_t, int& best) {
     if (S.reference_aabb()) {   // stored boxes that are not bounding boxes (Q14): the reference's own test
 #pragma unroll 1
@@ -720,133 +701,29 @@ RT_D void closest_hit_threaded(const Scene& S, int i, int end, const RayT<float>
             const float4 lo = S.nlo(i), hi = S.nhi(i);
             const int leaf = __float_as_int(hi.w);
             const bool box_hit = aabb_hit_reference(lo, hi, r, best_t);
-            if (box_hit && leaf >= 0) leaf_test<ORDERED>(S, leaf, r, last_prim, best_t, best);
+            if (box_hit && leaf >= 0) leaf_test(S, leaf, r, last_prim, best_t, best);
             i = box_hit && leaf < 0 ? i + 1 : __float_as_int(lo.w);
         }
         return;
     }
     const BoxRay br = make_box_ray(r);
-#if RT_BVH_DEFER_LEAF
-    // Experiment (-DRT_BVH_DEFER_LEAF=1, off by default): a lane that enters a leaf box parks the leaf and walks
-    // on; the parked leaves of the warp are tested together when some lane needs its slot again or has finished
-    // the walk.  Same tests in the same order per lane (the boxes in between are tested against a t_max that is
-    // at most one leaf stale: a superset), so the result is unchanged; the point is fuller warps in the leaf
-    // test, which runs at 5 of 32 lanes otherwise (profiles/r01_random_bvh_v2_regions.txt).
-    // Measured on the Random scene (precompiled kernel, SAH tree): 2.10e9 samples/s against 2.42e9 for the
-    // plain walk, images identical — sibling leaves are consecutive nodes, so a lane needs its slot again almost
-    // at once and the flushes are as frequent as the leaf visits were, with the vote and the parking on top.
-    // Kept as the measured alternative; a wider (per-warp) leaf queue is what would have to come next.
-    int parked = -1;
-#pragma unroll 1
-    while (true) {
-        int entered = -1;
-        if (i < end) {
-            const float4 lo = S.nlo(i), hi = S.nhi(i);
-            const int leaf = __float_as_int(hi.w);
-            const bool box_hit = aabb_hit_packed(lo, hi, br, best_t);
-            if (box_hit && leaf >= 0) entered = leaf;
-            i = box_hit && leaf < 0 ? i + 1 : __float_as_int(lo.w);
-        }
-        const bool finished = i >= end;
-        const bool need = parked >= 0 && (entered >= 0 || finished);
-        if (__any_sync(__activemask(), need) && parked >= 0) {
-            leaf_test<ORDERED>(S, parked, r, last_prim, best_t, best);
-            parked = -1;
-        }
-        if (entered >= 0) parked = entered;
-        if (finished && parked < 0) break;
-    }
-#else
 #pragma unroll 1
     while (i < end) {
         const float4 lo = S.nlo(i), hi = S.nhi(i);
         const int leaf = __float_as_int(hi.w);
         const bool box_hit = aabb_hit_packed(lo, hi, br, best_t);
         // the only divergent branch of a step is the leaf; the next node is a select
-        if (box_hit && leaf >= 0) leaf_test<ORDERED>(S, leaf, r, last_prim, best_t, best);
+        if (box_hit && leaf >= 0) leaf_test(S, leaf, r, last_prim, best_t, best);
         i = box_hit && leaf < 0 ? i + 1 : __float_as_int(lo.w);
     }
-#endif
 }
 
-// Ordered traversal: at an inner node both children are tested (the left child is the next node, the
-// right child is where the left one's skip link points), the nearer one is entered first and the
-// farther one waits on a small per-lane stack together with its entry distance, so that it can be
-// dropped without a second box test once a nearer hit is known.  Same result as the threaded walk
-// (see leaf_test), far fewer node visits when the tree is deep: the nearest leaves shrink t_max first.
-// Scenes whose boxes are not bounding boxes (RotateY, Q14: ref_aabb) keep the reference's order.
-//
-// Measured on the Random scene (1920x1080, 256 spp, one B200): 1.51e9 samples/s against 1.80e9 for the
-// threaded walk — two box tests per step and a stack in local memory cost more than the pruning saves on
-// a 9-level tree whose rays mostly end on the ground sphere — so the threaded walk stays the default and
-// this one is compiled in with -DRT_BVH_ORDERED=1.
-#ifndef RT_BVH_ORDERED
-#define RT_BVH_ORDERED 0
-#endif
-#define RT_BVH_STACK 24
 template <class Scene>
 RT_D int closest_hit_bvh(const Scene& S, int n_nodes, const RayT<float>& r, int last_prim, float& best_t) {
     int best = -1;
     best_t = RT_NO_HIT;
-    if (!RT_BVH_ORDERED || S.reference_aabb()) {
-        closest_hit_threaded<false>(S, 0, n_nodes, r, last_prim, best_t, best);
-        return best;
-    }
-    int stack_node[RT_BVH_STACK];
-    float stack_t[RT_BVH_STACK];
-    int sp = 0;
-    int node = 0;
-    {   // the root's own box (Node::hit tests it first, bvh_node.rs:119)
-        const float4 lo = S.nlo(0), hi = S.nhi(0);
-        if (aabb_entry(lo, hi, r, best_t) < 0.0f) return -1;
-        const int leaf = __float_as_int(hi.w);
-        if (leaf >= 0) { leaf_test<true>(S, leaf, r, last_prim, best_t, best); return best; }
-    }
-#pragma unroll 1
-    while (true) {
-        // `node` is an inner node whose box the ray enters before best_t
-        const int L = node + 1;
-        const float4 llo = S.nlo(L), lhi = S.nhi(L);
-        const int R = __float_as_int(llo.w);
-        const float4 rlo = S.nlo(R), rhi = S.nhi(R);
-        float tl = aabb_entry(llo, lhi, r, best_t), tr = aabb_entry(rlo, rhi, r, best_t);
-        const int lleaf = __float_as_int(lhi.w), rleaf = __float_as_int(rhi.w);
-        // leaves are intersected at once (nearer first), inner children are entered / stacked
-        if (tl >= 0.0f && lleaf >= 0 && !(tr >= 0.0f && rleaf >= 0 && tr < tl)) {
-            leaf_test<true>(S, lleaf, r, last_prim, best_t, best);
-            tl = -1.0f;
-            if (tr > best_t) tr = -1.0f;
-        }
-        if (tr >= 0.0f && rleaf >= 0) {
-            leaf_test<true>(S, rleaf, r, last_prim, best_t, best);
-            tr = -1.0f;
-            if (tl > best_t) tl = -1.0f;
-        }
-        if (tl >= 0.0f && lleaf >= 0) {
-            leaf_test<true>(S, lleaf, r, last_prim, best_t, best);
-            tl = -1.0f;
-        }
-        int next = -1;
-        if (tl >= 0.0f && tr >= 0.0f) {   // two inner children: nearer first
-            const bool left_first = tl <= tr;
-            const int far = left_first ? R : L;
-            const float tfar = left_first ? tr : tl;
-            next = left_first ? L : R;
-            if (sp < RT_BVH_STACK) { stack_node[sp] = far; stack_t[sp] = tfar; ++sp; }
-            else {   // stack exhausted (a degenerate, very deep tree): walk the nearer subtree in reference order now
-                closest_hit_threaded<true>(S, next, __float_as_int(S.nlo(next).w), r, last_prim, best_t, best);
-                next = far;
-                if (tfar > best_t) next = -1;
-            }
-        } else if (tl >= 0.0f) next = L;
-        else if (tr >= 0.0f) next = R;
-        while (next < 0) {   // pop; drop entries that start beyond the best hit found meanwhile
-            if (sp == 0) return best;
-            --sp;
-            if (stack_t[sp] <= best_t) next = stack_node[sp];
-        }
-        node = next;
-    }
+    closest_hit_threaded(S, 0, n_nodes, r, last_prim, best_t, best);
+    return best;
 }
 
 // ---------------------------------------------------------------------------

@@ -1,7 +1,7 @@
 // rt_wavefront.cuh — the wavefront variant of the render path.
 //
 // A pool of N path slots lives in device memory (sized to stay in the 126 MB
-// L2: 1 Mi slots x 80 B = 80 MB; RC_WF_SLOTS overrides).  One pass over the pool is four kinds of
+// L2: 1 Mi slots x 80 B = 80 MB).  One pass over the pool is four kinds of
 // kernels, each full-width and free of the megakernel's regenerate / miss /
 // material divergence:
 //
@@ -354,8 +354,7 @@ int wavefront_run(WavefrontState& w, const KParams& kp, float* accum, size_t sme
 
 inline int wavefront_prepare(WavefrontState& w, const KParams& kp, int sm_count) {
     (void)sm_count;
-    const char* env = getenv("RC_WF_SLOTS");
-    size_t slots = env ? (size_t)atol(env) : (size_t)1024 * 1024;
+    size_t slots = (size_t)1024 * 1024;
     const size_t n_pix_share = (size_t)kp.n_tiles * 128;
     const int spp = kp.s_end - kp.s_begin;
     const size_t chunks = (size_t)(spp + RT_WF_CHUNK - 1) / RT_WF_CHUNK;

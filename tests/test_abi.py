@@ -117,14 +117,6 @@ def test_specialised_source_compiles_for_sm_100a(cuda_lib, cfg, tmp_path):
     assert "spec_closest_hit" in src and "#define RT_SPEC_MATS 9" in src   # lambertian + light
     # ... relative to the kernel's own origin, the centre of the box: the light's plane y = 554 is 276.5 above it
     assert "#define RT_SPEC_SHIFT mk3(277.5f, 277.5f, 277.5f)" in src and "276.5f" in src and "554.0f" not in src
-    os.environ["RC_SPEC_NO_SHIFT"] = "1"
-    try:
-        n0 = cuda_lib.rc_spec_source(job.scene.ptr, None, 0)
-        buf0 = C.create_string_buffer(n0 + 1)
-        cuda_lib.rc_spec_source(job.scene.ptr, buf0, n0 + 1)
-    finally:
-        os.environ.pop("RC_SPEC_NO_SHIFT")
-    assert "554.0f" in buf0.value.decode() and "RT_SPEC_SHIFT" not in buf0.value.decode()
     cu = tmp_path / "spec.cu"
     cu.write_text(src)
     subprocess.run(["/usr/local/cuda/bin/nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-std=c++17", "-I",
@@ -246,14 +238,13 @@ def test_opposite_walls_become_one_test_only_when_every_ray_starts_between_them(
 
 
 def test_generated_kernel_variants_compile_and_agree_on_their_planes(cuda_lib, cfg, tmp_path, monkeypatch):
-    """The pieces of the generated Cornell kernel that can be switched off one at a time (DESIGN §3.1 v25 / v26) all
-    compile, and in every variant the plane constant the hit record snaps a point to (spec_snap_row: the staged
-    table's K) is the same literal as the plane the rectangle TEST uses — if the two differed by an ulp, a ray leaving
-    a wall would re-hit it at t != 0."""
+    """The generated Cornell kernel with and without slab pairs (DESIGN §3.1 v25) compiles, and in both the plane
+    constant the hit record snaps a point to (spec_snap_row: the staged table's K) is the same literal as the plane the
+    rectangle TEST uses — if the two differed by an ulp, a ray leaving a wall would re-hit it at t != 0."""
     import re
     from conftest import scene_path
     job = harness.prepare_job(scene_path("cornell_box"), cfg, 64, 64)
-    for env in ({}, {"RC_SPEC_NO_REG_CONSTS": "1"}, {"RC_SPEC_PACK_ALL": "1"}, {"RC_SPEC_NO_SHIFT": "1"}, {"RC_SPEC_NO_SLAB": "1"}):
+    for env in ({}, {"RC_SPEC_NO_SLAB": "1"}):
         for k, v in env.items():
             monkeypatch.setenv(k, v)
         src = _spec_source(cuda_lib, job, camera=job.camera.origin)
@@ -267,9 +258,6 @@ def test_generated_kernel_variants_compile_and_agree_on_their_planes(cuda_lib, c
             if "// planes" not in src or (a, b) not in re.findall(r"// planes (-?[0-9.]+f), (-?[0-9.]+f)", src):
                 tested += [a, b]
         rows = re.findall(r"case \d+: a = make_float4\(([^)]*)\); bx = (-?[0-9.]+f); cw = [0-9.]+f;", src)
-        if "RC_SPEC_NO_SHIFT" in env:
-            assert not rows and "RT_SPEC_SNAP_TABLE" not in src      # world coordinates: the table keeps the uploaded k
-            continue
         assert len(rows) == 6 and "#define RT_SPEC_SNAP_TABLE 1" in src
         snapped = []
         for a, bx in rows:

@@ -504,37 +504,6 @@ def test_gpu_lbvh_build_and_parity(renderer, oracle, cfg, name):
     assert np.array_equal(renderer.primary_aov(p, 64)[0], ids)
 
 
-def test_generated_kernel_switches_trace_the_same_image(renderer, oracle, cfg):
-    """The pieces of the generated kernel of DESIGN §3.1 v25 / v26, switched off one at a time.  Register constants and
-    packed / scalar in-plane coordinates are the same arithmetic on the same values: the image is the same bit for
-    bit.  The scene-origin shift (with the p*M+K snap table) computes the same paths in other coordinates: fp32
-    roundings differ, so the images agree the way the specialised and the precompiled kernel do — and each agrees with
-    the oracle."""
-    w, h, spp = 320, 180, 16
-    job = job_for("cornell_box", cfg, w, h)
-    p = harness.make_params(w, h, spp, 20, seed=9, specialize=1)
-    renderer.upload(job)
-    base = renderer.render(p)
-    assert renderer.stats().specialized == 1
-    ref = oracle.render(job, harness.make_params(w, h, spp, 20, seed=9))
-    assert float((np.abs(base - ref).max(axis=2) > 2e-3).mean()) < 0.03
-    for switch, exact in (("RC_SPEC_NO_REG_CONSTS", True), ("RC_SPEC_PACK_ALL", True), ("RC_SPEC_NO_SHIFT", False)):
-        os.environ[switch] = "1"
-        try:
-            renderer.upload(job)          # the source is regenerated at the next render
-            img = renderer.render(p)
-        finally:
-            del os.environ[switch]
-        assert renderer.stats().specialized == 1
-        if exact:
-            assert np.array_equal(img, base), switch
-        else:
-            err = np.abs(img - base).max(axis=2)
-            assert np.median(err) < 1e-6 and float((err > 2e-3).mean()) < 0.01, (switch, np.median(err), (err > 2e-3).mean())
-            assert float((np.abs(img - ref).max(axis=2) > 2e-3).mean()) < 0.03
-    renderer.upload(job)
-
-
 def test_library_resplits_a_median_tree_by_sah(renderer, oracle, cfg, monkeypatch):
     """A host that passes the reference's own median-split tree (Node::build, src/bvh_node.rs:31-82) — what the Rust
     shim does — gets the surface-area-heuristic tree anyway: rc_upload_scene re-splits the same leaves when that

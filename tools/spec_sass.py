@@ -2,7 +2,7 @@
 """Compiles the scene-specialised megakernel source (rc_spec_source) with nvcc for sm_100a — no GPU
 needed — and prints registers, the static SASS opcode mix of the main loop and, with --dump, the SASS.
 
-    python tools/spec_sass.py cornell_box [--dump out.sass] [-D RT_REGEN_MIN=8]
+    python tools/spec_sass.py cornell_box [--dump out.sass] [-D RT_STEAL=0]
 """
 import argparse
 import collections
