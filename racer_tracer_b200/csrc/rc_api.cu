@@ -11,6 +11,7 @@
 #include <map>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "rt_kernels.cuh"
@@ -76,6 +77,66 @@ struct DevBuf {
     }
 };
 
+template <class T> using HostVec = std::vector<T>;
+
+// What order a scene table's entries follow: rc_build_lbvh permutes the ORDER_PRIM tables (one entry per primitive) into
+// the leaf order of the tree it builds and replaces the ORDER_TREE tables with that tree.
+enum TableOrder { ORDER_NONE, ORDER_PRIM, ORDER_TREE };
+template <TableOrder O> using Order = std::integral_constant<TableOrder, O>;
+
+// The tables of an uploaded scene: built on the host (Buf = HostVec, build_tables) and held on every device (Buf = DevBuf).
+template <template <class> class Buf>
+struct SceneTables {
+    Buf<DevPrim> prims;            // fp32 primitives, BVH depth-first order
+    Buf<DevPrim> prims_lin;        // the same sorted by type (linear modes)
+    Buf<DevNode> nodes;            // threaded BVH
+    Buf<DevTexture> textures;
+    Buf<DevInstance> instances;
+    Buf<float4> perlin;            // n_perlin x 256 gradients
+    Buf<uint8_t> perm;             // n_perlin x 3 x 256
+    Buf<DevPrimD> prims_d;         // f64 tables of primary_aov_kernel_f64
+    Buf<int> prim_kind;
+    Buf<uint32_t> prim_id;
+    Buf<DevNodeD> nodes_d;
+    Buf<int> prim_inst;
+    Buf<DevInstanceD> instances_d;
+
+    // f(Order<order of the table>(), table of *this, the same table of each of `other`...) for every table
+    template <class F, class... Other>
+    void each(F&& f, Other&... other) {
+        f(Order<ORDER_PRIM>(), prims, other.prims...);
+        f(Order<ORDER_NONE>(), prims_lin, other.prims_lin...);
+        f(Order<ORDER_TREE>(), nodes, other.nodes...);
+        f(Order<ORDER_NONE>(), textures, other.textures...);
+        f(Order<ORDER_NONE>(), instances, other.instances...);
+        f(Order<ORDER_NONE>(), perlin, other.perlin...);
+        f(Order<ORDER_NONE>(), perm, other.perm...);
+        f(Order<ORDER_PRIM>(), prims_d, other.prims_d...);
+        f(Order<ORDER_PRIM>(), prim_kind, other.prim_kind...);
+        f(Order<ORDER_PRIM>(), prim_id, other.prim_id...);
+        f(Order<ORDER_TREE>(), nodes_d, other.nodes_d...);
+        f(Order<ORDER_PRIM>(), prim_inst, other.prim_inst...);
+        f(Order<ORDER_NONE>(), instances_d, other.instances_d...);
+    }
+
+    // DevBuf::assign of every table (the caller synchronises `st` before `h` goes away)
+    cudaError_t upload(const SceneTables<HostVec>& h, cudaStream_t st) {
+        cudaError_t e = cudaSuccess;
+        each([&](auto, auto& dev, const auto& host) { if (e == cudaSuccess) e = dev.assign(host, st); }, h);
+        return e;
+    }
+    void release() { each([](auto, auto& dev) { dev.release(); }); }
+    void bind(KParams& kp) const {
+        kp.prims = prims.p; kp.prims_lin = prims_lin.p; kp.nodes = nodes.p; kp.textures = textures.p;
+        kp.instances = instances.p;
+        kp.perlin = perlin.p; kp.perlin_perm = perm.p;
+    }
+    void bind(AovParamsD& ap) const {
+        ap.prims = prims_d.p; ap.prim_kind = prim_kind.p; ap.prim_id = prim_id.p; ap.nodes = nodes_d.p;
+        ap.prim_inst = prim_inst.p; ap.instances = instances_d.p;
+    }
+};
+
 struct DeviceState {
     int device = 0;
     cudaStream_t stream = nullptr;
@@ -84,19 +145,7 @@ struct DeviceState {
     cudaEvent_t ev_traced = nullptr;   // this device's share of the current render has been traced (cancel relay, fork)
     DevBuf<int> cancel_word;           // the word this device's kernels watch during a cancellable render (KParams::cancel_flag)
     cudaStream_t cancel_stream = nullptr;   // carries the 4-byte copy that raises it while the render kernel runs
-    DevBuf<DevPrim> prims;
-    DevBuf<DevPrim> prims_lin;
-    DevBuf<DevNode> nodes;
-    DevBuf<DevTexture> textures;
-    DevBuf<DevInstance> instances;
-    DevBuf<float4> perlin;
-    DevBuf<uint8_t> perm;
-    DevBuf<DevPrimD> prims_d;
-    DevBuf<int> prim_kind;
-    DevBuf<uint32_t> prim_id;
-    DevBuf<DevNodeD> nodes_d;
-    DevBuf<int> prim_inst;
-    DevBuf<DevInstanceD> instances_d;
+    SceneTables<DevBuf> tables;
     std::vector<cudaArray_t> arrays;
     std::vector<std::pair<int, int>> array_dims;   // width, height of arrays[i]: a re-upload with the same image sizes reuses array and texture object
     std::vector<cudaTextureObject_t> tex;
@@ -147,13 +196,11 @@ struct rc_ctx {
     int spec_rounds = 10;        // Philox rounds spec_source and spec_source_moments were generated for
     std::vector<LbvhObject> objects, objects_next;   // top-level objects of the uploaded scene (rc_build_lbvh)
     std::vector<int> prim_order;       // device primitive i = uploaded primitive prim_order[i] (empty: identity)
-    bool lbvh = false;
     std::vector<rc_frame*> frames;     // rc_frame_create / rc_frame_open
     bool stats_pending = false;        // the last render's time / counters have not been read back yet
     std::vector<void*> shared_owned, shared_opened;   // rc_shared_alloc / rc_shared_open
     int n_prims = 0, n_perlin = 0;
     bool instanced = false;
-    rc_camera camera;
     rc_stats stats;
     MultiState multi;
     int* cancel_relay = nullptr;       // one page-locked word holding 1: the source of the copy that raises a device's cancel word
@@ -169,12 +216,6 @@ void free_scene(DeviceState& d) {
     d.tex.clear();
     d.arrays.clear();
     d.array_dims.clear();
-}
-
-void free_tables(DeviceState& d) {
-    d.prims.release(); d.prims_lin.release(); d.nodes.release(); d.textures.release(); d.instances.release();
-    d.perlin.release(); d.perm.release(); d.prims_d.release(); d.prim_kind.release();
-    d.prim_id.release(); d.nodes_d.release(); d.prim_inst.release(); d.instances_d.release();
 }
 
 // Checker levels of the longest chain of checker textures (checkered.rs:32-43 follows children without a limit), or -1
@@ -290,18 +331,30 @@ void set_skip(const rc_scene* s, int i, int skip, std::vector<int>& out) {
 }
 
 #define RC_SMEM_STAGE_LIMIT (36 * 1024)
-int pick_mode(const rc_scene* s, bool rects_fit, bool instanced, size_t& smem_bytes) {
-    const char* force = std::getenv("RC_SCENE_MODE");  // experiments: const | smem | global | smemlin
-    size_t perlin_bytes = (size_t)s->n_perlin * (256 * 16 + 768);
-    size_t bvh_bytes = (size_t)s->n_nodes * sizeof(DevNode) + (size_t)s->n_prims * sizeof(DevPrim);
-    int mode;
-    // instanced scenes always traverse the BVH: its (possibly non-bounding, Q14) boxes are part of the semantics
-    if (!instanced && s->n_prims <= RT_MAX_CONST_PRIMS && rects_fit) mode = RT_MODE_CONST_LINEAR;
+#define RC_MODE_BVH (-1)   // scene_staging picks RT_MODE_SMEM_BVH or RT_MODE_GLOBAL_BVH
+
+// The dynamic shared memory a CTA of `mode` fills in stage_scene (rt_kernels.cuh): [nodes][prims][Perlin gradients]
+// [Perlin permutations].  `perlin` is the Perlin part, which kernels without texture work launch without.
+struct Staging { int mode; size_t bytes, perlin; };
+
+Staging scene_staging(int mode, int n_nodes, int n_prims, int n_perlin) {
+    const size_t nodes = (size_t)n_nodes * sizeof(DevNode), prims = (size_t)n_prims * sizeof(DevPrim);
+    const size_t perlin = (size_t)n_perlin * (256 * 16 + 768);   // 256 float4 gradients, three 256-byte permutations
     // shared-memory staging pays only while it does not cost occupancy (profiles/r01_random_bvh_v1_ncu.md:
     // 62 KB per CTA left 12 warps per SM and 44 % issue utilisation; the same tables read through L1 ran 1.5x
     // faster): keep the per-CTA copy below a sixth of the SM's 227 KB, larger tables are read through L1/L2
-    else if (s->n_nodes > 0 && bvh_bytes + perlin_bytes <= RC_SMEM_STAGE_LIMIT) mode = RT_MODE_SMEM_BVH;
-    else if (s->n_nodes > 0) mode = RT_MODE_GLOBAL_BVH;
+    if (mode == RC_MODE_BVH) mode = nodes + prims + perlin <= RC_SMEM_STAGE_LIMIT ? RT_MODE_SMEM_BVH : RT_MODE_GLOBAL_BVH;
+    // the linear modes stage the type-sorted table (the constant-bank mode too: its hit records and shading index it
+    // per lane)
+    return Staging{mode, perlin + (mode == RT_MODE_SMEM_BVH ? nodes : 0) + (mode != RT_MODE_GLOBAL_BVH ? prims : 0), perlin};
+}
+
+int pick_mode(const rc_scene* s, bool rects_fit, bool instanced, size_t& smem_bytes) {
+    const char* force = std::getenv("RC_SCENE_MODE");  // experiments: const | smem | global | smemlin
+    int mode;
+    // instanced scenes always traverse the BVH: its (possibly non-bounding, Q14) boxes are part of the semantics
+    if (!instanced && s->n_prims <= RT_MAX_CONST_PRIMS && rects_fit) mode = RT_MODE_CONST_LINEAR;
+    else if (s->n_nodes > 0) mode = RC_MODE_BVH;
     else mode = RT_MODE_SMEM_LINEAR;
     if (force && !instanced) {
         std::string f(force);
@@ -310,12 +363,8 @@ int pick_mode(const rc_scene* s, bool rects_fit, bool instanced, size_t& smem_by
         else if (f == "global" && s->n_nodes > 0) mode = RT_MODE_GLOBAL_BVH;
         else if (f == "smemlin") mode = RT_MODE_SMEM_LINEAR;
     }
-    smem_bytes = perlin_bytes;
-    if (mode == RT_MODE_SMEM_BVH) smem_bytes += bvh_bytes;
-    // the linear modes stage the type-sorted table (the constant-bank mode too: its hit records
-    // and shading index it per lane)
-    if (mode == RT_MODE_SMEM_LINEAR || mode == RT_MODE_CONST_LINEAR) smem_bytes += (size_t)s->n_prims * sizeof(DevPrim);
-    return mode;
+    const Staging st = scene_staging(mode, s->n_nodes, s->n_prims, s->n_perlin);
+    smem_bytes = st.bytes; return st.mode;
 }
 
 template <typename K>
@@ -352,17 +401,13 @@ int launch_moments_mode(const KParams& kp, float* accum, int blocks, size_t smem
 // active != NULL: an adaptive round (megakernel_moments)
 int launch_mega(int mode, bool tex, const KParams& kp, float* accum, int sampler, int rounds, int blocks, size_t smem, cudaStream_t st,
                 const uint8_t* active = nullptr, float* round_m2 = nullptr) {
-#define RC_MODE(M) (!active ? (tex ? launch_mega_mode<M, true>(kp, accum, sampler, rounds, blocks, smem, st)          \
-                                   : launch_mega_mode<M, false>(kp, accum, sampler, rounds, blocks, smem, st))        \
-                             : (tex ? launch_moments_mode<M, true>(kp, accum, blocks, smem, st, active, round_m2)     \
-                                    : launch_moments_mode<M, false>(kp, accum, blocks, smem, st, active, round_m2)))
-    switch (mode) {
-    case RT_MODE_CONST_LINEAR: return RC_MODE(RT_MODE_CONST_LINEAR);
-    case RT_MODE_SMEM_BVH: return RC_MODE(RT_MODE_SMEM_BVH);
-    case RT_MODE_GLOBAL_BVH: return RC_MODE(RT_MODE_GLOBAL_BVH);
-    default: return RC_MODE(RT_MODE_SMEM_LINEAR);
-    }
-#undef RC_MODE
+    return with_mode(mode, [&](auto m) {
+        constexpr int M = decltype(m)::value;
+        if (!active) return tex ? launch_mega_mode<M, true>(kp, accum, sampler, rounds, blocks, smem, st)
+                                : launch_mega_mode<M, false>(kp, accum, sampler, rounds, blocks, smem, st);
+        return tex ? launch_moments_mode<M, true>(kp, accum, blocks, smem, st, active, round_m2)
+                   : launch_moments_mode<M, false>(kp, accum, blocks, smem, st, active, round_m2);
+    });
 }
 
 int check_params(const rc_params* p) {
@@ -489,9 +534,7 @@ int trace_share(rc_ctx* ctx, const rc_params* p, const ShareCall& call, bool& wa
         DeviceState& d = ctx->devs[k];
         CUDA_TRY(cudaSetDevice(d.device));
         KParams kp = ctx->kp;
-        kp.prims = d.prims.p; kp.prims_lin = d.prims_lin.p; kp.nodes = d.nodes.p; kp.textures = d.textures.p;
-        kp.instances = d.instances.p;
-        kp.perlin = d.perlin.p; kp.perlin_perm = d.perm.p;
+        d.tables.bind(kp);
         for (size_t i = 0; i < d.tex.size(); ++i) kp.images[i] = d.tex[i];
         kp.segment_counter = d.counter.p;
         kp.cancel_flag = relay ? d.cancel_word.p : nullptr;
@@ -516,7 +559,8 @@ int trace_share(rc_ctx* ctx, const rc_params* p, const ShareCall& call, bool& wa
         if (kp.n_tiles == 0 || kp.s_end <= kp.s_begin) { if (relay) CUDA_TRY(cudaEventRecord(d.ev_traced, d.stream)); continue; }
         if (p->variant == RC_VARIANT_WAVEFRONT) {
             if (kp.has_motion && rounds != 10) return fail(RC_ERR_INVALID, "the wavefront variant traces moving spheres with 10 Philox rounds only");
-            int rc = wavefront_render(d.wf, ctx->mode, kp, accum, p->sampler, rounds, ctx->smem_bytes, d.stream, d.sm_count, launches);
+            const size_t perlin = scene_staging(ctx->mode, kp.n_nodes, kp.n_prims, kp.n_perlin).perlin;
+            int rc = wavefront_render(d.wf, ctx->mode, kp, accum, p->sampler, rounds, ctx->smem_bytes, perlin, d.stream, launches);
             if (rc != RC_OK) return fail(rc, "wavefront launch failed: " + std::string(cudaGetErrorString(cudaGetLastError())));
             continue;
         }
@@ -864,19 +908,7 @@ static bool resplit_sah(const rc_scene* s, ResplitScene& out) {
     return true;
 }
 
-struct HostTables {   // everything rc_upload_scene derives from an rc_scene, before any device call
-    std::vector<DevPrim> prims, prims_lin;
-    std::vector<DevPrimD> prims_d;
-    std::vector<int> kinds;
-    std::vector<uint32_t> ids;
-    std::vector<DevNode> nodes;
-    std::vector<DevNodeD> nodes_d;
-    std::vector<DevTexture> textures;
-    std::vector<float4> perlin;
-    std::vector<uint8_t> perm;
-    std::vector<DevInstance> instances;
-    std::vector<DevInstanceD> instances_d;
-    std::vector<int> prim_inst;
+struct HostTables : SceneTables<HostVec> {   // everything rc_upload_scene derives from an rc_scene, before any device call
     KParams kp;
     int mode = RT_MODE_CONST_LINEAR;
     size_t smem_bytes = 0;
@@ -891,8 +923,8 @@ static void build_tables(const rc_scene* s, HostTables& t) {
     // ---- fp32 + f64 primitive tables ----
     std::vector<DevPrim>& prims = t.prims; prims.assign(s->n_prims, DevPrim());
     std::vector<DevPrimD>& prims_d = t.prims_d; prims_d.assign(s->n_prims, DevPrimD());
-    std::vector<int>& kinds = t.kinds; kinds.assign(s->n_prims, 0);
-    std::vector<uint32_t>& ids = t.ids; ids.assign(s->n_prims, 0u);
+    std::vector<int>& kinds = t.prim_kind; kinds.assign(s->n_prims, 0);
+    std::vector<uint32_t>& ids = t.prim_id; ids.assign(s->n_prims, 0u);
     double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
     bool any_textured = false, any_motion = false;
     for (int i = 0; i < s->n_prims; ++i) {
@@ -1183,7 +1215,7 @@ int rc_destroy(rc_ctx* ctx) {
         cudaSetDevice(d.device);
         cudaDeviceSynchronize();
         free_scene(d);
-        free_tables(d);
+        d.tables.release();
         d.accum.release(); d.slice_buf.release(); d.out64.release(); d.counter.release(); d.cancel_word.release();
         d.ad_active.release(); d.ad_spp.release(); d.ad_m2.release(); d.ad_s2.release(); d.ad_err.release();
         if (d.cancel_stream) cudaStreamDestroy(d.cancel_stream);
@@ -1242,7 +1274,6 @@ int rc_upload_scene(rc_ctx* ctx, const rc_scene* s) {
     ctx->objects.clear();
     ctx->prim_order.clear();
     if (resplit_done) ctx->prim_order = resplit.order;
-    ctx->lbvh = false;
     ctx->n_prims = s->n_prims; ctx->n_perlin = s->n_perlin;
     ctx->instanced = !t.instances.empty();
     if (s->prim_aabb)
@@ -1258,11 +1289,6 @@ int rc_upload_scene(rc_ctx* ctx, const rc_scene* s) {
             o.first = i; o.count = 1;
             ctx->objects.push_back(o);
         }
-    std::vector<DevPrim>& prims = t.prims; std::vector<DevPrim>& prims_lin = t.prims_lin;
-    std::vector<DevPrimD>& prims_d = t.prims_d; std::vector<int>& kinds = t.kinds; std::vector<uint32_t>& ids = t.ids;
-    std::vector<DevNode>& nodes = t.nodes; std::vector<DevNodeD>& nodes_d = t.nodes_d;
-    std::vector<DevTexture>& textures = t.textures; std::vector<float4>& perlin = t.perlin; std::vector<uint8_t>& perm = t.perm;
-
     for (auto& d : ctx->devs) {
         // An interactive host re-uploads after every scene edit (main.rs:178-183): the table allocations are kept
         // and refilled with stream-ordered copies — the stream also orders them after any render still reading the
@@ -1276,19 +1302,7 @@ int rc_upload_scene(rc_ctx* ctx, const rc_scene* s) {
                 same = d.array_dims[i].first == s->images[i].width && d.array_dims[i].second == s->images[i].height;
             if (!same) free_scene(d);
         }
-        CUDA_TRY(d.prims.assign(prims, d.stream));
-        CUDA_TRY(d.prims_lin.assign(prims_lin, d.stream));
-        CUDA_TRY(d.nodes.assign(nodes, d.stream));
-        CUDA_TRY(d.textures.assign(textures, d.stream));
-        CUDA_TRY(d.perlin.assign(perlin, d.stream));
-        CUDA_TRY(d.perm.assign(perm, d.stream));
-        CUDA_TRY(d.prims_d.assign(prims_d, d.stream));
-        CUDA_TRY(d.prim_kind.assign(kinds, d.stream));
-        CUDA_TRY(d.prim_id.assign(ids, d.stream));
-        CUDA_TRY(d.nodes_d.assign(nodes_d, d.stream));
-        CUDA_TRY(d.instances.assign(t.instances, d.stream));
-        CUDA_TRY(d.instances_d.assign(t.instances_d, d.stream));
-        CUDA_TRY(d.prim_inst.assign(t.prim_inst, d.stream));
+        CUDA_TRY(d.tables.upload(t, d.stream));
         for (int i = 0; i < s->n_images; ++i) {
             // image textures as CUDA texture objects: point filter, clamp, u8 -> float/255
             // (src/texture/image.rs:28-51, Q21)
@@ -1339,7 +1353,6 @@ int rc_upload_scene(rc_ctx* ctx, const rc_scene* s) {
 
 int rc_set_camera(rc_ctx* ctx, const rc_camera* c) {
     if (!ctx || !c) return fail(RC_ERR_INVALID, "ctx or camera is NULL");
-    ctx->camera = *c;
     auto v3f = [](const double* p) { return mk3<float>((float)p[0], (float)p[1], (float)p[2]); };
     auto v3d = [](const double* p) { return mk3<double>(p[0], p[1], p[2]); };
     // (upper_left_corner - origin) is formed in f64 here so the fp32 kernels
@@ -1761,23 +1774,19 @@ int rc_build_lbvh(rc_ctx* ctx) {
         }
         lbvh_prim_offsets<<<1, 1024, 0, d.stream>>>(keys.p, obj.p, n, first_new.p);
         lbvh_prim_order<<<grid(n), B, 0, d.stream>>>(keys.p, obj.p, n, first_new.p, order.p);
-        DevBuf<DevNode> nodes;
-        DevBuf<DevNodeD> nodes_d;
-        CUDA_TRY(nodes.resize((size_t)n_nodes));
-        CUDA_TRY(nodes_d.resize((size_t)n_nodes));
-        lbvh_emit<<<grid(n_nodes), B, 0, d.stream>>>(keys.p, obj.p, n, tree.p, leaf_parent.p, first_new.p, nodes.p, nodes_d.p, preorder.p);
+        SceneTables<DevBuf> next;   // the tables that follow primitive order, for the new tree
+        CUDA_TRY(next.nodes.resize((size_t)n_nodes));
+        CUDA_TRY(next.nodes_d.resize((size_t)n_nodes));
+        lbvh_emit<<<grid(n_nodes), B, 0, d.stream>>>(keys.p, obj.p, n, tree.p, leaf_parent.p, first_new.p, next.nodes.p, next.nodes_d.p, preorder.p);
         // primitive tables into the tree's depth-first leaf order
-        DevBuf<DevPrim> prims;
-        DevBuf<DevPrimD> prims_d;
-        DevBuf<int> kind, inst;
-        DevBuf<uint32_t> id;
-        CUDA_TRY(prims.resize((size_t)np)); CUDA_TRY(prims_d.resize((size_t)np)); CUDA_TRY(kind.resize((size_t)np));
-        CUDA_TRY(inst.resize((size_t)np)); CUDA_TRY(id.resize((size_t)np));
-        lbvh_gather<<<grid(np), B, 0, d.stream>>>(d.prims.p, prims.p, order.p, np);
-        lbvh_gather<<<grid(np), B, 0, d.stream>>>(d.prims_d.p, prims_d.p, order.p, np);
-        lbvh_gather<<<grid(np), B, 0, d.stream>>>(d.prim_kind.p, kind.p, order.p, np);
-        lbvh_gather<<<grid(np), B, 0, d.stream>>>(d.prim_inst.p, inst.p, order.p, np);
-        lbvh_gather<<<grid(np), B, 0, d.stream>>>(d.prim_id.p, id.p, order.p, np);
+        cudaError_t e = cudaSuccess;
+        d.tables.each([&](auto order_of, auto& cur, auto& sorted) {
+            if constexpr (decltype(order_of)::value == ORDER_PRIM) {
+                if (e == cudaSuccess) e = sorted.resize((size_t)np);
+                if (e == cudaSuccess) lbvh_gather<<<grid(np), B, 0, d.stream>>>(cur.p, sorted.p, order.p, np);
+            }
+        }, next);
+        CUDA_TRY(e);
         CUDA_TRY(cudaGetLastError());
         if (&d == &ctx->devs[0]) {   // the composed permutation and the object table follow the primitives
             std::vector<int> ord((size_t)np);
@@ -1793,23 +1802,18 @@ int rc_build_lbvh(rc_ctx* ctx) {
             ctx->objects_next = moved;
         }
         CUDA_TRY(cudaStreamSynchronize(d.stream));
-        std::swap(d.prims, prims); std::swap(d.prims_d, prims_d); std::swap(d.prim_kind, kind); std::swap(d.prim_inst, inst); std::swap(d.prim_id, id);
-        std::swap(d.nodes, nodes); std::swap(d.nodes_d, nodes_d);
-        prims.release(); prims_d.release(); kind.release(); inst.release(); id.release(); nodes.release(); nodes_d.release();
+        d.tables.each([](auto order_of, auto& cur, auto& sorted) { if (decltype(order_of)::value != ORDER_NONE) std::swap(cur, sorted); }, next);
+        next.release();
         obj.release(); keys.release(); bounds.release(); tree.release(); leaf_parent.release(); arrived.release(); first_new.release();
         order.release(); preorder.release();
     }
     ctx->objects = ctx->objects_next;
     ctx->kp.n_nodes = n_nodes;
     ctx->aov.n_nodes = n_nodes;
-    // the traversal modes: shared memory when nodes + primitives (+ Perlin tables) fit, global memory otherwise
-    const size_t perlin_bytes = (size_t)ctx->n_perlin * (256 * 16 + 768);
-    const size_t bvh_bytes = (size_t)n_nodes * sizeof(DevNode) + (size_t)np * sizeof(DevPrim);
-    ctx->mode = bvh_bytes + perlin_bytes <= RC_SMEM_STAGE_LIMIT ? RT_MODE_SMEM_BVH : RT_MODE_GLOBAL_BVH;
-    ctx->smem_bytes = perlin_bytes + (ctx->mode == RT_MODE_SMEM_BVH ? bvh_bytes : 0);
+    const Staging st = scene_staging(RC_MODE_BVH, n_nodes, np, ctx->n_perlin);
+    ctx->mode = st.mode; ctx->smem_bytes = st.bytes;
     ctx->spec_source.clear();
     ctx->spec_source_moments.clear();
-    ctx->lbvh = true;
     CUDA_TRY(cudaSetDevice(ctx->devs[0].device));
     return RC_OK;
 }
@@ -1822,7 +1826,7 @@ int rc_get_bvh(rc_ctx* ctx, rc_bvh_node* nodes, int32_t node_capacity, int32_t* 
         DeviceState& d = ctx->devs[0];
         CUDA_TRY(cudaSetDevice(d.device));
         std::vector<DevNodeD> h((size_t)n_nodes);
-        CUDA_TRY(cudaMemcpy(h.data(), d.nodes_d.p, (size_t)n_nodes * sizeof(DevNodeD), cudaMemcpyDeviceToHost));
+        CUDA_TRY(cudaMemcpy(h.data(), d.tables.nodes_d.p, (size_t)n_nodes * sizeof(DevNodeD), cudaMemcpyDeviceToHost));
         for (int i = 0; i < n_nodes; ++i) {
             for (int a = 0; a < 3; ++a) { nodes[i].bmin[a] = h[i].lo[a]; nodes[i].bmax[a] = h[i].hi[a]; }
             if (h[i].leaf >= 0) { nodes[i].left = ~(h[i].leaf & 0xffffff); nodes[i].right = h[i].leaf >> 24; }
@@ -1885,37 +1889,24 @@ int rc_primary_aov(rc_ctx* ctx, const rc_params* p, int32_t precision, uint32_t*
     CUDA_TRY(d_id.resize(np)); CUDA_TRY(d_t.resize(np)); CUDA_TRY(d_n.resize(np * 3)); CUDA_TRY(d_p.resize(np * 3));
     if (precision == 32) {
         KParams kp = ctx->kp;
-        kp.prims = d.prims.p; kp.prims_lin = d.prims_lin.p; kp.nodes = d.nodes.p; kp.textures = d.textures.p;
-        kp.instances = d.instances.p;
-        kp.perlin = d.perlin.p; kp.perlin_perm = d.perm.p;
+        d.tables.bind(kp);
         kp.segment_counter = nullptr;
         rc_params q = *p;
         q.fixed_jitter = 1; q.split = RC_SPLIT_TILES;
         partition(kp, &q, 0, 1);
-        kp.n_perlin = 0;  // no texture work in the AOV: skip the Perlin staging
-        size_t smem = ctx->smem_bytes - (size_t)ctx->kp.n_perlin * (256 * 16 + 768);
-        switch (ctx->mode) {
-        case RT_MODE_CONST_LINEAR:
-            primary_aov_kernel<RT_MODE_CONST_LINEAR><<<kp.n_tiles, RT_BLOCK, smem, d.stream>>>(kp, d_id.p, d_t.p, d_n.p, d_p.p);
-            break;
-        case RT_MODE_SMEM_BVH:
-            rc = set_smem(primary_aov_kernel<RT_MODE_SMEM_BVH>, smem);
-            if (rc != RC_OK) return rc;
-            primary_aov_kernel<RT_MODE_SMEM_BVH><<<kp.n_tiles, RT_BLOCK, smem, d.stream>>>(kp, d_id.p, d_t.p, d_n.p, d_p.p);
-            break;
-        case RT_MODE_GLOBAL_BVH:
-            primary_aov_kernel<RT_MODE_GLOBAL_BVH><<<kp.n_tiles, RT_BLOCK, smem, d.stream>>>(kp, d_id.p, d_t.p, d_n.p, d_p.p);
-            break;
-        default:
-            rc = set_smem(primary_aov_kernel<RT_MODE_SMEM_LINEAR>, smem);
-            if (rc != RC_OK) return rc;
-            primary_aov_kernel<RT_MODE_SMEM_LINEAR><<<kp.n_tiles, RT_BLOCK, smem, d.stream>>>(kp, d_id.p, d_t.p, d_n.p, d_p.p);
-        }
+        // no texture work in the AOV: skip the Perlin staging
+        const size_t smem = ctx->smem_bytes - scene_staging(ctx->mode, kp.n_nodes, kp.n_prims, kp.n_perlin).perlin;
+        kp.n_perlin = 0;
+        rc = with_mode(ctx->mode, [&](auto m) {
+            const int r = set_smem(primary_aov_kernel<decltype(m)::value>, smem);
+            if (r == RC_OK) primary_aov_kernel<decltype(m)::value><<<kp.n_tiles, RT_BLOCK, smem, d.stream>>>(kp, d_id.p, d_t.p, d_n.p, d_p.p);
+            return r;
+        });
+        if (rc != RC_OK) return rc;
     } else {
         AovParamsD ap = ctx->aov;
         ap.width = p->width; ap.height = p->height;
-        ap.prims = d.prims_d.p; ap.prim_kind = d.prim_kind.p; ap.prim_id = d.prim_id.p; ap.nodes = d.nodes_d.p;
-        ap.prim_inst = d.prim_inst.p; ap.instances = d.instances_d.p;
+        d.tables.bind(ap);
         dim3 block(16, 8), grid((p->width + 15) / 16, (p->height + 7) / 8);
         primary_aov_kernel_f64<<<grid, block, 0, d.stream>>>(ap, d_id.p, d_t.p, d_n.p, d_p.p);
     }

@@ -22,7 +22,7 @@
 
 // ---------------------------------------------------------------------------
 // Shared-memory staging of the scene tables (coalesced 16-byte copies).
-// Layout of the dynamic shared segment: [nodes][prims][perlin grads][perms]
+// Layout of the dynamic shared segment: [nodes][prims][perlin grads][perms]; scene_staging (rc_api.cu) sizes it
 // ---------------------------------------------------------------------------
 struct SmemLayout {
     const DevNode* nodes;

@@ -88,19 +88,8 @@ template <typename T> RT_D Vec3T<T> reflect(Vec3T<T> v, Vec3T<T> n) { return v -
 #define PHILOX2_M 0xD256D193u
 #define PHILOX2_W 0x9E3779B9u
 
-template <int ROUNDS>
-RT_HD uint2 philox2x32(uint32_t c0, uint32_t c1, uint32_t key) {
-#pragma unroll
-    for (int r = 0; r < ROUNDS; ++r) {
-        const uint64_t p = (uint64_t)PHILOX2_M * c0;   // IMAD.WIDE.U32
-        c0 = (uint32_t)(p >> 32) ^ (key + (uint32_t)r * PHILOX2_W) ^ c1;
-        c1 = (uint32_t)p;
-    }
-    return make_uint2(c0, c1);
-}
-
-// Device form with the key schedule (key + r*W, r = 0..9) precomputed by the host into the
-// kernel parameters: every round is IMAD.WIDE.U32 + one LOP3 with a constant-bank operand.
+// The key schedule (key + r*W, r = 0..9) is precomputed by the host into the kernel parameters:
+// every round is IMAD.WIDE.U32 + one LOP3 with a constant-bank operand.
 template <int ROUNDS>
 RT_D uint2 philox2x32_ks(uint32_t c0, uint32_t c1, const uint32_t* ks) {
 #pragma unroll

@@ -352,18 +352,6 @@ RT_D float prim_test_local(const Scene& S, int i, float4 a, float4 b, const RayT
     return rect_hit<float>(type, r.o, r.d, r.inv_d, a.x, a.y, a.z, a.w, b.x, (float)RT_T_MIN, t_max);
 }
 
-// One primitive against a world-space ray (SceneObject::hit, src/scene.rs:98-101).
-template <class Scene>
-RT_D float prim_test(const Scene& S, int i, const RayT<float>& r, int last_prim, float t_max) {
-    float4 a = S.pa(i), b = S.pb(i);
-    const int inst = kinds_inst(b.z);
-    if (inst >= 0) {
-        const RayT<float> lr = to_local(S.instances()[inst], r);
-        return prim_test_local(S, i, a, b, lr, i == last_prim, true, t_max);
-    }
-    return prim_test_local(S, i, a, b, r, i == last_prim, false, t_max);
-}
-
 #define RT_NO_HIT 3.0e38f   /* closest-hit distances start here; +inf marks "no candidate" */
 
 // Candidate distance of one axis-aligned rectangle: t when the in-plane hit point lies inside
@@ -610,24 +598,14 @@ RT_D int closest_hit_linear(const KParams& P, const Scene& S, const RayT<float>&
     return best;
 }
 
-// Slab test against [t_min, t_max]; conservative with respect to
-// src/aabb.rs:42-59 (which clips every axis against the original interval and
-// so accepts a superset).  Boxes are padded at upload, see rc_api.cu.
-RT_D bool aabb_hit(float4 lo, float4 hi, const RayT<float>& r, float t_max) {
-    float tx0 = (lo.x - r.o.x) * r.inv_d.x, tx1 = (hi.x - r.o.x) * r.inv_d.x;
-    float ty0 = (lo.y - r.o.y) * r.inv_d.y, ty1 = (hi.y - r.o.y) * r.inv_d.y;
-    float tz0 = (lo.z - r.o.z) * r.inv_d.z, tz1 = (hi.z - r.o.z) * r.inv_d.z;
-    float tn = fmaxf(fmaxf(fminf(tx0, tx1), fminf(ty0, ty1)), fmaxf(fminf(tz0, tz1), (float)RT_T_MIN));
-    float tf = fminf(fminf(fmaxf(tx0, tx1), fmaxf(ty0, ty1)), fminf(fmaxf(tz0, tz1), t_max));
-    return tn <= tf;
-}
-
-// The same slab test for the BVH walk, where it is most of the instructions: per ray, the reciprocal
-// direction I (a zero component gives +-1e20 instead of infinity, so that no product is inf - inf) and
-// N = -o * I; per box, t = bound * I + N — two packed multiply-adds for x and y of both corners (lo.xy and
-// hi.xy are register pairs as loaded) and two scalar ones for z, instead of six subtractions and six
-// multiplications.  Rounds differently from aabb_hit by an ulp of |o * I|: the same order as the
-// rounding of (bound - o) there, and inside the pad the boxes get at upload.
+// Slab test against [t_min, t_max] for the BVH walk, conservative with respect to src/aabb.rs:42-59 (which
+// clips every axis against the original interval and so accepts a superset).  It is most of the walk's
+// instructions: per ray, the reciprocal direction I (a zero component gives +-1e20 instead of infinity, so
+// that no product is inf - inf) and N = -o * I; per box, t = bound * I + N — two packed multiply-adds for x
+// and y of both corners (lo.xy and hi.xy are register pairs as loaded) and two scalar ones for z, instead of
+// six subtractions and six multiplications.  That rounds differently from t = (bound - o) * I by an ulp of
+// |o * I|: the same order as the rounding of (bound - o) there, and inside the pad the boxes get at upload
+// (rc_api.cu).
 struct BoxRay {
     float ix, iy, iz, nx, ny, nz;
 };

@@ -24,6 +24,7 @@
 // shading are the megakernel's own functions, so both variants trace exactly
 // the same paths; only the fp32 summation order differs.
 #pragma once
+#include <type_traits>
 #include "rt_kernels.cuh"
 
 #define RT_WF_CHUNK 32
@@ -312,13 +313,24 @@ __global__ void wf_flush(WfPool W, float* __restrict__ accum) {
 // ---------------------------------------------------------------------------
 // Host driver
 // ---------------------------------------------------------------------------
+// f(std::integral_constant<int, M>()) for the runtime scene mode M (RT_MODE_*): where the host picks the kernels of a mode
+template <class F>
+auto with_mode(int mode, F&& f) {
+    switch (mode) {
+    case RT_MODE_CONST_LINEAR: return f(std::integral_constant<int, RT_MODE_CONST_LINEAR>());
+    case RT_MODE_SMEM_BVH: return f(std::integral_constant<int, RT_MODE_SMEM_BVH>());
+    case RT_MODE_GLOBAL_BVH: return f(std::integral_constant<int, RT_MODE_GLOBAL_BVH>());
+    default: return f(std::integral_constant<int, RT_MODE_SMEM_LINEAR>());
+    }
+}
+
+// smem: the scene staged per CTA; smem_perlin: its Perlin part, which wf_intersect does without
 template <int MODE, int SAMPLER, int ROUNDS>
-int wavefront_run(WavefrontState& w, const KParams& kp, float* accum, size_t smem, cudaStream_t st, unsigned segment_hint,
+int wavefront_run(WavefrontState& w, const KParams& kp, float* accum, size_t smem, size_t smem_perlin, cudaStream_t st,
                   uint64_t& launches) {
-    (void)segment_hint;
     WfPool& W = w.pool;
     const int blocks = (W.n_slots + RT_WF_BLOCK - 1) / RT_WF_BLOCK;
-    const size_t smem_int = smem - (size_t)kp.n_perlin * (256 * 16 + 768);   // geometry only
+    const size_t smem_int = smem - smem_perlin;   // geometry only
     KParams kp_int = kp;
     kp_int.n_perlin = 0;
     if (smem > 48 * 1024) {
@@ -352,8 +364,7 @@ int wavefront_run(WavefrontState& w, const KParams& kp, float* accum, size_t sme
     return cudaGetLastError() == cudaSuccess ? RC_OK : RC_ERR_CUDA;
 }
 
-inline int wavefront_prepare(WavefrontState& w, const KParams& kp, int sm_count) {
-    (void)sm_count;
+inline int wavefront_prepare(WavefrontState& w, const KParams& kp) {
     size_t slots = (size_t)1024 * 1024;
     const size_t n_pix_share = (size_t)kp.n_tiles * 128;
     const int spp = kp.s_end - kp.s_begin;
@@ -394,25 +405,17 @@ inline int wavefront_prepare(WavefrontState& w, const KParams& kp, int sm_count)
     return RC_OK;
 }
 
-template <int MODE>
-int wavefront_dispatch(WavefrontState& w, const KParams& kp, float* accum, int sampler, int rounds, size_t smem,
-                       cudaStream_t st, uint64_t& launches) {
-    if (rounds == 7) {
-        if (sampler == RC_SAMPLER_REJECTION) return wavefront_run<MODE, 1, 7>(w, kp, accum, smem, st, 0, launches);
-        return wavefront_run<MODE, 0, 7>(w, kp, accum, smem, st, 0, launches);
-    }
-    if (sampler == RC_SAMPLER_REJECTION) return wavefront_run<MODE, 1, 10>(w, kp, accum, smem, st, 0, launches);
-    return wavefront_run<MODE, 0, 10>(w, kp, accum, smem, st, 0, launches);
-}
-
 inline int wavefront_render(WavefrontState& w, int mode, const KParams& kp, float* accum, int sampler, int rounds,
-                            size_t smem, cudaStream_t st, int sm_count, uint64_t& launches) {
-    int rc = wavefront_prepare(w, kp, sm_count);
+                            size_t smem, size_t smem_perlin, cudaStream_t st, uint64_t& launches) {
+    int rc = wavefront_prepare(w, kp);
     if (rc != RC_OK) return rc;
-    switch (mode) {
-    case RT_MODE_CONST_LINEAR: return wavefront_dispatch<RT_MODE_CONST_LINEAR>(w, kp, accum, sampler, rounds, smem, st, launches);
-    case RT_MODE_SMEM_BVH: return wavefront_dispatch<RT_MODE_SMEM_BVH>(w, kp, accum, sampler, rounds, smem, st, launches);
-    case RT_MODE_GLOBAL_BVH: return wavefront_dispatch<RT_MODE_GLOBAL_BVH>(w, kp, accum, sampler, rounds, smem, st, launches);
-    default: return wavefront_dispatch<RT_MODE_SMEM_LINEAR>(w, kp, accum, sampler, rounds, smem, st, launches);
-    }
+    return with_mode(mode, [&](auto m) {
+        constexpr int M = decltype(m)::value;
+        if (rounds == 7) {
+            if (sampler == RC_SAMPLER_REJECTION) return wavefront_run<M, 1, 7>(w, kp, accum, smem, smem_perlin, st, launches);
+            return wavefront_run<M, 0, 7>(w, kp, accum, smem, smem_perlin, st, launches);
+        }
+        if (sampler == RC_SAMPLER_REJECTION) return wavefront_run<M, 1, 10>(w, kp, accum, smem, smem_perlin, st, launches);
+        return wavefront_run<M, 0, 10>(w, kp, accum, smem, smem_perlin, st, launches);
+    });
 }
