@@ -336,6 +336,65 @@ int rc_render_adaptive(rc_ctx* ctx, const rc_params* params, const rc_adaptive* 
                        double* out_rgb, int32_t* out_spp, double* out_err,
                        const volatile int32_t* cancel);
 
+/* Denoised rendering: a render of params->samples (S >= 2) samples per pixel, filtered on the GPU by an edge-avoiding
+ * à-trous wavelet filter guided by per-pixel variance and first-hit features (SVGF's spatial filter, without its
+ * temporal part).
+ * Inputs of the filter, per pixel p of the W x H image (what rc_denoise_aux returns):
+ *   m_p    linear mean radiance (rgb): sum / S of the same samples rc_render traces (up to the order of fp32 sums);
+ *   v_p    variance of the mean of y = (r + g + b) / 3: s^2 / S with s^2 = max(0, (S2 - S1^2 / S) / (S - 1)), S1 = sum y,
+ *          S2 = sum y^2 over the pixel's samples (S2 from fp32 sums of y^2, as rc_render_adaptive's test);
+ *   alb_p  the first hit's albedo: the texture colour for Lambertian and Metal, (1, 1, 1) for dielectrics, lights and
+ *          misses;
+ *   n_p, z_p, id_p   the first hit's normal, t (the primary direction is not normalised, so t is proportional to
+ *          depth along the view axis) and object id (0 = miss): rc_primary_aov's precision-32 values, from the centre ray
+ *          of the pixel (fixed jitter).
+ * Every input is rounded to fp32; the filter runs in fp32.
+ *   Demodulate: a_p = max(alb_p, 1e-3) per channel, c_p = m_p / a_p, abar_p = mean(a_p), var_p = v_p / abar_p^2;
+ *     l = (c.r + c.g + c.b) / 3.
+ *   Level k = 0 .. levels-1, step s = 2^k: taps q = p + s (i, j), i, j in -2..2; taps outside the image are skipped.
+ *     g_p = 3x3 blur of var with weights [1/4, 1/2, 1/4]^2 over the in-image pixels around p (unit spacing),
+ *       renormalised by the weights used, no id test; recomputed from each level's input var.
+ *     w(p, q) = h(i) h(j) [id_p == id_q] w_l w_n w_z, h = [1/16, 1/4, 3/8, 1/4, 1/16],
+ *       w_l = exp(-|l_p - l_q| / (sigma_l sqrt(g_p) + 1e-3)), w_n = max(0, n_p . n_q)^sigma_n,
+ *       w_z = exp(-|z_p - z_q| / (sigma_z z_p |(i, j)| s / H)); w_n = w_z = 1 for q = p and where id_p = 0.
+ *     c'_p = sum w c_q / sum w, var'_p = sum w^2 var_q / (sum w)^2 (the centre tap keeps sum w >= (3/8)^2).
+ *   Remodulate and gamma: out_p = sqrt(max(0, a_p c_p)) per channel — rc_render's units.  levels = 0 gives the noisy
+ *   image up to rounding.
+ * out_rgb: width*height*3 doubles.  aux (may be NULL; each of its pointers may be NULL): the filter's inputs in f64 as
+ * this call built them — mean (W*H*3), var (W*H), albedo (W*H*3), normal (W*H*3), depth (W*H; DBL_MAX for a miss),
+ * id (W*H) — so rc_denoise_filter on them gives the same out_rgb bit for bit.
+ * rc_get_stats: samples = W*H*S; segments, gpu_ms and kernel_launches of the whole call (render, guides, filter);
+ * specialized as for rc_render.  `cancel`: as for rc_render (checked at entry and relayed during the render; a
+ * cancelled call writes nothing).  Supported: a one-device context, world <= 1, the megakernel, the direct sampler,
+ * 10 Philox rounds, samples >= 2; specialize as for rc_render.  Anything else is RC_ERR_INVALID, and so are levels
+ * outside 0..10, sigma_l <= 0, sigma_z <= 0, sigma_n < 0 and any sigma that is not finite. */
+typedef struct rc_denoise {
+    int32_t levels;        /* à-trous levels, 0..10 (SVGF: 5)                                          */
+    int32_t reserved;
+    double  sigma_l;       /* luminance edge stop, > 0 (SVGF: 4)                                        */
+    double  sigma_n;       /* normal edge stop exponent, >= 0 (SVGF: 128)                               */
+    double  sigma_z;       /* depth edge stop, > 0 (SVGF: 1)                                            */
+} rc_denoise;
+
+typedef struct rc_denoise_aux {   /* optional outputs of rc_render_denoised; any may be NULL */
+    double*   mean;
+    double*   var;
+    double*   albedo;
+    double*   normal;
+    double*   depth;
+    uint32_t* id;
+} rc_denoise_aux;
+
+int rc_render_denoised(rc_ctx* ctx, const rc_params* params, const rc_denoise* denoise, double* out_rgb,
+                       const rc_denoise_aux* aux, const volatile int32_t* cancel);
+
+/* The filter of rc_render_denoised on the caller's inputs (layouts as rc_denoise_aux; depth must be finite and > 0
+ * where id != 0), on device 0 of the context; needs no scene.  rc_get_stats: gpu_ms of the filter's kernels (not the
+ * copies), kernel_launches = 2 + levels, samples = 0.  Same parameter checks as rc_render_denoised. */
+int rc_denoise_filter(rc_ctx* ctx, const rc_denoise* denoise, int32_t width, int32_t height, const double* mean,
+                      const double* var, const double* albedo, const double* normal, const double* depth,
+                      const uint32_t* id, double* out_rgb);
+
 /* The whole of CpuRendererScaled::render (src/renderer/cpu_scaled.rs:37-121), the preview renderer
  * (`preview_renderer`, src/config.rs:203-207, used while the camera moves, src/main.rs:174-190).
  * params->width/height are the screen; params->samples / max_depth come from config.preview

@@ -95,6 +95,16 @@ class rc_adaptive(C.Structure):
     _fields_ = [("min_samples", C.c_int32), ("reserved", C.c_int32), ("threshold", C.c_double)]
 
 
+class rc_denoise(C.Structure):
+    _fields_ = [("levels", C.c_int32), ("reserved", C.c_int32), ("sigma_l", C.c_double), ("sigma_n", C.c_double),
+                ("sigma_z", C.c_double)]
+
+
+class rc_denoise_aux(C.Structure):
+    _fields_ = [("mean", C.POINTER(C.c_double)), ("var", C.POINTER(C.c_double)), ("albedo", C.POINTER(C.c_double)),
+                ("normal", C.POINTER(C.c_double)), ("depth", C.POINTER(C.c_double)), ("id", C.POINTER(C.c_uint32))]
+
+
 class rc_tone_map(C.Structure):
     _fields_ = [("type", C.c_int32), ("reserved", C.c_int32), ("max_white", C.c_double),
                 ("hable", C.c_double * 6), ("exposure_bias", C.c_double),
@@ -115,6 +125,7 @@ ABI_SYMBOLS = [
     "rc_shared_close", "rc_frame_create", "rc_frame_open", "rc_frame_close", "rc_render_frame",
     "rc_render_accumulate", "rc_finalize", "rc_postprocess", "rc_primary_aov", "rc_get_stats",
     "rc_last_error", "rc_abi_version", "rc_fp32_peak", "rc_partition", "rc_spec_source", "rc_render_adaptive",
+    "rc_render_denoised", "rc_denoise_filter",
 ]
 
 
@@ -147,6 +158,10 @@ def load(path: str | None = None) -> C.CDLL:
     lib.rc_render.argtypes = [vp, C.POINTER(rc_params), C.POINTER(C.c_double), C.POINTER(C.c_int32)]
     lib.rc_render_adaptive.argtypes = [vp, C.POINTER(rc_params), C.POINTER(rc_adaptive), C.POINTER(C.c_double),
                                        C.POINTER(C.c_int32), C.POINTER(C.c_double), C.POINTER(C.c_int32)]
+    lib.rc_render_denoised.argtypes = [vp, C.POINTER(rc_params), C.POINTER(rc_denoise), C.POINTER(C.c_double),
+                                       C.POINTER(rc_denoise_aux), C.POINTER(C.c_int32)]
+    lib.rc_denoise_filter.argtypes = [vp, C.POINTER(rc_denoise), C.c_int32, C.c_int32] + [C.POINTER(C.c_double)] * 5 + \
+        [C.POINTER(C.c_uint32), C.POINTER(C.c_double)]
     lib.rc_render_tiles_into.argtypes = [vp, C.POINTER(rc_params), vp, C.POINTER(C.c_int32)]
     lib.rc_shared_alloc.argtypes = [vp, C.c_uint64, C.POINTER(vp), C.POINTER(C.c_uint8)]
     lib.rc_shared_open.argtypes = [vp, C.POINTER(C.c_uint8), C.POINTER(vp)]

@@ -21,6 +21,7 @@
 #include "rc_multi.cuh"
 #include "rc_lbvh.cuh"
 #include "rc_spec.cuh"
+#include "rt_denoise.cuh"
 
 namespace {
 
@@ -160,6 +161,11 @@ struct DeviceState {
     DevBuf<int> ad_spp;
     DevBuf<float> ad_m2;
     DevBuf<double> ad_s2, ad_err;
+    // rc_render_denoised / rc_denoise_filter: the filter's f64 inputs (mean, var, albedo, normal, depth, id), its
+    // fp32 working images ((c.rgb, var) ping-pong, (n.xyz, z), albedo)
+    DevBuf<double> dn_mean, dn_var, dn_alb, dn_nrm, dn_depth;
+    DevBuf<uint32_t> dn_id;
+    DevBuf<float4> dn_cv[2], dn_nz, dn_a;
     WavefrontState wf;
     std::map<std::string, SpecKernel> spec_cache;   // scene-specialised kernels loaded on this device
     int sm_count = 0, clock_khz = 0;
@@ -1218,6 +1224,8 @@ int rc_destroy(rc_ctx* ctx) {
         d.tables.release();
         d.accum.release(); d.slice_buf.release(); d.out64.release(); d.counter.release(); d.cancel_word.release();
         d.ad_active.release(); d.ad_spp.release(); d.ad_m2.release(); d.ad_s2.release(); d.ad_err.release();
+        d.dn_mean.release(); d.dn_var.release(); d.dn_alb.release(); d.dn_nrm.release(); d.dn_depth.release(); d.dn_id.release();
+        d.dn_cv[0].release(); d.dn_cv[1].release(); d.dn_nz.release(); d.dn_a.release();
         if (d.cancel_stream) cudaStreamDestroy(d.cancel_stream);
         d.pp_in.release(); d.pp_mapped.release(); d.pp_rgba.release();
         if (d.ev_traced) cudaEventDestroy(d.ev_traced);
@@ -1683,6 +1691,167 @@ int rc_render_adaptive(rc_ctx* ctx, const rc_params* p, const rc_adaptive* a, do
     ctx->stats.samples = samples;
     ctx->stats.kernel_launches = launches;
     ctx->stats.specialized = specialized;
+    return RC_OK;
+}
+
+static int check_denoise(const rc_denoise* dn) {
+    if (dn->levels < 0 || dn->levels > 10) return fail(RC_ERR_INVALID, "levels must be in 0..10");
+    if (!std::isfinite(dn->sigma_l) || !std::isfinite(dn->sigma_n) || !std::isfinite(dn->sigma_z))
+        return fail(RC_ERR_INVALID, "sigma_l, sigma_n and sigma_z must be finite");
+    if (!(dn->sigma_l > 0.0) || !(dn->sigma_z > 0.0) || !(dn->sigma_n >= 0.0))
+        return fail(RC_ERR_INVALID, "sigma_l and sigma_z must be > 0, sigma_n >= 0");
+    return RC_OK;
+}
+
+static int reserve_denoise(DeviceState& d, size_t n_pix) {
+    CUDA_TRY(d.dn_mean.reserve(3 * n_pix)); CUDA_TRY(d.dn_var.reserve(n_pix)); CUDA_TRY(d.dn_alb.reserve(3 * n_pix));
+    CUDA_TRY(d.dn_nrm.reserve(3 * n_pix)); CUDA_TRY(d.dn_depth.reserve(n_pix)); CUDA_TRY(d.dn_id.reserve(n_pix));
+    CUDA_TRY(d.dn_cv[0].reserve(n_pix)); CUDA_TRY(d.dn_cv[1].reserve(n_pix));
+    CUDA_TRY(d.dn_nz.reserve(n_pix)); CUDA_TRY(d.dn_a.reserve(n_pix));
+    CUDA_TRY(d.out64.reserve(3 * n_pix));
+    return RC_OK;
+}
+
+// The filter on the f64 inputs in d.dn_*: prepare, `levels` à-trous levels, finish into d.out64 (2 + levels launches)
+static int run_denoise_filter(DeviceState& d, const rc_denoise* dn, int width, int height) {
+    const size_t n_pix = (size_t)width * height;
+    const unsigned grid = (unsigned)((n_pix + 255) / 256);
+    denoise_prepare_kernel<<<grid, 256, 0, d.stream>>>(d.dn_mean.p, d.dn_var.p, d.dn_alb.p, d.dn_nrm.p, d.dn_depth.p,
+                                                       d.dn_cv[0].p, d.dn_nz.p, d.dn_a.p, n_pix);
+    CUDA_TRY(cudaGetLastError());
+    const dim3 block(RT_DENOISE_BX, RT_DENOISE_BY), grid2((width + RT_DENOISE_BX - 1) / RT_DENOISE_BX, (height + RT_DENOISE_BY - 1) / RT_DENOISE_BY);
+    int cur = 0;
+    for (int k = 0; k < dn->levels; ++k, cur ^= 1) {
+        denoise_level_kernel<<<grid2, block, 0, d.stream>>>(d.dn_cv[cur].p, d.dn_cv[cur ^ 1].p, d.dn_nz.p, d.dn_id.p, width, height,
+                                                            1 << k, (float)dn->sigma_l, (float)dn->sigma_n, (float)dn->sigma_z);
+        CUDA_TRY(cudaGetLastError());
+    }
+    denoise_finish_kernel<<<grid, 256, 0, d.stream>>>(d.dn_cv[cur].p, d.dn_a.p, d.out64.p, n_pix);
+    CUDA_TRY(cudaGetLastError());
+    return RC_OK;
+}
+
+int rc_render_denoised(rc_ctx* ctx, const rc_params* p, const rc_denoise* dn, double* out_rgb, const rc_denoise_aux* aux,
+                       const volatile int32_t* cancel) {
+    if (!ctx || !dn || !out_rgb) return fail(RC_ERR_INVALID, "ctx, denoise or out_rgb is NULL");
+    int rc = check_params(p);
+    if (rc != RC_OK) return rc;
+    if (ctx->devs.size() != 1 || p->world > 1) return fail(RC_ERR_INVALID, "denoised rendering needs a one-device context and world <= 1");
+    if (p->variant != RC_VARIANT_MEGAKERNEL || p->sampler != RC_SAMPLER_DIRECT || (p->rng_rounds != 0 && p->rng_rounds != 10))
+        return fail(RC_ERR_INVALID, "denoised rendering needs the megakernel, the direct sampler and 10 Philox rounds");
+    if (p->specialize == 1 && p->fixed_jitter) return fail(RC_ERR_INVALID, "specialize = 1 needs fixed_jitter = 0");
+    if (p->samples < 2) return fail(RC_ERR_INVALID, "denoised rendering needs samples >= 2 (the variance of a pixel)");
+    rc = check_denoise(dn);
+    if (rc != RC_OK) return rc;
+    if (!ctx->has_scene || !ctx->has_camera) return fail(RC_ERR_STATE, "upload a scene and set a camera first");
+    if (cancelled(cancel)) return fail(RC_ERR_CANCELLED, "cancel flag set before the render started");
+    DeviceState& d = ctx->devs[0];
+    CUDA_TRY(cudaSetDevice(d.device));
+    const size_t n_pix = (size_t)p->width * p->height;
+    CUDA_TRY(d.ad_active.reserve(n_pix));
+    CUDA_TRY(d.ad_m2.reserve(n_pix));
+    rc = reserve_denoise(d, n_pix);
+    if (rc != RC_OK) return rc;
+    // the call's start: the moments round is timed and counted with the guide and filter kernels (trace_share leaves both alone)
+    CUDA_TRY(cudaEventRecord(d.ev0, d.stream));
+    CUDA_TRY(cudaMemsetAsync(d.counter.p, 0, sizeof(unsigned long long), d.stream));
+    rc = ensure_accum(ctx, p, true);
+    if (rc != RC_OK) return rc;
+    // the noisy render: one moments round [0, S) over every pixel, the kernel rc_render_adaptive's rounds run
+    CUDA_TRY(cudaMemsetAsync(d.ad_active.p, 1, n_pix, d.stream));
+    const AdaptiveRound round{d.ad_active.p, d.ad_m2.p, 0, p->samples};
+    ShareCall call{d.accum.p, cancel};
+    call.round = &round;
+    bool was_cancelled = false;
+    rc = trace_share(ctx, p, call, was_cancelled);
+    if (rc != RC_OK) return rc;
+    if (was_cancelled) return RC_OK;   // a cancelled render writes nothing, cpu.rs:55-62
+    uint64_t launches = ctx->stats.kernel_launches;
+    const int specialized = ctx->stats.specialized;
+    const unsigned grid = (unsigned)((n_pix + 255) / 256);
+    denoise_moments_kernel<<<grid, 256, 0, d.stream>>>(d.accum.p, d.ad_m2.p, d.dn_mean.p, d.dn_var.p, n_pix, p->samples);
+    CUDA_TRY(cudaGetLastError());
+    // The guides, from the centre ray of each pixel (fixed jitter): id, t and normal from the very kernel rc_primary_aov
+    // runs (precision 32), the albedo from its GUIDE instantiation.  That one is compiled on its own, and its fp32 t
+    // came out different in the last bits on three of the five BASELINE scenes, so it supplies the albedo only.
+    {
+        KParams kp = ctx->kp;
+        d.tables.bind(kp);
+        for (size_t i = 0; i < d.tex.size(); ++i) kp.images[i] = d.tex[i];
+        kp.segment_counter = nullptr;
+        kp.cancel_flag = nullptr;
+        rc_params q = *p;
+        q.fixed_jitter = 1; q.split = RC_SPLIT_TILES;
+        partition(kp, &q, 0, 1);
+        // Perlin tables are read from global memory: one texture lookup per pixel
+        const size_t smem = ctx->smem_bytes - scene_staging(ctx->mode, kp.n_nodes, kp.n_prims, kp.n_perlin).perlin;
+        kp.n_perlin = 0;
+        rc = with_mode(ctx->mode, [&](auto m) {
+            int r = set_smem(primary_aov_kernel<decltype(m)::value>, smem);
+            if (r == RC_OK) r = set_smem(primary_aov_kernel<decltype(m)::value, true>, smem);
+            if (r != RC_OK) return r;
+            primary_aov_kernel<decltype(m)::value><<<kp.n_tiles, RT_BLOCK, smem, d.stream>>>(kp, d.dn_id.p, d.dn_depth.p, d.dn_nrm.p, nullptr);
+            primary_aov_kernel<decltype(m)::value, true><<<kp.n_tiles, RT_BLOCK, smem, d.stream>>>(kp, nullptr, nullptr, nullptr, nullptr,
+                                                                                                   d.dn_alb.p);
+            return r;
+        });
+        if (rc != RC_OK) return rc;
+        CUDA_TRY(cudaGetLastError());
+    }
+    rc = run_denoise_filter(d, dn, p->width, p->height);
+    if (rc != RC_OK) return rc;
+    launches += 5 + dn->levels;   // moments, two guide kernels, prepare, the levels, finish
+    rc = finish_stats(ctx, p);
+    if (rc != RC_OK) return rc;
+    CUDA_TRY(cudaMemcpyAsync(out_rgb, d.out64.p, 3 * n_pix * sizeof(double), cudaMemcpyDeviceToHost, d.stream));
+    if (aux) {
+        auto get = [&](void* dst, const void* src, size_t bytes) {
+            return dst ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, d.stream) : cudaSuccess;
+        };
+        CUDA_TRY(get(aux->mean, d.dn_mean.p, 3 * n_pix * sizeof(double)));
+        CUDA_TRY(get(aux->var, d.dn_var.p, n_pix * sizeof(double)));
+        CUDA_TRY(get(aux->albedo, d.dn_alb.p, 3 * n_pix * sizeof(double)));
+        CUDA_TRY(get(aux->normal, d.dn_nrm.p, 3 * n_pix * sizeof(double)));
+        CUDA_TRY(get(aux->depth, d.dn_depth.p, n_pix * sizeof(double)));
+        CUDA_TRY(get(aux->id, d.dn_id.p, n_pix * sizeof(uint32_t)));
+    }
+    CUDA_TRY(cudaStreamSynchronize(d.stream));
+    ctx->stats.kernel_launches = launches;
+    ctx->stats.specialized = specialized;
+    return RC_OK;
+}
+
+int rc_denoise_filter(rc_ctx* ctx, const rc_denoise* dn, int32_t width, int32_t height, const double* mean, const double* var,
+                      const double* albedo, const double* normal, const double* depth, const uint32_t* id, double* out_rgb) {
+    if (!ctx || !dn || !mean || !var || !albedo || !normal || !depth || !id || !out_rgb)
+        return fail(RC_ERR_INVALID, "ctx, denoise, an input or out_rgb is NULL");
+    if (width < 1 || height < 1 || (long long)width * height > (1 << 24)) return fail(RC_ERR_INVALID, "width and height must be >= 1, at most 2^24 pixels");
+    int rc = check_denoise(dn);
+    if (rc != RC_OK) return rc;
+    DeviceState& d = ctx->devs[0];
+    CUDA_TRY(cudaSetDevice(d.device));
+    const size_t n_pix = (size_t)width * height;
+    rc = reserve_denoise(d, n_pix);
+    if (rc != RC_OK) return rc;
+    auto put = [&](void* dst, const void* src, size_t bytes) { return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, d.stream); };
+    CUDA_TRY(put(d.dn_mean.p, mean, 3 * n_pix * sizeof(double)));
+    CUDA_TRY(put(d.dn_var.p, var, n_pix * sizeof(double)));
+    CUDA_TRY(put(d.dn_alb.p, albedo, 3 * n_pix * sizeof(double)));
+    CUDA_TRY(put(d.dn_nrm.p, normal, 3 * n_pix * sizeof(double)));
+    CUDA_TRY(put(d.dn_depth.p, depth, n_pix * sizeof(double)));
+    CUDA_TRY(put(d.dn_id.p, id, n_pix * sizeof(uint32_t)));
+    // timed: the filter's kernels only, not the copies
+    CUDA_TRY(cudaEventRecord(d.ev0, d.stream));
+    CUDA_TRY(cudaMemsetAsync(d.counter.p, 0, sizeof(unsigned long long), d.stream));
+    rc = run_denoise_filter(d, dn, width, height);
+    if (rc != RC_OK) return rc;
+    CUDA_TRY(cudaEventRecord(d.ev1, d.stream));
+    CUDA_TRY(cudaMemcpyAsync(out_rgb, d.out64.p, 3 * n_pix * sizeof(double), cudaMemcpyDeviceToHost, d.stream));
+    CUDA_TRY(cudaStreamSynchronize(d.stream));
+    ctx->stats.samples = 0;
+    ctx->stats.kernel_launches = 2 + dn->levels;
+    ctx->stats.specialized = 0;
+    ctx->stats_pending = true;
     return RC_OK;
 }
 

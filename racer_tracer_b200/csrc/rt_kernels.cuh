@@ -720,14 +720,27 @@ __global__ void adaptive_init_kernel(uint8_t* __restrict__ active, int* __restri
 }
 
 
+// The albedo shade_hit multiplies a path's throughput by at this hit: the texture colour for Lambertian and Metal,
+// (1, 1, 1) for dielectrics and lights (rc_render_denoised's albedo guide)
+template <class Scene>
+RT_D vec3f hit_albedo(const KParams& P, const SmemLayout& L, const Scene& S, int prim, const Hit& h) {
+    const float mat = S.pn(prim).w;
+    if (mat != (float)RT_MAT_LAMBERTIAN && mat != (float)RT_MAT_METAL) return mk3(1.0f, 1.0f, 1.0f);
+    const float4 pb = S.pb(prim), pc = S.pc(prim);
+    if (kinds_tex(pb.z) == RT_TEX_SOLID) return mk3(pc.x, pc.y, pc.z);
+    TexCtx X; X.perlin = L.perlin; X.perm = L.perm;
+    return texture_value(P, X, S, __float_as_int(pb.w), prim, h);
+}
+
 // ---------------------------------------------------------------------------
 // Primary-visibility AOV (RayImageData, src/renderer.rs:33-39): fixed jitter,
 // one closest hit per pixel through the renderer's fp32 code.
+// GUIDE: also the hit's albedo (hit_albedo; (1, 1, 1) for a miss) into `albedo`.
 // ---------------------------------------------------------------------------
-template <int MODE>
+template <int MODE, bool GUIDE = false>
 __global__ void __launch_bounds__(RT_BLOCK)
 primary_aov_kernel(const __grid_constant__ KParams P, uint32_t* __restrict__ id, double* __restrict__ t_out,
-                   double* __restrict__ normal, double* __restrict__ point) {
+                   double* __restrict__ normal, double* __restrict__ point, double* __restrict__ albedo = nullptr) {
     extern __shared__ __align__(16) unsigned char smem[];
     SmemLayout L = stage_scene<MODE>(P, smem);
     const int tile = P.tile_first + blockIdx.x * P.tile_stride;
@@ -745,16 +758,20 @@ primary_aov_kernel(const __grid_constant__ KParams P, uint32_t* __restrict__ id,
     int prim;
     Hit h;
     uint32_t oid = 0;
+    vec3f alb = mk3(1.0f, 1.0f, 1.0f);
     if (MODE == RT_MODE_CONST_LINEAR) {
         ConstScene S(P, L.prims);
         prim = closest_hit<MODE>(P, S, r, -1, t);
         if (prim >= 0) { h = make_hit(S, prim, r, t); oid = (uint32_t)__float_as_int(S.pc(prim).w); }
+        if constexpr (GUIDE) { if (prim >= 0) alb = hit_albedo(P, L, S, prim, h); }
     } else {
         PtrScene S; S.prims = L.prims; S.nodes = L.nodes; S.inst = P.instances; S.ref_aabb = P.ref_aabb;
         prim = closest_hit<MODE>(P, S, r, -1, t);
         if (prim >= 0) { h = make_hit(S, prim, r, t); oid = (uint32_t)__float_as_int(S.pc(prim).w); }
+        if constexpr (GUIDE) { if (prim >= 0) alb = hit_albedo(P, L, S, prim, h); }
     }
     size_t i = pc.pixel;
+    if constexpr (GUIDE) { albedo[3 * i] = alb.x; albedo[3 * i + 1] = alb.y; albedo[3 * i + 2] = alb.z; }
     if (prim < 0) {
         if (id) id[i] = 0;
         if (t_out) t_out[i] = 1.7976931348623157e308;

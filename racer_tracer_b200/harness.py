@@ -789,6 +789,11 @@ def make_params(width, height, samples, max_depth, seed=0, variant=capi.RC_VARIA
     return p
 
 
+def default_denoise(levels=5, sigma_l=4.0, sigma_n=128.0, sigma_z=1.0) -> capi.rc_denoise:
+    """rc_denoise with SVGF's published parameters unless given."""
+    return capi.rc_denoise(levels=levels, sigma_l=sigma_l, sigma_n=sigma_n, sigma_z=sigma_z)
+
+
 def preview_scales(cfg: "Config", width: int, height: int) -> tuple[int, int]:
     """CpuRendererScaled::new (src/renderer/cpu_scaled.rs:17-43): the highest divisor of
     image.width / num_threads_width (height likewise) that does not exceed config.preview.scale."""
@@ -963,6 +968,41 @@ class CudaRenderer:
                                                          spp.ctypes.data_as(C.POINTER(C.c_int32)),
                                                          err.ctypes.data_as(C.POINTER(C.c_double)), cptr))
         return rgb, spp, err
+
+    def render_denoised(self, params: rc_params, denoise: capi.rc_denoise | None = None, aux=False, cancel=None):
+        """rc_render_denoised -> rgb (H, W, 3) float64, or (rgb, aux) with aux = the filter's inputs as the call built
+        them: {"mean": (H, W, 3), "var": (H, W), "albedo": (H, W, 3), "normal": (H, W, 3), "depth": (H, W),
+        "id": (H, W) uint32}.  denoise=None: SVGF's parameters (levels 5, sigma_l 4, sigma_n 128, sigma_z 1)."""
+        h, w = params.height, params.width
+        dn = denoise if denoise is not None else default_denoise()
+        rgb = np.empty((h, w, 3), dtype=np.float64)
+        arrays, aux_ptr = None, None
+        if aux:
+            arrays = {"mean": np.empty((h, w, 3)), "var": np.empty((h, w)), "albedo": np.empty((h, w, 3)),
+                      "normal": np.empty((h, w, 3)), "depth": np.empty((h, w)), "id": np.empty((h, w), dtype=np.uint32)}
+            a = capi.rc_denoise_aux()
+            for k, v in arrays.items():
+                setattr(a, k, v.ctypes.data_as(C.POINTER(C.c_uint32 if k == "id" else C.c_double)))
+            aux_ptr = C.byref(a)
+        cptr = C.cast(C.pointer(cancel), C.POINTER(C.c_int32)) if cancel is not None else None
+        capi.check(self.lib, self.lib.rc_render_denoised(self.ctx, C.byref(params), C.byref(dn),
+                                                         rgb.ctypes.data_as(C.POINTER(C.c_double)), aux_ptr, cptr))
+        return (rgb, arrays) if aux else rgb
+
+    def denoise_filter(self, mean, var, albedo, normal, depth, ids, denoise: capi.rc_denoise | None = None) -> np.ndarray:
+        """rc_denoise_filter on host arrays shaped as render_denoised's aux -> rgb (H, W, 3) float64."""
+        h, w = np.shape(var)
+        dn = denoise if denoise is not None else default_denoise()
+        f64 = [np.ascontiguousarray(x, dtype=np.float64) for x in (mean, var, albedo, normal, depth)]
+        for x, shape in zip(f64, ((h, w, 3), (h, w), (h, w, 3), (h, w, 3), (h, w))):
+            assert x.shape == shape, (x.shape, shape)
+        ids = np.ascontiguousarray(ids, dtype=np.uint32)
+        assert ids.shape == (h, w)
+        rgb = np.empty((h, w, 3), dtype=np.float64)
+        capi.check(self.lib, self.lib.rc_denoise_filter(
+            self.ctx, C.byref(dn), w, h, *[x.ctypes.data_as(C.POINTER(C.c_double)) for x in f64],
+            ids.ctypes.data_as(C.POINTER(C.c_uint32)), rgb.ctypes.data_as(C.POINTER(C.c_double))))
+        return rgb
 
     def render_preview(self, params: rc_params, scale_w: int, scale_h: int, cancel=None) -> np.ndarray:
         """rc_render_preview: what CpuRendererScaled sends (cpu_scaled.rs); params = screen size + config.preview."""

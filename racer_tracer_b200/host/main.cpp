@@ -7,6 +7,7 @@
 //   racer_render --config config.yml --scene scene.yml [--width W --height H] [--samples N]
 //                [--max-depth D] [--seed S] [--preview] [--out image.png] [--image-dir DIR]
 //                [--adaptive T [--min-samples N]]   (adaptive sampling up to --samples per pixel: gpu.adaptive)
+//                [--denoise [--denoise-levels N]]   (a filtered render: gpu.denoise; excludes --adaptive)
 //                [--dump-flat scene.json]      (flat tables as JSON; needs no GPU)
 #include <chrono>
 #include <cstdio>
@@ -50,6 +51,8 @@ int main(int argc, char** argv) {
     bool have_adaptive = false;
     double adaptive = 0.0;
     long min_samples = -1;
+    bool have_denoise = false;
+    long denoise_levels = -1;
     try {
         for (int i = 1; i < argc; ++i) {
             const std::string a = argv[i];
@@ -86,6 +89,8 @@ int main(int argc, char** argv) {
             else if (a == "--preview") preview = true;
             else if (a == "--adaptive") { adaptive = std::atof(next().c_str()); have_adaptive = true; }
             else if (a == "--min-samples") min_samples = std::atol(next().c_str());
+            else if (a == "--denoise") have_denoise = true;
+            else if (a == "--denoise-levels") denoise_levels = std::atol(next().c_str());
             else throw TracerError(TracerError::ArgumentParsingError, "Argument parsing Error: unknown argument " + a);
         }
         Config config = config_path.empty() ? Config() : Config::from_file(config_path);
@@ -99,6 +104,14 @@ int main(int argc, char** argv) {
             if (!config.gpu.adaptive) throw TracerError(TracerError::ArgumentParsingError, "Argument parsing Error: --min-samples needs --adaptive");
             config.gpu.adaptive_min_samples = (int32_t)min_samples;
         }
+        if (denoise_levels >= 0 && !have_denoise)
+            throw TracerError(TracerError::ArgumentParsingError, "Argument parsing Error: --denoise-levels needs --denoise");
+        if (have_denoise) {
+            config.gpu.denoise = true;
+            if (denoise_levels >= 0) config.gpu.denoise_levels = (int32_t)denoise_levels;
+        }
+        if (config.gpu.adaptive && config.gpu.denoise)   // (both blocks in the file: a configuration error already)
+            throw TracerError(TracerError::ArgumentParsingError, "Argument parsing Error: --denoise and --adaptive exclude each other");
         if (scene_path.empty() && config.loader.kind == SceneLoaderConfig::Yml) scene_path = config.loader.path;
         if (scene_path.empty() && config.loader.kind == SceneLoaderConfig::Random) scene_path = "random";
         if (scene_path.empty() && config.loader.kind == SceneLoaderConfig::Sandbox) scene_path = "sandbox:../resources/scenes/cornell_box.yml";   // sandbox.rs:41-42

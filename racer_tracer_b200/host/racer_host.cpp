@@ -433,6 +433,14 @@ Config Config::from_file(const std::string& file) {
                 if (a->has("threshold")) cfg.gpu.adaptive_threshold = a->at("threshold").as_double();
                 if (a->has("min_samples")) cfg.gpu.adaptive_min_samples = (int32_t)a->at("min_samples").as_int();
             }
+            if (const Node* dn = g->find("denoise")) {
+                cfg.gpu.denoise = true;
+                if (dn->has("levels")) cfg.gpu.denoise_levels = (int32_t)dn->at("levels").as_int();
+                if (dn->has("sigma_l")) cfg.gpu.denoise_sigma_l = dn->at("sigma_l").as_double();
+                if (dn->has("sigma_n")) cfg.gpu.denoise_sigma_n = dn->at("sigma_n").as_double();
+                if (dn->has("sigma_z")) cfg.gpu.denoise_sigma_z = dn->at("sigma_z").as_double();
+            }
+            if (cfg.gpu.adaptive && cfg.gpu.denoise) throw TracerError(TracerError::Configuration, "Config Error (" + file + "): gpu.adaptive and gpu.denoise exclude each other");
         }
     } catch (const yaml_lite::ParseError& e) {
         throw TracerError(TracerError::Configuration, "Config Error (" + file + "): " + e.what());
@@ -973,6 +981,12 @@ void CudaRenderer::render(const RenderData& rd, const DataWriter<ImageBufferEven
         a.threshold = gpu_.adaptive_threshold;
         check(rc_render_adaptive(ctx_, &p, &a, reinterpret_cast<double*>(ev.rgb.data()), nullptr, nullptr, rd.cancel_event),
               "rc_render_adaptive");
+    } else if (gpu_.denoise) {
+        rc_denoise dn;
+        std::memset(&dn, 0, sizeof(dn));
+        dn.levels = gpu_.denoise_levels;
+        dn.sigma_l = gpu_.denoise_sigma_l; dn.sigma_n = gpu_.denoise_sigma_n; dn.sigma_z = gpu_.denoise_sigma_z;
+        check(rc_render_denoised(ctx_, &p, &dn, reinterpret_cast<double*>(ev.rgb.data()), nullptr, rd.cancel_event), "rc_render_denoised");
     } else {
         check(rc_render(ctx_, &p, reinterpret_cast<double*>(ev.rgb.data()), rd.cancel_event), "rc_render");
     }

@@ -77,6 +77,11 @@ struct GpuConfig {      // new optional `gpu:` block
     bool adaptive = false;
     double adaptive_threshold = 0.0;
     int32_t adaptive_min_samples = 16;
+    // optional `denoise: {levels, sigma_l, sigma_n, sigma_z}`: the full renderer filters its render (rc_render_denoised);
+    // excludes `adaptive`
+    bool denoise = false;
+    int32_t denoise_levels = 5;
+    double denoise_sigma_l = 4.0, denoise_sigma_n = 128.0, denoise_sigma_z = 1.0;
 };
 struct Config {         // config.rs:183-215
     RenderConfig preview, render;

@@ -99,6 +99,18 @@ pub struct rc_adaptive {
     pub min_samples: i32, pub reserved: i32, pub threshold: f64,
 }
 
+/// rc_render_denoised / rc_denoise_filter: the à-trous filter's levels and edge-stopping parameters.
+#[repr(C)] #[derive(Clone, Copy)]
+pub struct rc_denoise {
+    pub levels: i32, pub reserved: i32, pub sigma_l: f64, pub sigma_n: f64, pub sigma_z: f64,
+}
+
+/// rc_render_denoised: optional outputs, the filter's inputs as the call built them (any pointer may be null).
+#[repr(C)] #[derive(Clone, Copy)]
+pub struct rc_denoise_aux {
+    pub mean: *mut f64, pub var: *mut f64, pub albedo: *mut f64, pub normal: *mut f64, pub depth: *mut f64, pub id: *mut u32,
+}
+
 #[repr(C)] #[derive(Clone, Copy)]
 pub struct rc_tone_map {
     pub type_: i32, pub reserved: i32, pub max_white: f64, pub hable: [f64; 6], pub exposure_bias: f64,
@@ -123,6 +135,10 @@ extern "C" {
     pub fn rc_render(ctx: *mut rc_ctx, params: *const rc_params, out_rgb: *mut f64, cancel: *const i32) -> c_int;
     pub fn rc_render_adaptive(ctx: *mut rc_ctx, params: *const rc_params, a: *const rc_adaptive, out_rgb: *mut f64, out_spp: *mut i32,
                               out_err: *mut f64, cancel: *const i32) -> c_int;
+    pub fn rc_render_denoised(ctx: *mut rc_ctx, params: *const rc_params, denoise: *const rc_denoise, out_rgb: *mut f64,
+                              aux: *const rc_denoise_aux, cancel: *const i32) -> c_int;
+    pub fn rc_denoise_filter(ctx: *mut rc_ctx, denoise: *const rc_denoise, width: i32, height: i32, mean: *const f64, var: *const f64,
+                             albedo: *const f64, normal: *const f64, depth: *const f64, id: *const u32, out_rgb: *mut f64) -> c_int;
     pub fn rc_render_preview(ctx: *mut rc_ctx, params: *const rc_params, scale_w: i32, scale_h: i32, out_rgb: *mut f64,
                              cancel: *const i32) -> c_int;
     pub fn rc_render_tiles_into(ctx: *mut rc_ctx, params: *const rc_params, d_image: *mut f32, cancel: *const i32) -> c_int;
